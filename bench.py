@@ -2,7 +2,7 @@
 """bench.py — the reference's headline metric on B200: instance-samples/s (and DSP instructions/s)
 of the batched FX8010 interpreter, next to the reference's own CPU interpreter.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg3|cfg4|cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg3|cfg4|cfg5] [--dump-outputs DIR]
 
 One "step" = one fx8010_gpu_process_batch call = one block of 1 024 samples for every instance of
 this rank (BASELINE.json configs[1]: MACS gain + LOG waveshaper, 4 096 instances per GPU).  Instances
@@ -34,6 +34,7 @@ import progs  # noqa: E402  (program texts + stimuli shared with the tests)
 
 BLOCK = 1024          # samples per step (48 kHz blocks of 1 024 samples)
 L2_BYTES = 126 << 20
+DUMP_BYTES = 64 * 10**6       # --dump-outputs writes at most this much
 
 
 def workload(name: str):
@@ -369,6 +370,18 @@ class Workload:
         finally:
             g.close()
 
+    def dump_last_step(self, steps: int, path: str):
+        """The output block of the last of `steps` timed steps, [samples][instances] float32, as path/out.npy (call it before
+        anything else runs on the rotating buffers).  A block larger than DUMP_BYTES is cut to a fixed seeded sample of the
+        instances, in ascending order, so that runs with the same arguments write the same array."""
+        y = self.d_out[(steps - 1) % self.n_bufs]
+        k = (DUMP_BYTES - 4096) // (4 * BLOCK)
+        if self.n > k:
+            idx = np.sort(np.random.default_rng(progs.SEED).choice(self.n, k, replace=False))
+            y = y.index_select(1, self.torch.from_numpy(idx).to(y.device))
+        os.makedirs(path, exist_ok=True)
+        np.save(os.path.join(path, "out.npy"), y.cpu().numpy())
+
     def executed_per_step(self):
         g = self.new_handle()
         g.process_device(self.d_in[0], self.d_out[0], BLOCK, self.st); g.synchronize(self.st)
@@ -384,7 +397,8 @@ def main():
     faulthandler.enable()               # a native fault in any rank leaves a Python traceback on stderr
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="blocks per timed region of the headline measurement (and of its per-call and "
+                    "interpreter legs); the e2e leg runs max(10, min(K, 200)) steps and the sharded cfg3 / cfg4 / cfg5 records 10 / 20 / 3")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="cfg2")
@@ -396,7 +410,11 @@ def main():
     ap.add_argument("--no-interpreter-leg", action="store_true", help="skip timing the same steps on the interpreter kernels")
     ap.add_argument("--no-sharded", action="store_true", help="skip the cfg4 / cfg5 records of the scaling line")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the output block of the last one as DIR/out.npy "
+                    "(float32 [samples][instances] of rank 0; a fixed sample of the instances when larger than 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed (--impl ours)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -484,6 +502,8 @@ def main():
     ms_all, launches = W.timed(args.steps, args.warmup, max(1, args.repeats), barrier)
     ms_all = [max_over_ranks(m) for m in ms_all]
     ms = statistics.median(ms_all)
+    if args.dump_outputs and rank == 0:
+        W.dump_last_step(args.steps, args.dump_outputs)
     # keep the clock sampler running over a longer window of the same work so it sees load
     if rank == 0:
         ptrs = W.pointers(W.gpu, min(32, max(args.steps, 8)))

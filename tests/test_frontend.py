@@ -36,7 +36,7 @@ def test_frontend_matches_reference_records(fx):
     assert checked > 300
 
 
-def test_shipped_testcode_image(fx):
+def test_shipped_testcode_image(fx, tmp_path):
     """Decoded image of the reference's shipped testcode.da (SURVEY.md §8c): 14 registers, 2 instructions."""
     g = json.load(open(GOLD))["shipped_testcode_da"]
     names = [r[3] for r in g["registers"]]
@@ -46,11 +46,16 @@ def test_shipped_testcode_image(fx):
     # the same program without its comment lines decodes identically through our front-end
     r = record(fx, progs.CFG1A_TESTCODE)
     assert r["registers"] == g["registers"] and r["instructions"] == g["instructions"] and r["controls"] == g["controls"]
-    path = "/root/reference/source/testcode.da"
-    if os.path.exists(path):
-        p = fx.Program(path=path)
-        assert p.loaded and [list(i) for i in p.instructions()] == g["instructions"]
-        assert p.metadata() == g["metadata"]
+    # loaded from a file, with the shipped file's metadata lines (taken from the record) in front of the program:
+    # every field of the record, metadata included.  The file's text is rebuilt from the record, so this checks that
+    # `key "value"` lines decode to the recorded metadata, not the exact byte layout (comments) of the shipped file.
+    meta = "".join(f'{k} "{v}"\n' for k, v in g["metadata"].items())
+    path = tmp_path / "testcode.da"
+    path.write_text(meta + progs.CFG1A_TESTCODE.split("\n", 2)[2])          # the program after its name and copyright lines
+    p = fx.Program(path=str(path))
+    assert p.loaded and [list(i) for i in p.instructions()] == g["instructions"]
+    assert p.metadata() == g["metadata"]
+    assert record(fx, path.read_text()) == {k: g[k] for k in r}
 
 
 def test_frontend_live_fuzz_vs_reference(fx, po):
