@@ -60,6 +60,14 @@ class CControlEvent(C.Structure):
     _fields_ = [("sample", C.c_int32), ("reg_index", C.c_int32), ("broadcast", C.c_int32), ("reserved", C.c_int32), ("values", C.c_void_p)]
 
 
+class CControlCurve(C.Structure):
+    _fields_ = [("reg_index", C.c_int32), ("broadcast", C.c_int32), ("d_values", C.c_void_p)]
+
+
+MAX_CONTROL_CURVES = 8
+VARIANT_CURVES = 16        # fx8010_launch_info.kernel_variant: the last launch read control curves inside the kernel
+
+
 class CLaunchInfo(C.Structure):
     _fields_ = [("kernel_launches", C.c_ulonglong), ("last_grid", C.c_int32), ("last_block", C.c_int32),
                 ("last_time_split", C.c_int32), ("last_smem_bytes", C.c_int32), ("last_late_wait", C.c_int32),
@@ -114,6 +122,11 @@ GPU_SYMBOLS = {
     "fx8010_gpu_get_launch_info": (C.c_int, [C.c_void_p, C.POINTER(CLaunchInfo)]),
     "fx8010_gpu_translate_status": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_char_p, C.c_size_t]),
     "fx8010_translate_source": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_char_p, C.c_size_t, C.c_int, C.POINTER(C.c_int)]),
+    "fx8010_gpu_translate_status_curves": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                                     C.c_char_p, C.c_size_t]),
+    "fx8010_gpu_process_batch_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
+    "fx8010_translate_source_curves": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_char_p, C.c_size_t,
+                                                      C.c_int, C.POINTER(C.c_int)]),
 }
 
 MULTI_SYMBOLS = {
@@ -169,6 +182,8 @@ HOST_SYMBOLS = {
     "fx8010_host_instruction_counter": (C.c_int, [C.c_void_p]),
     "fx8010_host_instruction_counter_total": (C.c_ulonglong, [C.c_void_p]),
     "fx8010_host_gpu": (C.c_void_p, [C.c_void_p]),
+    "fx8010_host_process_block_device_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_char_p), C.c_void_p,
+                                                          C.c_void_p, C.c_int, C.c_void_p]),
 }
 
 
@@ -341,6 +356,15 @@ class Program:
         self._check(self.L.fx8010_host_process(self.h, x.ctypes.data, out.ctypes.data, x.shape[0]), "process")
         return out
 
+    def process_block_device_curves(self, d_in, d_out, n_samples: int, curves, stream=None):
+        """FX8010::processBlockDeviceWithCurves: curves = [(register name, device tensor, broadcast)] (see Gpu.process_device_curves)."""
+        n = len(curves)
+        names = (C.c_char_p * max(1, n))(*[c[0].encode() for c in curves])
+        ptrs = (C.c_void_p * max(1, n))(*[_ptr(c[1]) for c in curves])
+        bc = (C.c_int32 * max(1, n))(*[1 if c[2] else 0 for c in curves])
+        self._check(self.L.fx8010_host_process_block_device_curves(self.h, _ptr(d_in), _ptr(d_out), n_samples, names, ptrs, bc, n, stream),
+                    "processBlockDeviceWithCurves")
+
     def process_block(self, x, n_samples=None) -> np.ndarray:
         """Batched path with host buffers: x [C][S][N] -> [C][S][N]."""
         if x is not None:
@@ -369,6 +393,22 @@ def translate_source(prog: "Program", channels: int = 1, compile_check: bool = F
     buf = C.create_string_buffer(int(n) + 1)
     cub = C.c_int(0)
     L.fx8010_translate_source(prog.image_ptr(), instances, channels, buf, int(n) + 1, 1 if compile_check else 0, C.byref(cub))
+    return buf.value.decode(), (cub.value if compile_check else None)
+
+
+def translate_source_curves(prog: "Program", curves, channels: int = 1, compile_check: bool = False, instances: int = 1):
+    """translate_source for the translation fx8010_gpu_process_batch_curves uses: curves = [(register index, broadcast)].
+    Returns (None, None) when the program is not eligible (e.g. an automated SKIP count)."""
+    L = gpu_lib()
+    k = len(curves)
+    regs = (C.c_int32 * max(1, k))(*[int(c[0]) for c in curves])
+    bc = (C.c_int32 * max(1, k))(*[1 if c[1] else 0 for c in curves])
+    n = L.fx8010_translate_source_curves(prog.image_ptr(), instances, channels, regs, bc, k, None, 0, 0, None)
+    if n < 0:
+        return None, None
+    buf = C.create_string_buffer(int(n) + 1)
+    cub = C.c_int(0)
+    L.fx8010_translate_source_curves(prog.image_ptr(), instances, channels, regs, bc, k, buf, int(n) + 1, 1 if compile_check else 0, C.byref(cub))
     return buf.value.decode(), (cub.value if compile_check else None)
 
 
@@ -466,6 +506,14 @@ class Gpu:
         self._check(self.L.fx8010_gpu_translate_status(self.h, C.byref(st), C.byref(regs), C.byref(loc), msg, 4096))
         return {"state": st.value, "regs_per_thread": regs.value, "local_bytes": loc.value, "message": msg.value.decode(errors="replace")}
 
+    def translate_status_curves(self) -> dict:
+        """translate_status for the most recent control-curve set (process_device_curves), plus the kernel kind in use (-1: none)."""
+        st, regs, loc, kind = C.c_int(0), C.c_int(0), C.c_int(0), C.c_int(-1)
+        msg = C.create_string_buffer(4096)
+        self._check(self.L.fx8010_gpu_translate_status_curves(self.h, C.byref(st), C.byref(regs), C.byref(loc), C.byref(kind), msg, 4096))
+        return {"state": st.value, "regs_per_thread": regs.value, "local_bytes": loc.value, "kind": kind.value,
+                "message": msg.value.decode(errors="replace")}
+
     def process_device_events(self, d_in, d_out, n_samples: int, events, stream=None):
         """events: iterable of (sample, reg_index, value) with value a float (broadcast) or an array of N floats."""
         arr = (CControlEvent * max(1, len(events)))()
@@ -475,6 +523,15 @@ class Gpu:
             keep.append(v)
             arr[i].sample, arr[i].reg_index, arr[i].broadcast, arr[i].values = sample, reg, int(v.size == 1), v.ctypes.data
         self._check(self.L.fx8010_gpu_process_batch_events(self.h, _ptr(d_in), _ptr(d_out), n_samples, C.addressof(arr), len(events), stream))
+
+    def process_device_curves(self, d_in, d_out, n_samples: int, curves, stream=None):
+        """curves: iterable of (reg_index, device buffer, broadcast) — [n_samples][N] float32 values, or [n_samples] with broadcast —
+        followed sample period by sample period (fx8010_gpu_process_batch_curves)."""
+        curves = list(curves)
+        arr = (CControlCurve * max(1, len(curves)))()
+        for i, (reg, vals, bc) in enumerate(curves):
+            arr[i].reg_index, arr[i].broadcast, arr[i].d_values = int(reg), 1 if bc else 0, _ptr(vals)
+        self._check(self.L.fx8010_gpu_process_batch_curves(self.h, _ptr(d_in), _ptr(d_out), n_samples, C.addressof(arr), len(curves), stream))
 
     def process_device_planar(self, d_in, d_out, n_samples: int, stream=None):
         self._check(self.L.fx8010_gpu_process_batch_planar(self.h, _ptr(d_in), _ptr(d_out), n_samples, stream))

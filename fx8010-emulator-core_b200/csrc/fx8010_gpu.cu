@@ -64,6 +64,27 @@ struct Launch { int K, B, n_seg, seg_len, grid_x; size_t smem; int M; int chunk;
 struct PlanKey { int ns = -1; unsigned align = 0; int deep = -1; int n_blk = -1; int wave = -1; };   // deep: the TRAM delays are known to allow 64-sample batches; n_blk: sample blocks per launch; wave: planned for overlap with the neighbouring launches
 enum RowClass { ROW_NONE = 0, ROW_RO, ROW_WO, ROW_RW, ROW_IN, ROW_TR };
 
+// One translation of the handle's program (fx8010_translate.inc): the plain one, or the one for a set of control curves.
+struct Translation {
+    int state = 0;                               // 0 not looked at, 1 compiling, 2 kernel loaded, -1 not eligible / failed (error says why)
+    void* fn = nullptr;                          // CUfunction of the translated kernel
+    unsigned long long key = 0; bool attached = false;     // its entry in the per-process kernel cache (reference-counted)
+    int regs = 0, local = 0;                     // its registers per thread / local-memory bytes (spills)
+    int kind = 0;                                // 0 serial kernel, 1 streaming kernel (stateless program), 2 streaming kernel with TRAM (time-cut delay line)
+    int lanes = 1;                               // (serial kernel) instances per thread
+    int ring_floats = 0;                         // (serial kernel) floats of the shared-memory input ring per thread
+    std::shared_ptr<void> job;                   // the running compilation
+    std::string error;
+    std::vector<uint8_t> folded;                 // per register: its value is an immediate of the translated kernel ...
+    std::vector<float> fold_value;               // ... namely this one
+    std::vector<int> cv_reg;                     // control curves the kernel reads (registers; empty = the plain translation) ...
+    std::vector<uint8_t> cv_bcast;               // ... and whether each is one value per period for all instances
+    bool serial = false;                         // ... and a launch of it did not fit the streaming kernel: it takes the serial kernel
+};
+
+// The curves of one call as the kernels take them (a by-value parameter of the automated translated kernels: FxtCurves there).
+struct CurveBlock { const float* p[FX8010_MAX_CONTROL_CURVES]; int bcast[FX8010_MAX_CONTROL_CURVES]; };
+
 }  // namespace
 
 struct fx8010_gpu {
@@ -162,17 +183,9 @@ struct fx8010_gpu {
     // program translator (fx8010_translate.inc)
     int tr_recurrences = 0;                      // FX8010_TR_RECUR: self-recurrence programs of the instruction-major kernel take the translated serial kernel too
     int use_translate = 1;                       // FX8010_OPT_TRANSLATE: 0 never, 1 background compile + switch when ready, 2 compile before the first launch
-    int tr_state = 0;                            // 0 not looked at, 1 compiling, 2 kernel loaded, -1 not eligible / failed (tr_error says why)
-    void* tr_fn = nullptr;                       // CUfunction of the translated kernel
-    unsigned long long tr_key = 0; bool tr_attached = false;     // its entry in the per-process kernel cache (reference-counted)
-    int tr_regs = 0, tr_local = 0;               // its registers per thread / local-memory bytes (spills)
-    int tr_kind = 0;                             // 0 serial kernel, 1 streaming kernel (stateless program), 2 streaming kernel with TRAM (time-cut delay line)
-    int tr_lanes = 1;                            // (serial kernel) instances per thread
-    int tr_ring_floats = 0;                      // (serial kernel) floats of the shared-memory input ring per thread
-    std::shared_ptr<void> tr_job;                // the running compilation
-    std::string tr_error;
-    std::vector<uint8_t> tr_folded;              // per register: its value is an immediate of the translated kernel ...
-    std::vector<float> tr_fold_value;            // ... namely this one
+    Translation tr;                              // the plain translation
+    Translation tr_cv;                           // the translation for the most recent set of control curves (fx8010_gpu_process_batch_curves)
+    const Translation* tr_gen = nullptr;         // the translation being generated: its curve registers are never folded
     std::vector<uint8_t> tr_volatile;            // per register: the host changed it after load — never folded again
     std::string err;
     fx8010_launch_info info = {};
@@ -780,6 +793,9 @@ bool use_short_kernel(const fx8010_gpu* h) {
 }
 KernelFn pick_short_kernel(int K, bool ext, int ni) { return short_kernel(K, ext, ni); }
 
+int known_tram_span(const fx8010_gpu* h);
+constexpr int MIN_TSPLIT_SPAN = 64;      // shorter spans would mean too many tiny launches: the serial kernel (with its sample split) takes those
+
 #include "fx8010_translate.inc"
 
 // Geometry of one launch: contexts per thread, block size, time split.
@@ -901,8 +917,6 @@ int known_tram_span(const fx8010_gpu* h) {
     // a ring with a WRITE but no READ stream, or a READ of a ring nobody writes, constrains nothing beyond the ring size
     return span == (1 << 30) ? 0 : span;
 }
-constexpr int MIN_TSPLIT_SPAN = 64;      // shorter spans would mean too many tiny launches: the serial kernel (with its sample split) takes those
-
 // Geometry for the stateless kernel: all the parallelism a launch needs comes from cutting the time
 // axis, so K is as wide as alignment allows and the segment count fills exactly one wave.
 int plan_stateless(fx8010_gpu* h, const float*, const float*, unsigned align, int n_samples, int n_blk, bool may_overlap, bool tsplit, Launch& L) {
@@ -1104,7 +1118,7 @@ int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, in
     if (span >= MIN_TSPLIT_SPAN && 2L * span < n_samples && tr_kind(h) == 2 && h->use_translate && h->N % 4 == 0 && (in_cs * 4) % 16 == 0 && (out_cs * 4) % 16 == 0) {
         tr_stretch = true;
         for (int b = 0; b < n_blk && tr_stretch; ++b) tr_stretch = (((uintptr_t)ins[b] | (uintptr_t)outs[b]) & 15u) == 0;
-        tr_stretch = tr_stretch && tr_ready(h);
+        tr_stretch = tr_stretch && tr_ready(h, h->tr);
     }
     const bool tsplit = span >= MIN_TSPLIT_SPAN && (2L * span >= n_samples || tr_stretch);
     if (tsplit && n_samples > span) {
@@ -1120,9 +1134,9 @@ int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, in
     // Programs of the general interpreter run on their translated kernel once it exists (fx8010_translate.inc).
     // FX8010_TR_RECUR (developer switch): bit 0 = self recurrences (cfg4), bit 1 = delay lines (cfg3) take the translated serial kernel
     const bool tr_recur = h->sl_ok && h->sl_serial && (((h->tr_recurrences & 1) && !h->sl_tram) || ((h->tr_recurrences & 2) && h->sl_tram));
-    if (!h->stateless && (tr_recur || (!(h->sl_ok && h->use_sl) && !use_short_kernel(h))) && !h->trace_mode && tr_ready(h) && tr_aligned(h, ins, outs, n_blk, in_cs, out_cs, n_samples)) {
+    if (!h->stateless && (tr_recur || (!(h->sl_ok && h->use_sl) && !use_short_kernel(h))) && !h->trace_mode && tr_ready(h, h->tr) && tr_aligned(h, h->tr, ins, outs, n_blk, in_cs, out_cs, n_samples, nullptr)) {
         for (int b = 0; b < n_blk; ++b) {
-            const int rc = tr_launch(h, ins[b], outs[b], in_cs, out_cs, n_samples, st);
+            const int rc = tr_launch(h, h->tr, ins[b], outs[b], in_cs, out_cs, n_samples, st, nullptr);
             if (rc) return rc;
             h->tram_periods += (unsigned long long)n_samples;
         }
@@ -1135,7 +1149,7 @@ int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, in
     const bool tr_delay = !h->stateless && tsplit && ns <= span && tr_kind(h) == 2;       // a time-cut launch of a delay line
     bool tr_sl = (h->stateless || tr_delay) && !h->trace_mode && h->N % 4 == 0 && (in_cs * 4) % 16 == 0 && (out_cs * 4) % 16 == 0 && ((size_t)ns * h->N * 4) % 16 == 0;
     for (int b = 0; b < n_blk && tr_sl; ++b) tr_sl = (((uintptr_t)ins[b] | (uintptr_t)outs[b]) & 15u) == 0;
-    tr_sl = tr_sl && tr_ready(h);
+    tr_sl = tr_sl && tr_ready(h, h->tr);
     for (int b0 = 0; b0 < n_blk;) {
         const int nb = (fusable || (tr_sl && h->stateless)) ? std::min(n_blk - b0, MAX_FUSED_BLOCKS) : 1;
         if (h->encode_dirty && !tr_sl) { select_tables(h); h->plan_key.ns = -1; }
@@ -1220,7 +1234,7 @@ int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, in
         cfg.attrs = attrs; cfg.numAttrs = h->use_pdl ? 1 : 0;
         const float* in = ins[b0]; float* out = outs[b0];
         if (tr_sl) {
-            const int rc = tr_sl_launch(h, ins + b0, outs + b0, nb, in_cs, out_cs, ns, st, late_wait, L);
+            const int rc = tr_sl_launch(h, h->tr, ins + b0, outs + b0, nb, in_cs, out_cs, ns, st, late_wait, L, nullptr);
             if (rc) return rc;
             h->info.last_tma = 0;
         } else if (L.M > 0) {
@@ -1323,6 +1337,67 @@ int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, in
 
 int launch_block(fx8010_gpu* h, const float* d_in, float* d_out, size_t in_cs, size_t out_cs, int n_samples, cudaStream_t st, bool own_prev = false) {
     return launch_blocks(h, &d_in, &d_out, 1, in_cs, out_cs, n_samples, st, own_prev);
+}
+
+// ---- control curves (fx8010_gpu_process_batch_curves) ----
+// A curve list the call accepts: registers in range, each named once, each a CONTROL or STATIC register.
+bool curves_valid(const std::vector<fx8010_reg>& regs, const std::vector<int>& cv_reg, std::string& why) {
+    for (size_t j = 0; j < cv_reg.size(); ++j) {
+        const int r = cv_reg[j];
+        if (r < 0 || r >= (int)regs.size()) { why = "control curve: register index out of range"; return false; }
+        if (regs[r].type != FX_REG_CONTROL && regs[r].type != FX_REG_STATIC) { why = "control curve: the register is neither CONTROL nor STATIC"; return false; }
+        for (size_t k = 0; k < j; ++k) if (cv_reg[k] == r) { why = "control curve: a register is named twice"; return false; }
+    }
+    return true;
+}
+// The curves from period s0 of the call on.
+CurveBlock curves_from(const CurveBlock& cb, int n, size_t s0, size_t N) {
+    CurveBlock r = cb;
+    for (int j = 0; j < n; ++j) r.p[j] = cb.p[j] + (cb.bcast[j] ? s0 : s0 * N);
+    return r;
+}
+struct CurveRows { CurveBlock cv; int reg[FX8010_MAX_CONTROL_CURVES]; int n; };
+// Period s of every curve into its register row: the per-period path of fx8010_gpu_process_batch_curves (grid.y = curve).
+__global__ void fx_curve_rows_kernel(float* __restrict__ gpr, const CurveRows rows, int s, int N) {
+    const int j = blockIdx.y;
+    const float* p = rows.cv.p[j];
+    float* dst = gpr + (size_t)rows.reg[j] * N;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x)
+        dst[i] = rows.cv.bcast[j] ? p[s] : p[(size_t)s * N + i];
+}
+
+// n_samples periods with the curves `cb` on the automated translation (returns 1 when the launch does not qualify: nothing queued).
+int curves_translated(fx8010_gpu* h, const float* d_in, float* d_out, size_t cs, int ns, const CurveBlock& cb, int n, cudaStream_t st) {
+    Translation& T = h->tr_cv;
+    const size_t N = (size_t)h->N;
+    if (T.kind == 0) {
+        if (!tr_aligned(h, T, &d_in, &d_out, 1, cs, cs, ns, &cb)) return 1;
+        const int rc = tr_launch(h, T, d_in, d_out, cs, cs, ns, st, &cb);
+        if (rc) return rc;
+        h->tram_periods += (unsigned long long)ns;
+        return FX8010_OK;
+    }
+    // the streaming kernel: 16-byte accesses at i0 to the samples and to the per-instance curves; a delay line is cut along time
+    bool ok = ((((uintptr_t)d_in | (uintptr_t)d_out) & 15u) == 0) && (cs * 4) % 16 == 0;
+    for (int j = 0; j < n; ++j) ok = ok && (cb.bcast[j] || ((uintptr_t)cb.p[j] & 15u) == 0);
+    const int span = T.kind == 2 ? known_tram_span(h) : ns;
+    if (!ok || span < std::min(ns, MIN_TSPLIT_SPAN)) return 1;
+    for (int s0 = 0; s0 < ns; s0 += span) {
+        const int k = std::min(span, ns - s0);
+        const float* in = d_in ? d_in + (size_t)s0 * N : nullptr;
+        float* out = d_out + (size_t)s0 * N;
+        const CurveBlock cv = curves_from(cb, n, (size_t)s0, N);
+        Launch L = {};
+        const int rc = tr_sl_launch(h, T, &in, &out, 1, cs, cs, k, st, 0, L, &cv);
+        if (rc) return rc;
+        h->tram_periods += (unsigned long long)k;
+        h->chain.clear();
+        h->info.kernel_launches++;
+        h->info.last_grid = L.grid_x * L.n_seg; h->info.last_block = L.B; h->info.last_time_split = L.n_seg; h->info.last_smem_bytes = 0;
+        h->info.last_late_wait = 0; h->info.last_fused_blocks = 1; h->info.last_tma = 0;
+        h->info.kernel_variant = (h->has_skip ? 1 : 0) | (h->has_ext ? 2 : 0) | (h->stateless ? 4 : 0) | 16 | 128 | (L.K << 8);
+    }
+    return FX8010_OK;
 }
 
 int sync_all(fx8010_gpu* h) {
@@ -1522,7 +1597,7 @@ int fx8010_gpu_load_program(fx8010_gpu* h, const fx8010_program_image* im) {
     h->reg_uniform.assign(nr, 1);
     h->reg_value.resize(nr);
     for (size_t r = 0; r < nr; ++r) h->reg_value[r] = im->regs[r].init_value;
-    h->tr_volatile.assign(nr, 0); h->tr_folded.assign(nr, 0); h->tr_fold_value.assign(nr, 0.0f);
+    h->tr_volatile.assign(nr, 0);
     tr_reset(h);
     analyse(h);
     FX_CUDA(h, cudaMalloc(&h->d_wb, sizeof(uint32_t) * std::max<size_t>(1, h->wb.size())));
@@ -1612,7 +1687,7 @@ int fx8010_gpu_set_option(fx8010_gpu* h, int option, int value) {
     if (option == FX8010_OPT_TRANSLATE) {
         if (value < 0 || value > 2) return fail(h, FX8010_ERR_ARG, "FX8010_OPT_TRANSLATE takes 0, 1 or 2");
         h->use_translate = value;
-        if (h->tr_state < 0) tr_reset(h);                    // look again (e.g. after FX8010_NVRTC was set)
+        for (Translation* T : {&h->tr, &h->tr_cv}) if (T->state < 0) tr_reset(h, *T);      // look again (e.g. after FX8010_NVRTC was set)
         return FX8010_OK;
     }
     return fail(h, FX8010_ERR_ARG, "unknown option");
@@ -1680,6 +1755,81 @@ int fx8010_gpu_process_batch_events(fx8010_gpu* h, const float* d_in, float* d_o
         if (rc) return rc;
         s0 = s1;
         if (e >= n_events && s0 >= n_samples) break;
+    }
+    return FX8010_OK;
+}
+
+int fx8010_gpu_process_batch_curves(fx8010_gpu* h, const float* d_in, float* d_out, int n_samples,
+                                    const fx8010_control_curve* curves, int n_curves, void* stream) {
+    FX_NEED_PROGRAM(h);
+    if (!d_out || n_samples < 0 || n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && !curves))
+        return fail(h, FX8010_ERR_ARG, "d_out or the curve list is NULL, n_samples negative, or the curve count outside 0..8");
+    std::vector<int> regs((size_t)n_curves);
+    std::vector<uint8_t> bc((size_t)n_curves);
+    CurveRows rows = {};
+    rows.n = n_curves;
+    for (int j = 0; j < n_curves; ++j) {
+        if (!curves[j].d_values) return fail(h, FX8010_ERR_ARG, "control curve: d_values is NULL");
+        regs[j] = rows.reg[j] = curves[j].reg_index;
+        bc[j] = curves[j].broadcast ? 1 : 0;
+        rows.cv.p[j] = curves[j].d_values; rows.cv.bcast[j] = bc[j];
+    }
+    {
+        std::string why;
+        if (!curves_valid(h->regs, regs, why)) return fail(h, FX8010_ERR_ARG, why);
+    }
+    if (n_samples == 0) return FX8010_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t N = (size_t)h->N, cs = (size_t)n_samples * N;
+    if (n_curves == 0) return launch_block(h, d_in, d_out, cs, cs, n_samples, st);
+    {
+        const int rc = order_on(h, st);
+        if (rc) return rc;
+    }
+    h->chain.clear();                 // every launch of the call waits for its predecessor at its start: a curve may be earlier work's output
+    // While the call runs the automated registers hold no one value: nothing may fold them (interpreter encoding, plain translation — a
+    // folded STATIC voids it, once).  Afterwards they hold the last period's values, which the host does not know: still not uniform.
+    for (int r : regs) {
+        h->reg_uniform[r] = 0;
+        if (h->enc_sensitive[r]) h->encode_dirty = true;
+        tr_touch(h, r);
+    }
+    if (h->tr_cv.cv_reg != regs || h->tr_cv.cv_bcast != bc) {
+        tr_reset(h, h->tr_cv);
+        h->tr_cv.cv_reg = regs; h->tr_cv.cv_bcast = bc; h->tr_cv.serial = false;
+    }
+    // per-launch executed-instruction counters are 32-bit: very long batches in pieces (as launch_blocks does)
+    const long long per_sample = (long long)h->instrs.size() * FX8010_MAX_PASSES;
+    const int max_samples = (int)std::max<long long>(1, std::min<long long>(0x7fffffffLL, 0xffffffffLL / per_sample));
+    for (int s0 = 0; s0 < n_samples; s0 += max_samples) {
+        const int ns = std::min(max_samples, n_samples - s0);
+        const float* in = d_in ? d_in + (size_t)s0 * N : nullptr;
+        float* out = d_out + (size_t)s0 * N;
+        const CurveBlock cv = curves_from(rows.cv, n_curves, (size_t)s0, N);
+        if (!h->trace_mode && tr_ready(h, h->tr_cv)) {
+            int rc = curves_translated(h, in, out, cs, ns, cv, n_curves, st);
+            if (rc == 1 && h->tr_cv.kind != 0) {
+                // The streaming kernel does not fit this launch (a buffer not 16-byte aligned, a delay line whose span is no longer known):
+                // from now on this curve set takes the serial kernel, which does not need either.
+                h->tr_cv.serial = true;
+                tr_reset(h, h->tr_cv);
+                rc = tr_ready(h, h->tr_cv) ? curves_translated(h, in, out, cs, ns, cv, n_curves, st) : 1;
+            }
+            if (rc == FX8010_OK) continue;
+            if (rc != 1) return rc;
+        }
+        // Per-period path (correctness, not speed): no translated kernel for this curve set, or the launch does not qualify.  Each period
+        // is one copy of the curves' values into the register rows and one ordinary one-period launch.
+        CurveRows r1 = rows;
+        r1.cv = cv;
+        for (int s = 0; s < ns; ++s) {
+            fx_curve_rows_kernel<<<dim3((unsigned)std::min<size_t>(1024, (N + 255) / 256), (unsigned)n_curves), 256, 0, st>>>(h->d_gpr, r1, s, (int)N);
+            h->info.kernel_launches++;
+            FX_CUDA(h, cudaGetLastError());
+            h->chain.clear();
+            const int rc = launch_block(h, in ? in + (size_t)s * N : nullptr, out + (size_t)s * N, cs, cs, 1, st);
+            if (rc) return rc;
+        }
     }
     return FX8010_OK;
 }
@@ -2006,19 +2156,30 @@ int fx8010_gpu_trace(fx8010_gpu* h, const float* in, float* out, int n_samples, 
 }
 
 // ---- program translator: status and the host-only source generator (tests/test_translate.py) ----
-int fx8010_gpu_translate_status(fx8010_gpu* h, int* state, int* regs_per_thread, int* local_bytes, char* message, size_t message_cap) {
-    if (!h) return FX8010_ERR_ARG;
-    if (h->tr_state == 1 && h->loaded && cudaSetDevice(h->device) == cudaSuccess) tr_ready(h);   // pick up a finished background compilation (the kernel loads into this device's context)
-    if (state) *state = h->tr_state;
-    if (regs_per_thread) *regs_per_thread = h->tr_regs;
-    if (local_bytes) *local_bytes = h->tr_local;
-    if (message && message_cap) { strncpy(message, h->tr_error.c_str(), message_cap - 1); message[message_cap - 1] = 0; }
+static int translate_status(fx8010_gpu* h, Translation& T, int* state, int* regs_per_thread, int* local_bytes, char* message, size_t message_cap) {
+    if (T.state == 1 && h->loaded && cudaSetDevice(h->device) == cudaSuccess) tr_ready(h, T);   // pick up a finished background compilation (the kernel loads into this device's context)
+    if (state) *state = T.state;
+    if (regs_per_thread) *regs_per_thread = T.regs;
+    if (local_bytes) *local_bytes = T.local;
+    if (message && message_cap) { strncpy(message, T.error.c_str(), message_cap - 1); message[message_cap - 1] = 0; }
     return FX8010_OK;
 }
+int fx8010_gpu_translate_status(fx8010_gpu* h, int* state, int* regs_per_thread, int* local_bytes, char* message, size_t message_cap) {
+    if (!h) return FX8010_ERR_ARG;
+    return translate_status(h, h->tr, state, regs_per_thread, local_bytes, message, message_cap);
+}
+int fx8010_gpu_translate_status_curves(fx8010_gpu* h, int* state, int* regs_per_thread, int* local_bytes, int* kind, char* message, size_t message_cap) {
+    if (!h) return FX8010_ERR_ARG;
+    if (kind) *kind = h->tr_cv.state == 2 ? h->tr_cv.kind : -1;
+    return translate_status(h, h->tr_cv, state, regs_per_thread, local_bytes, message, message_cap);
+}
 
-// Needs no device: analyses the image as load_program would and returns the CUDA source of its translated kernel.
-long long fx8010_translate_source(const fx8010_program_image* im, int n_instances, int n_channels, char* buf, size_t cap, int compile_check, int* regs_or_status) {
+// Needs no device: analyses the image as load_program would and returns the CUDA source of its translated kernel (for control curves
+// on cregs[n_curves] when n_curves > 0).
+static long long translate_source_impl(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
+                                       int n_curves, char* buf, size_t cap, int compile_check, int* regs_or_status) {
     if (!im || !im->instrs || !im->regs || im->n_instrs <= 0 || im->n_regs <= 0 || n_channels <= 0 || n_instances <= 0) return -1;
+    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && (!cregs || !cbcast))) return -1;
     fx8010_gpu tmp;
     tmp.C = n_channels; tmp.N = n_instances;
     tmp.instrs.assign(im->instrs, im->instrs + im->n_instrs);
@@ -2027,16 +2188,23 @@ long long fx8010_translate_source(const fx8010_program_image* im, int n_instance
         if (in.opcode < 0 || in.opcode >= FX_NUM_OPCODES || in.r < 0 || in.r >= im->n_regs || in.a < 0 || in.a >= im->n_regs ||
             in.x < 0 || in.x >= im->n_regs || in.y < 0 || in.y >= im->n_regs) return -1;
     for (const fx8010_reg& r : tmp.regs) if (r.io_index < 0 || r.io_index >= n_channels) return -1;
+    Translation T;
+    for (int j = 0; j < n_curves; ++j) { T.cv_reg.push_back(cregs[j]); T.cv_bcast.push_back(cbcast[j] ? 1 : 0); }
+    std::string why;
+    if (!curves_valid(tmp.regs, T.cv_reg, why)) return -1;
     tmp.itram_size = im->itram_size; tmp.xtram_size = im->xtram_size;
     tmp.reg_uniform.assign(im->n_regs, 1);
     tmp.reg_value.resize(im->n_regs);
     for (int r = 0; r < im->n_regs; ++r) tmp.reg_value[r] = im->regs[r].init_value;
+    for (int r : T.cv_reg) tmp.reg_uniform[r] = 0;            // (as fx8010_gpu_process_batch_curves leaves them)
     tmp.tr_volatile.assign(im->n_regs, 0);
     analyse(&tmp);
-    const int kind = (tr_kind(&tmp) == 2 && known_tram_span(&tmp) < MIN_TSPLIT_SPAN) ? 0 : tr_kind(&tmp);
+    const int kind = n_curves ? tr_kind_curves(&tmp, T) : ((tr_kind(&tmp) == 2 && known_tram_span(&tmp) < MIN_TSPLIT_SPAN) ? 0 : tr_kind(&tmp));
+    tmp.tr_gen = n_curves ? &T : nullptr;
     if (kind == 0 && !tr_eligible(&tmp)) return -2;
     std::vector<uint8_t> folded;
     const std::string src = kind ? tr_generate_sl(&tmp, folded, kind == 2) : tr_generate(&tmp, folded);
+    tmp.tr_gen = nullptr;
     if (buf && cap) { strncpy(buf, src.c_str(), cap - 1); buf[cap - 1] = 0; }
     if (compile_check) {                                     // NVRTC -> sm_100a CUBIN (works without a GPU)
         std::vector<char> cubin; std::string log;
@@ -2045,6 +2213,13 @@ long long fx8010_translate_source(const fx8010_program_image* im, int n_instance
         if (!ok) fprintf(stderr, "fx8010_translate_source: %s\n", log.c_str());
     }
     return (long long)src.size();
+}
+long long fx8010_translate_source(const fx8010_program_image* im, int n_instances, int n_channels, char* buf, size_t cap, int compile_check, int* regs_or_status) {
+    return translate_source_impl(im, n_instances, n_channels, nullptr, nullptr, 0, buf, cap, compile_check, regs_or_status);
+}
+long long fx8010_translate_source_curves(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* regs, const int32_t* broadcast,
+                                         int n_curves, char* buf, size_t cap, int compile_check, int* cubin_bytes) {
+    return translate_source_impl(im, n_instances, n_channels, regs, broadcast, n_curves, buf, cap, compile_check, cubin_bytes);
 }
 
 const char* fx8010_gpu_last_error(fx8010_gpu* h) { return h ? h->err.c_str() : g_create_error.c_str(); }

@@ -120,6 +120,18 @@ void FX8010::processBlockDeviceWithControls(const float* d_in, float* d_out, int
     check(fx8010_gpu_process_batch_events(gpu_, d_in, d_out, n_samples, ev.data(), (int)ev.size(), stream), "process_batch_events");
 }
 
+void FX8010::processBlockDeviceWithCurves(const float* d_in, float* d_out, int n_samples, const std::vector<Curve>& curves, void* stream) {
+    ensureUploaded();
+    if (multi_) throw std::runtime_error("FX8010 (B200): device-pointer members need a single device");
+    std::vector<fx8010_control_curve> cv;
+    for (const Curve& c : curves) {
+        const int reg = front_.findRegister(c.key);
+        if (reg < 0) throw std::runtime_error("FX8010: unknown register '" + c.key + "'");
+        cv.push_back(fx8010_control_curve{reg, c.broadcast ? 1 : 0, c.d_values});
+    }
+    check(fx8010_gpu_process_batch_curves(gpu_, d_in, d_out, n_samples, cv.data(), (int)cv.size(), stream), "process_batch_curves");
+}
+
 void FX8010::processBlockDevicePlanar(const float* d_in, float* d_out, int n_samples, void* stream) {
     ensureUploaded();
     if (multi_) throw std::runtime_error("FX8010 (B200): device-pointer members need a single device");

@@ -71,6 +71,11 @@ public:
     struct ControlChange { int sample; std::string key; float value; };
     void processBlockDeviceWithControls(const float* d_in, float* d_out, int n_samples,
                                         const std::vector<ControlChange>& changes, void* stream);
+    // sample-accurate automation (include/fx8010_gpu.h, fx8010_gpu_process_batch_curves): register `key` takes d_values[s] (broadcast: one
+    // value for every instance, d_values[n_samples]) or d_values[s * numInstances + i] (d_values[n_samples][numInstances]) right before
+    // sample period s; DEVICE buffers, asynchronous on `stream`; throws on an unknown name
+    struct Curve { std::string key; const float* d_values; bool broadcast; };
+    void processBlockDeviceWithCurves(const float* d_in, float* d_out, int n_samples, const std::vector<Curve>& curves, void* stream);
     // DEVICE buffers laid out [channel][instance][sample] (planar audio), asynchronous on `stream`
     void processBlockDevicePlanar(const float* d_in, float* d_out, int n_samples, void* stream);
     // program translator (include/fx8010_gpu.h, FX8010_OPT_TRANSLATE): 0 interpreter kernels only, 1 compile in the background and switch

@@ -119,6 +119,14 @@ int fx8010_host_process(fx8010_host* h, const float* in, float* out, int n_sampl
 int fx8010_host_process_block(fx8010_host* h, const float* in, float* out, int n_samples) {
     return guarded(h, [&] { h->fx.processBlock(in, out, n_samples); });
 }
+int fx8010_host_process_block_device_curves(fx8010_host* h, const float* d_in, float* d_out, int n_samples, const char* const* names,
+                                            const float* const* d_values, const int* broadcast, int n_curves, void* stream) {
+    return guarded(h, [&] {
+        std::vector<Klangraum::FX8010::Curve> cv;
+        for (int j = 0; j < n_curves; ++j) cv.push_back(Klangraum::FX8010::Curve{names[j], d_values[j], broadcast[j] != 0});
+        h->fx.processBlockDeviceWithCurves(d_in, d_out, n_samples, cv, stream);
+    });
+}
 int fx8010_host_instruction_counter(fx8010_host* h) {
     int v = 0;
     guarded(h, [&] { v = h->fx.getInstructionCounter(); });

@@ -212,6 +212,25 @@ typedef struct fx8010_control_event {
 FX8010_API int fx8010_gpu_process_batch_events(fx8010_gpu* h, const float* d_in, float* d_out, int n_samples,
                                                const fx8010_control_event* events, int n_events, void* stream);
 
+/* Sample-accurate automation: one control value per sample period (fades, filter sweeps, a host's LFO) without cutting the batch. */
+#define FX8010_MAX_CONTROL_CURVES 8
+typedef struct fx8010_control_curve {
+    int32_t reg_index;     /* a CONTROL or STATIC register                                                 */
+    int32_t broadcast;     /* 0: d_values is [n_samples][n_instances]; != 0: [n_samples], one value for all */
+    const float* d_values; /* DEVICE pointer, float32                                                      */
+} fx8010_control_curve;
+/* fx8010_gpu_process_batch with up to FX8010_MAX_CONTROL_CURVES registers following curves: equivalent, bit for bit in outputs and
+ * in the final state, to `for s in 0..n_samples-1: set_controls(reg_j, curve_j[s]) for every j; process_batch(1 period)` — and to
+ * process_batch_events with one event per curve at every period.  An automated register ends holding its last curve value, or what
+ * the program itself wrote to it in the last period.  The curves are read on the device while the block runs (FX8010_OPT_TRANSLATE
+ * != 0: inside the translated kernels, fx8010_launch_info.kernel_variant bit 4 set); without a translated kernel for the curve set
+ * (mode 0, no libnvrtc, still compiling in mode 1, a SKIP count automated, unaligned buffers) the call runs one sample period per
+ * launch: correct, but slow.  A curve buffer may be the output of earlier work on `stream` (another handle's output, say): the
+ * call's first launch waits for everything before it.  FX8010_ERR_ARG, with nothing queued, for more than 8 curves or a negative
+ * count, a NULL list or d_values, a register out of range, named twice, or neither CONTROL nor STATIC. */
+FX8010_API int fx8010_gpu_process_batch_curves(fx8010_gpu* h, const float* d_in, float* d_out, int n_samples,
+                                               const fx8010_control_curve* curves, int n_curves, void* stream);
+
 /* fx8010_gpu_process_batch for PLANAR audio buffers, as an audio host keeps them: DEVICE pointers,
  * [n_channels][n_instances][n_samples] float32 (one contiguous block of samples per instance and channel).
  * The [sample][instance] layout the interpreter streams is produced and undone by tiled transposes on `stream`. */
@@ -283,12 +302,21 @@ FX8010_API int fx8010_gpu_trace(fx8010_gpu* h, const float* in, float* out, int 
  * describe the loaded kernel.  Any pointer may be NULL. */
 FX8010_API int fx8010_gpu_translate_status(fx8010_gpu* h, int* state, int* regs_per_thread, int* local_bytes,
                                            char* message, size_t message_cap);
+/* The same for the translation of the most recent control-curve set (fx8010_gpu_process_batch_curves): state 0 also before any curve
+ * call; -1 with the reason (e.g. an automated SKIP count) when the calls run one launch per period.  kind: 0 serial kernel, 1 streaming
+ * kernel, 2 streaming kernel cut along time, -1 none loaded. */
+FX8010_API int fx8010_gpu_translate_status_curves(fx8010_gpu* h, int* state, int* regs_per_thread, int* local_bytes, int* kind,
+                                                  char* message, size_t message_cap);
 /* The CUDA source the translator generates for an image on n_instances instances (no device needed; a test and inspection aid — the generated
  * source also compiles as plain C++ with -DFXT_HOST_CHECK, which is how tests/test_translate.py checks it on the CPU).
  * Returns the source length (copied, truncated, into buf when given), -1 for a bad image, -2 when the program is not
  * eligible.  compile_check != 0 also runs NVRTC for sm_100a and stores the CUBIN size (or -1) in *cubin_bytes. */
 FX8010_API long long fx8010_translate_source(const fx8010_program_image* image, int n_instances, int n_channels, char* buf, size_t cap,
                                              int compile_check, int* cubin_bytes);
+/* Same for the translation fx8010_gpu_process_batch_curves uses for curves on registers regs[n_curves] (broadcast[j] != 0: one value
+ * per period for all instances).  With n_curves == 0 it is fx8010_translate_source.  -1 also for a curve list the call would reject. */
+FX8010_API long long fx8010_translate_source_curves(const fx8010_program_image* image, int n_instances, int n_channels, const int32_t* regs,
+                                                    const int32_t* broadcast, int n_curves, char* buf, size_t cap, int compile_check, int* cubin_bytes);
 
 /* Text of the last error on this handle (or of the last failed create when h == NULL). */
 FX8010_API const char* fx8010_gpu_last_error(fx8010_gpu* h);
@@ -302,7 +330,7 @@ typedef struct fx8010_launch_info {
     int32_t last_fused_blocks;            /* sample blocks the last launch covered (fx8010_gpu_process_blocks) */
     int32_t last_tma;                     /* the last launch staged its input with bulk tensor copies (TMA) */
     int32_t reserved;
-    int32_t kernel_variant;               /* bit0 SKIP, bit1 TRAM/noise/MACMV, bit2 stateless, bit3 instruction-major kernel, bit5 short-program kernel, bit6 producer/consumer pairs fused, bit7 translated kernel (FX8010_OPT_TRANSLATE), bits 8..15 instances per thread, bits 16.. samples per batch */
+    int32_t kernel_variant;               /* bit0 SKIP, bit1 TRAM/noise/MACMV, bit2 stateless, bit3 instruction-major kernel, bit4 control curves read inside the kernel (fx8010_gpu_process_batch_curves), bit5 short-program kernel, bit6 producer/consumer pairs fused, bit7 translated kernel (FX8010_OPT_TRANSLATE), bits 8..15 instances per thread, bits 16.. samples per batch */
 } fx8010_launch_info;
 FX8010_API int fx8010_gpu_get_launch_info(fx8010_gpu* h, fx8010_launch_info* out);
 

@@ -61,6 +61,9 @@ FX8010_API int fx8010_host_get_register_values(fx8010_host* h, const char* name,
 FX8010_API int fx8010_host_process(fx8010_host* h, const float* in, float* out, int n_samples);
 /* processBlock(): host buffers [channel][sample][instance] */
 FX8010_API int fx8010_host_process_block(fx8010_host* h, const float* in, float* out, int n_samples);
+/* processBlockDeviceWithCurves(): DEVICE buffers, curve j drives register names[j] (d_values[j], broadcast[j]: see fx8010_gpu_process_batch_curves) */
+FX8010_API int fx8010_host_process_block_device_curves(fx8010_host* h, const float* d_in, float* d_out, int n_samples, const char* const* names,
+                                                       const float* const* d_values, const int* broadcast, int n_curves, void* stream);
 FX8010_API int fx8010_host_instruction_counter(fx8010_host* h);                 /* getInstructionCounter */
 FX8010_API unsigned long long fx8010_host_instruction_counter_total(fx8010_host* h);
 FX8010_API fx8010_gpu* fx8010_host_gpu(fx8010_host* h);                          /* NULL on failure */
