@@ -74,6 +74,11 @@ class CLaunchInfo(C.Structure):
                 ("last_fused_blocks", C.c_int32), ("last_tma", C.c_int32), ("reserved", C.c_int32), ("kernel_variant", C.c_int32)]
 
 
+class CKernelCacheStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("nvrtc_compiles", "memory_hits", "store_hits", "joined_compiles", "disk_hits", "disk_writes",
+                                          "disk_rejected", "disk_write_failures")]
+
+
 TRACE_DTYPE = np.dtype([("index", np.int32), ("executed", np.int32), ("r", np.float32), ("a", np.float32), ("x", np.float32),
                         ("y", np.float32), ("ccr", np.float32), ("opcode", np.int32), ("acc", np.float64)])
 
@@ -127,6 +132,9 @@ GPU_SYMBOLS = {
     "fx8010_gpu_process_batch_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "fx8010_translate_source_curves": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_char_p, C.c_size_t,
                                                       C.c_int, C.POINTER(C.c_int)]),
+    "fx8010_kernel_cache_set_dir": (C.c_int, [C.c_char_p]),
+    "fx8010_kernel_cache_precompile": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "fx8010_kernel_cache_get_stats": (C.c_int, [C.POINTER(CKernelCacheStats)]),
 }
 
 MULTI_SYMBOLS = {
@@ -159,6 +167,7 @@ HOST_SYMBOLS = {
     "fx8010_host_ready": (C.c_int, [C.c_void_p]),
     "fx8010_host_set_relaxed": (None, [C.c_void_p, C.c_int]),
     "fx8010_host_set_translation": (C.c_int, [C.c_void_p, C.c_int]),
+    "fx8010_host_set_kernel_cache_dir": (None, [C.c_char_p]),
     "fx8010_host_num_registers": (C.c_int, [C.c_void_p]),
     "fx8010_host_register_info": (None, [C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_float),
                                          C.POINTER(C.c_int), C.c_char_p, C.c_int]),
@@ -410,6 +419,29 @@ def translate_source_curves(prog: "Program", curves, channels: int = 1, compile_
     cub = C.c_int(0)
     L.fx8010_translate_source_curves(prog.image_ptr(), instances, channels, regs, bc, k, buf, int(n) + 1, 1 if compile_check else 0, C.byref(cub))
     return buf.value.decode(), (cub.value if compile_check else None)
+
+
+def set_kernel_cache_dir(path) -> None:
+    """Directory of the translator's disk kernel cache for the whole process (overrides FX8010_KERNEL_CACHE); None or "" turns it off."""
+    gpu_lib().fx8010_kernel_cache_set_dir(os.fsencode(path) if path else None)
+
+
+def kernel_cache_stats() -> dict:
+    """Process-wide kernel cache counters (fx8010_kernel_cache_stats)."""
+    st = CKernelCacheStats()
+    gpu_lib().fx8010_kernel_cache_get_stats(C.byref(st))
+    return {name: int(getattr(st, name)) for name, _ in CKernelCacheStats._fields_}
+
+
+def precompile(prog: "Program", instances: int, channels: int = 1, curves=None) -> int:
+    """Compile the translated kernel a handle of `instances` instances would use for `prog` (curves = [(register index, broadcast)] for
+    the control-curve translation) into the disk kernel cache, without a device.  Returns fx8010_kernel_cache_precompile's code:
+    0 written, 1 already there, -1 bad arguments, -2 not eligible, -3 no cache directory, -4 compile failed, -5 write failed."""
+    curves = curves or []
+    k = len(curves)
+    regs = (C.c_int32 * max(1, k))(*[int(c[0]) for c in curves])
+    bc = (C.c_int32 * max(1, k))(*[1 if c[1] else 0 for c in curves])
+    return gpu_lib().fx8010_kernel_cache_precompile(prog.image_ptr(), instances, channels, regs, bc, k)
 
 
 class Gpu:

@@ -8,9 +8,14 @@
 #include <cuda.h>            // CUtensorMap and its enums only: cuTensorMapEncodeTiled is resolved at run time (no libcuda link)
 #include <cuda_runtime.h>
 
+#include <dirent.h>
 #include <dlfcn.h>
+#include <fcntl.h>
+#include <sys/stat.h>
+#include <unistd.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <cmath>
@@ -64,11 +69,13 @@ struct Launch { int K, B, n_seg, seg_len, grid_x; size_t smem; int M; int chunk;
 struct PlanKey { int ns = -1; unsigned align = 0; int deep = -1; int n_blk = -1; int wave = -1; };   // deep: the TRAM delays are known to allow 64-sample batches; n_blk: sample blocks per launch; wave: planned for overlap with the neighbouring launches
 enum RowClass { ROW_NONE = 0, ROW_RO, ROW_WO, ROW_RW, ROW_IN, ROW_TR };
 
+typedef std::array<uint8_t, 32> KernelDigest;    // SHA-256 identity of a translated kernel (fx8010_translate.inc)
+
 // One translation of the handle's program (fx8010_translate.inc): the plain one, or the one for a set of control curves.
 struct Translation {
     int state = 0;                               // 0 not looked at, 1 compiling, 2 kernel loaded, -1 not eligible / failed (error says why)
     void* fn = nullptr;                          // CUfunction of the translated kernel
-    unsigned long long key = 0; bool attached = false;     // its entry in the per-process kernel cache (reference-counted)
+    KernelDigest key{}; bool attached = false;   // its entry in the per-process kernel cache (reference-counted)
     int regs = 0, local = 0;                     // its registers per thread / local-memory bytes (spills)
     int kind = 0;                                // 0 serial kernel, 1 streaming kernel (stateless program), 2 streaming kernel with TRAM (time-cut delay line)
     int lanes = 1;                               // (serial kernel) instances per thread
@@ -187,6 +194,7 @@ struct fx8010_gpu {
     Translation tr_cv;                           // the translation for the most recent set of control curves (fx8010_gpu_process_batch_curves)
     const Translation* tr_gen = nullptr;         // the translation being generated: its curve registers are never folded
     std::vector<uint8_t> tr_volatile;            // per register: the host changed it after load — never folded again
+    std::string kc_env_dir;                      // FX8010_KERNEL_CACHE when the handle was created (the disk store; "" = none)
     std::string err;
     fx8010_launch_info info = {};
 };
@@ -1467,6 +1475,7 @@ int fx8010_gpu_create(int device, int n_instances, int n_channels, fx8010_gpu** 
     if (getenv("FX8010_NO_TRAM_IM")) h->use_tram_im = 0;
     if (getenv("FX8010_NO_SPLIT")) h->use_split = 0;
     if (getenv("FX8010_TR_RECUR")) h->tr_recurrences = atoi(getenv("FX8010_TR_RECUR"));
+    h->kc_env_dir = kc_env_dir();
     if (getenv("FX8010_TRANSLATE")) h->use_translate = std::min(2, std::max(0, atoi(getenv("FX8010_TRANSLATE"))));
     h->tune_P = env_int("FX8010_TUNE_P");
     h->tune_M = env_int("FX8010_TUNE_M");
@@ -2157,7 +2166,7 @@ int fx8010_gpu_trace(fx8010_gpu* h, const float* in, float* out, int n_samples, 
 
 // ---- program translator: status and the host-only source generator (tests/test_translate.py) ----
 static int translate_status(fx8010_gpu* h, Translation& T, int* state, int* regs_per_thread, int* local_bytes, char* message, size_t message_cap) {
-    if (T.state == 1 && h->loaded && cudaSetDevice(h->device) == cudaSuccess) tr_ready(h, T);   // pick up a finished background compilation (the kernel loads into this device's context)
+    if (T.state == 1 && h->loaded && cudaSetDevice(h->device) == cudaSuccess) tr_ready(h, T, false);   // pick up a finished background compilation (the kernel loads into this device's context)
     if (state) *state = T.state;
     if (regs_per_thread) *regs_per_thread = T.regs;
     if (local_bytes) *local_bytes = T.local;
@@ -2174,10 +2183,13 @@ int fx8010_gpu_translate_status_curves(fx8010_gpu* h, int* state, int* regs_per_
     return translate_status(h, h->tr_cv, state, regs_per_thread, local_bytes, message, message_cap);
 }
 
-// Needs no device: analyses the image as load_program would and returns the CUDA source of its translated kernel (for control curves
-// on cregs[n_curves] when n_curves > 0).
-static long long translate_source_impl(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
-                                       int n_curves, char* buf, size_t cap, int compile_check, int* regs_or_status) {
+// Needs no device: analyses the image as load_program would and generates the CUDA source of its translated kernel (for control curves
+// on cregs[n_curves] when n_curves > 0) into `src`.  0, -1 for a bad image or curve list, -2 when the program is not eligible.
+// For a freshly loaded image this is the source a handle generates at its first launch on a B200 (148 SMs), with one exception: a delay
+// line whose known span is below MIN_TSPLIT_SPAN gets the serial kernel here, where a handle runs the interpreter kernels and never asks;
+// and the developer switches a handle reads when it is created (FX8010_NO_STATELESS, FX8010_NO_TSPLIT, FX8010_TR_RECUR) are not applied.
+static int translate_source_gen(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
+                                int n_curves, std::string& src) {
     if (!im || !im->instrs || !im->regs || im->n_instrs <= 0 || im->n_regs <= 0 || n_channels <= 0 || n_instances <= 0) return -1;
     if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && (!cregs || !cbcast))) return -1;
     fx8010_gpu tmp;
@@ -2203,8 +2215,15 @@ static long long translate_source_impl(const fx8010_program_image* im, int n_ins
     tmp.tr_gen = n_curves ? &T : nullptr;
     if (kind == 0 && !tr_eligible(&tmp)) return -2;
     std::vector<uint8_t> folded;
-    const std::string src = kind ? tr_generate_sl(&tmp, folded, kind == 2) : tr_generate(&tmp, folded);
+    src = kind ? tr_generate_sl(&tmp, folded, kind == 2) : tr_generate(&tmp, folded);
     tmp.tr_gen = nullptr;
+    return 0;
+}
+static long long translate_source_impl(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
+                                       int n_curves, char* buf, size_t cap, int compile_check, int* regs_or_status) {
+    std::string src;
+    const int g = translate_source_gen(im, n_instances, n_channels, cregs, cbcast, n_curves, src);
+    if (g) return g;
     if (buf && cap) { strncpy(buf, src.c_str(), cap - 1); buf[cap - 1] = 0; }
     if (compile_check) {                                     // NVRTC -> sm_100a CUBIN (works without a GPU)
         std::vector<char> cubin; std::string log;
@@ -2220,6 +2239,26 @@ long long fx8010_translate_source(const fx8010_program_image* im, int n_instance
 long long fx8010_translate_source_curves(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* regs, const int32_t* broadcast,
                                          int n_curves, char* buf, size_t cap, int compile_check, int* cubin_bytes) {
     return translate_source_impl(im, n_instances, n_channels, regs, broadcast, n_curves, buf, cap, compile_check, cubin_bytes);
+}
+
+int fx8010_kernel_cache_set_dir(const char* dir) {
+    std::lock_guard<std::mutex> lk(g_kc_dir_mutex);
+    g_kc_dir_set = true;
+    g_kc_dir = dir ? dir : "";
+    return FX8010_OK;
+}
+int fx8010_kernel_cache_precompile(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* regs, const int32_t* broadcast,
+                                   int n_curves) {
+    std::string src;
+    const int g = translate_source_gen(im, n_instances, n_channels, regs, broadcast, n_curves, src);
+    return g ? g : kc_precompile(src);
+}
+int fx8010_kernel_cache_get_stats(fx8010_kernel_cache_stats* out) {
+    if (!out) return FX8010_ERR_ARG;
+    out->nvrtc_compiles = g_kc.nvrtc_compiles; out->memory_hits = g_kc.memory_hits; out->store_hits = g_kc.store_hits;
+    out->joined_compiles = g_kc.joined_compiles; out->disk_hits = g_kc.disk_hits; out->disk_writes = g_kc.disk_writes;
+    out->disk_rejected = g_kc.disk_rejected; out->disk_write_failures = g_kc.disk_write_failures;
+    return FX8010_OK;
 }
 
 const char* fx8010_gpu_last_error(fx8010_gpu* h) { return h ? h->err.c_str() : g_create_error.c_str(); }

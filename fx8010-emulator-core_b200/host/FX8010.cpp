@@ -78,6 +78,8 @@ void FX8010::setTranslation(int mode) {
     translate_mode_ = mode;                                     // applied by the next process* call (ensureUploaded)
 }
 
+void FX8010::setKernelCacheDir(const std::string& dir) { fx8010_kernel_cache_set_dir(dir.c_str()); }
+
 std::vector<float> FX8010::process(const std::vector<float>& inputSamples) {
     ensureUploaded();
     const size_t C = (size_t)front_.channels(), N = (size_t)instances_;

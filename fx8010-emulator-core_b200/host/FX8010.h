@@ -81,6 +81,9 @@ public:
     // program translator (include/fx8010_gpu.h, FX8010_OPT_TRANSLATE): 0 interpreter kernels only, 1 compile in the background and switch
     // over when the kernel is loaded (default), 2 compile before the first block
     void setTranslation(int mode);
+    // the translator's disk kernel cache for the whole process (include/fx8010_gpu.h, fx8010_kernel_cache_set_dir): translated kernels
+    // compiled once are reused by later processes; "" turns it off (it is off unless FX8010_KERNEL_CACHE names a directory)
+    static void setKernelCacheDir(const std::string& dir);
     unsigned long long getInstructionCounterTotal();           // summed over instances
     fx8010_gpu* gpuHandle();                                   // creates the handle / uploads the program if needed
     fx8010::Frontend& frontend() { return front_; }

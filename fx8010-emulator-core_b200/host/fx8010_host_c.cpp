@@ -45,6 +45,7 @@ void fx8010_host_set_relaxed(fx8010_host* h, int on) { h->fx.setRelaxedSyntax(on
 int fx8010_host_set_translation(fx8010_host* h, int mode) {
     try { h->fx.setTranslation(mode); return 0; } catch (...) { return 1; }
 }
+void fx8010_host_set_kernel_cache_dir(const char* dir) { Klangraum::FX8010::setKernelCacheDir(dir ? dir : ""); }
 int fx8010_host_ready(fx8010_host* h) { return h->fx.getReadyStatus() ? 1 : 0; }
 
 int fx8010_host_num_registers(fx8010_host* h) { return (int)h->fx.frontend().registers().size(); }

@@ -318,6 +318,50 @@ FX8010_API long long fx8010_translate_source(const fx8010_program_image* image, 
 FX8010_API long long fx8010_translate_source_curves(const fx8010_program_image* image, int n_instances, int n_channels, const int32_t* regs,
                                                     const int32_t* broadcast, int n_curves, char* buf, size_t cap, int compile_check, int* cubin_bytes);
 
+/* ---- kernel cache of the program translator ----------------------------------------------------------------------------
+ * A translated kernel is named by SHA-256 over these bytes, concatenated: "fx8010-kernel-v1\n", "sm_100a\n", each NVRTC option
+ * followed by "\n" ("--gpu-architecture=sm_100a", "--std=c++17", "--fmad=false", "--ftz=false", "--prec-div=true", "--prec-sqrt=true",
+ * "-lineinfo", "-default-device", in this order), "nvrtc <major>.<minor>\n" (nvrtcVersion), then the generated source exactly as
+ * fx8010_translate_source(_curves) returns it.  A handle looks its kernel up, at the first launch that can use it, in this order:
+ *   1. the module already loaded on its device (another handle with the same program);
+ *   2. the process-wide CUBIN store, or a compile of the same source already in flight, which it joins (one compile per process,
+ *      whatever the number of handles and devices; in mode 1 the handle runs the interpreter kernels until that compile ends);
+ *   3. the disk store, when a directory is set;
+ *   4. NVRTC, then the process store and the disk store.
+ * Steps 1-3 need no libnvrtc: a box without it runs kernels compiled elsewhere (it looks them up under every NVRTC version the
+ * directory's file headers name; the headers are read again only when the directory changes).  A disk hit in mode 1 means the
+ * first launch is already translated.  libnvrtc is looked up as "libnvrtc.so.12" and under /usr/local/cuda/lib64; FX8010_NVRTC
+ * names the one library to load instead, and when that cannot be loaded the process has no NVRTC.
+ *
+ * The disk store is off unless FX8010_KERNEL_CACHE=<dir> (read when a handle is created or a precompile runs) or
+ * fx8010_kernel_cache_set_dir names a directory.  One file per kernel, <dir>/fx8010-v1/<hex digest>.cubin: a 96-byte header
+ * (magic "FX8010KC", format 1, NVRTC major and minor, the digest, the payload length, the SHA-256 of the payload), then the CUBIN.
+ * Files are written to a unique temporary file and renamed into place, so concurrent processes never see a partial file.  A file
+ * that fails validation, or whose CUBIN the driver refuses, is counted as rejected, recompiled and replaced; an I/O error never fails
+ * a call (the kernel is used from memory and the failure counted).  Nothing is evicted: each file stands alone and may be deleted at
+ * any time.  The NVRTC version is part of the key: a process that loads another libnvrtc (a Python package may bring its own, and
+ * an already loaded one is what dlopen returns) compiles its own kernels, so precompile with the libnvrtc the application loads. */
+
+/* Sets the disk store's directory for the whole process, overriding FX8010_KERNEL_CACHE; NULL or "" turns it off.  Always 0. */
+FX8010_API int fx8010_kernel_cache_set_dir(const char* dir);
+/* Compiles the kernel a handle would generate for `image` on n_instances instances (with control curves on regs[n_curves], as in
+ * fx8010_translate_source_curves) and writes it to the disk store; needs libnvrtc, no device.  0 written, 1 a valid file was already
+ * there, -1 bad arguments, -2 not eligible, -3 no cache directory, -4 compile failed, -5 write failed. */
+FX8010_API int fx8010_kernel_cache_precompile(const fx8010_program_image* image, int n_instances, int n_channels, const int32_t* regs,
+                                              const int32_t* broadcast, int n_curves);
+/* Process-wide counters since the library was loaded. */
+typedef struct fx8010_kernel_cache_stats {
+    uint64_t nvrtc_compiles;       /* NVRTC compiles (fx8010_translate_source's compile_check included)          */
+    uint64_t memory_hits;          /* kernels found loaded on the handle's device                                 */
+    uint64_t store_hits;           /* CUBINs found in the process store                                           */
+    uint64_t joined_compiles;      /* NVRTC compiles in flight joined instead of started                          */
+    uint64_t disk_hits;            /* kernels loaded from the disk store                                          */
+    uint64_t disk_writes;          /* files written                                                               */
+    uint64_t disk_rejected;        /* files that failed validation or module load                                 */
+    uint64_t disk_write_failures;  /* writes that failed (directory missing, not writable, disk full)              */
+} fx8010_kernel_cache_stats;
+FX8010_API int fx8010_kernel_cache_get_stats(fx8010_kernel_cache_stats* out);
+
 /* Text of the last error on this handle (or of the last failed create when h == NULL). */
 FX8010_API const char* fx8010_gpu_last_error(fx8010_gpu* h);
 

@@ -33,6 +33,8 @@ FX8010_API int fx8010_host_ready(fx8010_host* h);                      /* getRea
 FX8010_API void fx8010_host_set_relaxed(fx8010_host* h, int on);
 /* FX8010::setTranslation: the program translator's mode (FX8010_OPT_TRANSLATE of fx8010_gpu.h: 0, 1 or 2); 0 ok / 1 bad mode */
 FX8010_API int fx8010_host_set_translation(fx8010_host* h, int mode);
+/* FX8010::setKernelCacheDir: the translator's disk kernel cache, process-wide (fx8010_kernel_cache_set_dir of fx8010_gpu.h); NULL or "" = off */
+FX8010_API void fx8010_host_set_kernel_cache_dir(const char* dir);
 
 /* decoded image (what loadFile leaves in the object) */
 FX8010_API int fx8010_host_num_registers(fx8010_host* h);
