@@ -128,7 +128,7 @@ struct fx8010_gpu {
     float* d_planar_in = nullptr; float* d_planar_out = nullptr; size_t planar_floats = 0;   // [C][S][N] scratch of process_batch_planar
     int enc_family = -1;                         // kernel family whose constant memory holds it
     PlanKey plan_key; Launch plan = {};          // last launch plan (reused while nothing relevant changes)
-    bool attr_set[3][2][2] = {};
+    std::vector<const void*> smem_optin_fns;     // kernels this handle let use the opt-in shared-memory limit (smem_optin_for)
     // Programmatic dependent launch: the buffers read / written by every launch since (and including) the last one
     // that waited for its predecessor at its START.  A launch that postpones its wait can still be running next to
     // any of them, so a new launch may postpone its own wait only if it is disjoint from the whole chain.
@@ -160,14 +160,12 @@ struct fx8010_gpu {
     int use_tma = 1;                             // 0 never, 1 launches with one time segment (recurrences), 2 every eligible launch
     int use_carry = 1;
     bool short_ok = false;                       // SKIP-free, nobody reads ccr, no noise/MACMV, every channel written: fx_short_kernel when short enough
-    bool short_attr_set[3][2][SH_MAX_NI_HOST] = {};
     int use_sl = 1, tune_M = 0, use_short = 1, tune_chunk = 0, use_fuse = 1;
     std::vector<int> sl_class, sl_index;         // per register: RowClass and index inside its class
     int sl_n_ro = 0, sl_n_wo = 0, sl_n_rw = 0;
     int sl_M = 0;                                // batch length of the uploaded encoding (0 = generic encoding uploaded)
     std::vector<uint2> sl_load, sl_wb;
     uint2* d_sl_load = nullptr; uint2* d_sl_wb = nullptr;
-    bool sl_attr_set[2][3] = {};                 // MaxDynamicSharedMemorySize set for kernel <K, SKIP, EXT>
     int n_exec = 0;                              // encoded instructions
     int n_unpred = 0;                            // ... of which no SKIP can reach (general interpreter: counted per pass, not per instruction)
     std::vector<uint32_t> latch_ch;              // channels served from the latch every sample period
@@ -783,7 +781,6 @@ void free_state(fx8010_gpu* h) {
     h->d_itram = nullptr; h->d_xtram = nullptr; h->d_counts = nullptr; h->d_wb = nullptr; h->d_latch_ch = nullptr; h->d_reg_map = nullptr; h->d_load_rows = nullptr; h->d_sl_load = nullptr; h->d_sl_wb = nullptr;
 }
 
-KernelFn pick_kernel(int K, bool skip, bool ext) { return generic_kernel(K, skip, ext); }
 // Encoded length of the program for the generic kernel (END/NOP are dropped when there is no SKIP).
 int encoded_length(const fx8010_gpu* h) {
     int e = 0;
@@ -799,21 +796,27 @@ bool use_short_kernel(const fx8010_gpu* h) {
     const int e = encoded_length(h);
     return h->use_short && h->short_ok && !h->trace_mode && e >= 1 && e <= SH_MAX_NI_HOST;
 }
-KernelFn pick_short_kernel(int K, bool ext, int ni) { return short_kernel(K, ext, ni); }
 
-int known_tram_span(const fx8010_gpu* h);
+int tr_kind(const fx8010_gpu* h, const Translation& T);
 constexpr int MIN_TSPLIT_SPAN = 64;      // shorter spans would mean too many tiny launches: the serial kernel (with its sample split) takes those
 
 #include "fx8010_translate.inc"
 
+// Every buffer of a call, both channel strides, one channel's ns periods and every per-instance curve of `cv` (n_cv of them) are
+// aligned to `bytes`: what a kernel that moves bytes / 4 adjacent instances per access needs.
+bool io_aligned(const fx8010_gpu* h, size_t bytes, const float* const* ins, const float* const* outs, int n_blk, size_t in_cs, size_t out_cs, int ns,
+                const CurveBlock* cv = nullptr, int n_cv = 0) {
+    const uintptr_t a = bytes - 1;
+    if (((in_cs * 4) & a) || ((out_cs * 4) & a) || (((size_t)ns * h->N * 4) & a)) return false;
+    for (int b = 0; b < n_blk; ++b) if (((uintptr_t)ins[b] | (uintptr_t)outs[b]) & a) return false;
+    for (int j = 0; cv && j < n_cv; ++j) if (!cv->bcast[j] && ((uintptr_t)cv->p[j] & a)) return false;
+    return true;
+}
+
 // Geometry of one launch: contexts per thread, block size, time split.
 int plan_launch(fx8010_gpu* h, const float* d_in, const float* d_out, size_t in_cs, size_t out_cs, int n_samples, Launch& L) {
     const int N = h->N, C = h->C, nr = (int)h->reg_map.size();
-    auto aligned = [&](int K) {
-        const size_t a = (size_t)K * 4;
-        return N % K == 0 && ((uintptr_t)d_in % a) == 0 && ((uintptr_t)d_out % a) == 0 &&
-               (in_cs * 4) % a == 0 && (out_cs * 4) % a == 0;
-    };
+    auto aligned = [&](int K) { return N % K == 0 && io_aligned(h, (size_t)K * 4, &d_in, &d_out, 1, in_cs, out_cs, n_samples); };
     const int min_seg = 8;
     const long max_seg = h->stateless ? std::max(1, n_samples / min_seg) : 1;
     const long want_threads = (long)h->num_sms * 512;
@@ -850,7 +853,7 @@ int plan_launch(fx8010_gpu* h, const float* d_in, const float* d_out, size_t in_
     L.grid_x = (N / K + B - 1) / B;
     L.n_seg = 1; L.seg_len = n_samples;
     if (h->stateless && n_samples > min_seg && !h->trace_mode) {
-        KernelFn fn = use_short_kernel(h) ? pick_short_kernel(K, h->has_ext, encoded_length(h)) : pick_kernel(K, h->has_skip, h->has_ext);
+        KernelFn fn = use_short_kernel(h) ? short_kernel(K, h->has_ext, encoded_length(h)) : generic_kernel(K, h->has_skip, h->has_ext);
         int occ = 1;
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, B, L.smem);
         occ = std::max(occ, 1);
@@ -865,12 +868,20 @@ int plan_launch(fx8010_gpu* h, const float* d_in, const float* d_out, size_t in_
     return FX8010_OK;
 }
 
-SLKernelFn pick_sl_kernel(int K, bool tram) { return sl_kernel(K, tram); }
+// READ-after-WRITE distance of a written TRAM stream in sample periods (0 = unknown): pointers untouched since load_program (both
+// pointers of a ring then advance in lockstep from 0), offsets held by registers that carry one known value in every instance.
+int ring_distance(const fx8010_gpu* h, const fx8010_gpu::TramStream& t) {
+    if (!h->tram_ptrs_pristine || !h->reg_uniform[t.yreg] || !h->reg_uniform[t.w_yreg]) return 0;
+    const int size = t.isx ? h->xtram_size : h->itram_size;
+    if (size <= 0) return 0;
+    const int pos = std::min(std::max(cvt_x86_host(h->reg_value[t.yreg]), 0), size - 1);
+    const int wpos = std::min(std::max(cvt_x86_host(h->reg_value[t.w_yreg]), 0), size - 1);
+    const int d = (wpos + pos) % size;
+    return (d == 0 && !t.w_first) ? size : d;
+}
 
-// Shortest READ-after-WRITE distance of the TRAM streams, in sample periods, when the host can tell: pointers untouched
-// since load_program (both pointers of a ring then advance in lockstep from 0) and offsets held by registers that
-// carry one known value in every instance.  0 = unknown.  (The kernel checks the real distance per thread anyway; this
-// only decides how long a batch is worth planning for.)
+// Shortest READ-after-WRITE distance of the TRAM streams (0 = unknown).  (The kernel checks the real distance per thread
+// anyway; this only decides how long a batch is worth planning for.)
 int known_tram_distance(const fx8010_gpu* h) {
     if (!h->tram_ptrs_pristine) return 0;
     int best = 1 << 30;
@@ -880,15 +891,10 @@ int known_tram_distance(const fx8010_gpu* h) {
         if (u == U_XWRITE) best = std::min(best, h->xtram_size);
     }
     for (int q = 0; q < h->sl_n_tr; ++q) {
-        const fx8010_gpu::TramStream& t = h->sl_tr[q];
-        if (t.w_yreg < 0) continue;                        // nobody writes this ring: any batch length is safe
-        if (!h->reg_uniform[t.yreg] || !h->reg_uniform[t.w_yreg]) return 0;
-        const int size = t.isx ? h->xtram_size : h->itram_size;
-        if (size <= 0) return 0;
-        const int pos = std::min(std::max(cvt_x86_host(h->reg_value[t.yreg]), 0), size - 1);
-        const int wpos = std::min(std::max(cvt_x86_host(h->reg_value[t.w_yreg]), 0), size - 1);
-        const int d = (wpos + pos) % size;
-        best = std::min(best, (d == 0 && !t.w_first) ? size : d);
+        if (h->sl_tr[q].w_yreg < 0) continue;              // nobody writes this ring: any batch length is safe
+        const int D = ring_distance(h, h->sl_tr[q]);
+        if (D <= 0) return 0;
+        best = std::min(best, D);
     }
     return best;
 }
@@ -913,11 +919,7 @@ int known_tram_span(const fx8010_gpu* h) {
         const fx8010_gpu::TramStream& t = h->sl_tr[q];
         if (t.w_yreg < 0) continue;                        // a ring nobody writes: its periods are independent anyway
         const int size = t.isx ? h->xtram_size : h->itram_size;
-        if (size <= 0) return 0;
-        const int pos = std::min(std::max(cvt_x86_host(h->reg_value[t.yreg]), 0), size - 1);
-        const int wpos = std::min(std::max(cvt_x86_host(h->reg_value[t.w_yreg]), 0), size - 1);
-        const int d = (wpos + pos) % size;
-        const int D = (d == 0 && !t.w_first) ? size : d;   // read-after-write distance
+        const int D = ring_distance(h, t);
         if (D <= 0) return 0;
         span = std::min(span, D);
         if (D < size) span = std::min(span, size - D);      // write-after-read distance
@@ -925,6 +927,36 @@ int known_tram_span(const fx8010_gpu* h) {
     // a ring with a WRITE but no READ stream, or a READ of a ring nobody writes, constrains nothing beyond the ring size
     return span == (1 << 30) ? 0 : span;
 }
+
+// Which translated kernel translation T gets: 0 = serial (fx_translated), 1 = streaming (a stateless program), 2 = streaming with
+// TRAM (a delay line whose only state across periods is its rings and whose known span allows the launches route() cuts along
+// time; the instruction-major kernel runs the rest).  With control curves every program the translator accepts runs translated
+// (the interpreter kernels read no curves, and one serial launch costs far less than one launch per period): the streaming kernel
+// also needs 16-byte accesses to whole groups of 4 instances, ring offsets that follow no curve (the cut needs offsets that are one
+// known value), and no launch of this curve set that it did not fit (T.serial).
+int tr_kind(const fx8010_gpu* h, const Translation& T) {
+    if (!T.cv_reg.empty() && (T.serial || h->N % 4)) return 0;
+    if (h->stateless) return 1;
+    if (!(h->sl_ok && h->sl_tram && h->use_sl && h->use_tsplit && !(h->tr_recurrences & 2))) return 0;
+    if (known_tram_span(h) < MIN_TSPLIT_SPAN) return 0;                 // (0 for a register recurrence)
+    for (const fx8010_instr& in : h->instrs) {
+        const Uop u = uop_of(h, in);
+        if (u == U_IREAD || u == U_XREAD || u == U_IWRITE || u == U_XWRITE)
+            for (int r : T.cv_reg) if (r == in.y) return 0;
+    }
+    return 2;
+}
+
+// Lets kernel fn use the device's opt-in dynamic shared-memory limit (once per kernel and handle; the occupancy query honours
+// the limit only once it is set on the function).
+template <class Fn> int smem_optin_for(fx8010_gpu* h, Fn fn) {
+    const void* f = reinterpret_cast<const void*>(fn);
+    if (std::find(h->smem_optin_fns.begin(), h->smem_optin_fns.end(), f) != h->smem_optin_fns.end()) return FX8010_OK;
+    FX_CUDA(h, cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin));
+    h->smem_optin_fns.push_back(f);
+    return FX8010_OK;
+}
+
 // Geometry for the stateless kernel: all the parallelism a launch needs comes from cutting the time
 // axis, so K is as wide as alignment allows and the segment count fills exactly one wave.
 int plan_stateless(fx8010_gpu* h, const float*, const float*, unsigned align, int n_samples, int n_blk, bool may_overlap, bool tsplit, Launch& L) {
@@ -973,19 +1005,15 @@ int plan_stateless(fx8010_gpu* h, const float*, const float*, unsigned align, in
     L.smem = sl_smem_bytes(h, B, K, M);
     L.grid_x = (N / K + B - 1) / B;
     int occ = 1;
-    {   // (the occupancy query honours the opt-in shared-memory limit only once it is set on the function)
-        bool& attr = h->sl_attr_set[h->sl_tram ? 1 : 0][K == 4 ? 2 : (K == 2 ? 1 : 0)];
-        if (!attr) { FX_CUDA(h, cudaFuncSetAttribute(pick_sl_kernel(K, h->sl_tram), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin)); attr = true; }
-    }
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pick_sl_kernel(K, h->sl_tram), B, L.smem);
+    const int rc = smem_optin_for(h, sl_kernel(K, h->sl_tram));
+    if (rc) return rc;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, sl_kernel(K, h->sl_tram), B, L.smem);
     occ = std::max(occ, 1);
     // A launch that can overlap its neighbours (late wait, programmatic dependent launch) is planned as half a wave:
     // two consecutive launches share the SMs, and fewer, longer segments spend fewer instructions on per-thread start-up.
     // One that waits at its start has the SMs to itself: one full wave.
     const long slots = (long)h->num_sms * occ;
     long n_seg = std::max(1L, slots / ((may_overlap ? 2 : 1) * L.grid_x));
-    // ... a launch much longer than its own ramp-up (many instances, or several sample blocks fused into it) is cut
-    // into work items of about 128 samples, but into no fewer than two waves' worth, so that the tail balances
     // ... a launch much longer than its own ramp-up (many instances, or several sample blocks fused into it): all thread
     // blocks do the same amount of work, so the last wave is as long as a full one however few blocks it holds — pick
     // the segment count whose block count sits just below a whole number of waves (cfg2, 20 blocks per launch: 3 segments =
@@ -1092,74 +1120,315 @@ int order_on(fx8010_gpu* h, cudaStream_t st) {
     return FX8010_OK;
 }
 
-// Launches n_blk consecutive sample blocks of ns samples each (block b: ins[b] -> outs[b]).  A time-split (stateless)
-// program runs up to MAX_FUSED_BLOCKS of them in ONE launch — its work items are (block, time segment, instance group)
-// and all are independent; everything else runs block after block.  `own_prev`: the operation right before this one on
-// `st` is known to be this handle's own launch (or nothing that signals programmatic completion early).
-int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, int n_blk, size_t in_cs, size_t out_cs, int n_samples, cudaStream_t st, bool own_prev) {
-    if (n_samples == 0 || n_blk == 0) return FX8010_OK;
-    {
-        const int rc = order_on(h, st);
-        if (rc) return rc;
-    }
+// How the next piece of a call runs (route).
+enum Path {
+    PATH_SPLIT,           // cut every block into pieces of `len` periods and route each piece again
+    PATH_TR_SERIAL,       // the translated serial kernel, block after block
+    PATH_TR_STREAM,       // the translated streaming kernel: a stateless program, or a delay line cut along time
+    PATH_INTERP,          // the instruction-major kernel, else the short-program kernel, else the general interpreter
+    PATH_PER_PERIOD,      // (control curves) per period, one copy of the curves into the registers and one plain one-period call
+};
+struct Route {
+    Path path;
+    int len;              // periods per launch: the whole block, a stretch of known_tram_span, the counter limit (PATH_SPLIT), or one
+    int fuse = 1;         // sample blocks one launch may take
+    bool tsplit = false;  // (PATH_INTERP) a delay line whose periods in this launch are independent: planned like a stateless program
+};
+
+// Which kernel runs the next piece of a call: n_blk blocks of ns periods (plain translation h->tr), or one with the curves cv (h->tr_cv).
+// Reaching tr_ready starts a compile: the order of the conditions decides which programs ever compile (a plain cfg4 call never does).
+Route route(fx8010_gpu* h, const float* const* ins, float* const* outs, int n_blk, size_t in_cs, size_t out_cs, int ns, const CurveBlock* cv) {
     // per-launch executed-instruction counters are 32-bit: split very long batches
     const long long per_sample = (long long)h->instrs.size() * FX8010_MAX_PASSES;
     const int max_samples = (int)std::max<long long>(1, std::min<long long>(0x7fffffffLL, 0xffffffffLL / per_sample));
-    if (n_samples > max_samples) {
-        for (int b = 0; b < n_blk; ++b)
-            for (int s0 = 0; s0 < n_samples; s0 += max_samples) {
-                const float* in = ins[b] ? ins[b] + (size_t)s0 * h->N : nullptr;
-                float* out = outs[b] + (size_t)s0 * h->N;
-                const int rc = launch_blocks(h, &in, &out, 1, in_cs, out_cs, std::min(max_samples, n_samples - s0), st, own_prev || b > 0 || s0 > 0);
-                if (rc) return rc;
-            }
-        return FX8010_OK;
+    if (ns > max_samples) return Route{PATH_SPLIT, max_samples};
+    if (cv) {
+        // Control curves run translated or period by period (the interpreter kernels read no curves).
+        const Route per_period{PATH_PER_PERIOD, 1};
+        Translation& T = h->tr_cv;
+        const int n_cv = (int)T.cv_reg.size();
+        if (h->trace_mode || !tr_ready(h, T)) return per_period;
+        if (T.kind != 0) {
+            // the streaming kernel: 16-byte accesses at i0 to the samples and to the per-instance curves; a delay line is cut along time
+            const int span = T.kind == 2 ? known_tram_span(h) : ns;
+            if (io_aligned(h, 16, ins, outs, 1, in_cs, out_cs, ns, cv, n_cv) && span >= std::min(ns, MIN_TSPLIT_SPAN))
+                return Route{span < ns ? PATH_SPLIT : PATH_TR_STREAM, std::min(span, ns)};
+            // It does not fit this launch (a buffer not 16-byte aligned, a delay line whose span is no longer known): from now on
+            // this curve set takes the serial kernel, which needs neither.
+            T.serial = true;
+            tr_reset(h, T);
+            if (!tr_ready(h, T)) return per_period;
+        }
+        return io_aligned(h, (size_t)T.lanes * 4, ins, outs, 1, in_cs, out_cs, ns, cv, n_cv) ? Route{PATH_TR_SERIAL, ns} : per_period;
     }
     // Delay lines: periods closer than the known span are independent, so a block is cut into stretches of at most that
     // many periods, each one launch cut along time like a stateless program (the stretches themselves run in order).
     const int span = (h->sl_ok && h->use_sl && !h->trace_mode && h->use_tsplit) ? known_tram_span(h) : 0;
     // (worth it when the block needs at most two launches — cfg3 at 16 384 instances x 1 024 periods: span 100, eleven launches,
     //  198 us against 139 us for the serial kernel with its sample split; span 1 000, two launches, 111 against 112; one launch, 82)
-    // ... or any number of launches when they run on the translated streaming kernel (fx8010_translate.inc, tr_kind 2): a stretch of 100 periods
+    // ... or any number of launches when they run on the translated streaming kernel (tr_kind 2): a stretch of 100 periods
     // of cfg3 is a 6 us launch there (cfg3, ring of 100: 11 launches 66 us against 134 us serial)
-    bool tr_stretch = false;
-    if (span >= MIN_TSPLIT_SPAN && 2L * span < n_samples && tr_kind(h) == 2 && h->use_translate && h->N % 4 == 0 && (in_cs * 4) % 16 == 0 && (out_cs * 4) % 16 == 0) {
-        tr_stretch = true;
-        for (int b = 0; b < n_blk && tr_stretch; ++b) tr_stretch = (((uintptr_t)ins[b] | (uintptr_t)outs[b]) & 15u) == 0;
-        tr_stretch = tr_stretch && tr_ready(h, h->tr);
-    }
-    const bool tsplit = span >= MIN_TSPLIT_SPAN && (2L * span >= n_samples || tr_stretch);
-    if (tsplit && n_samples > span) {
-        for (int b = 0; b < n_blk; ++b)
-            for (int s0 = 0; s0 < n_samples; s0 += span) {
-                const float* in = ins[b] ? ins[b] + (size_t)s0 * h->N : nullptr;
-                float* out = outs[b] + (size_t)s0 * h->N;
-                const int rc = launch_blocks(h, &in, &out, 1, in_cs, out_cs, std::min(span, n_samples - s0), st, own_prev || b > 0 || s0 > 0);
-                if (rc) return rc;
-            }
-        return FX8010_OK;
-    }
+    const bool stretch = span >= MIN_TSPLIT_SPAN && 2L * span < ns && tr_kind(h, h->tr) == 2 && h->use_translate && h->N % 4 == 0 &&
+                         io_aligned(h, 16, ins, outs, n_blk, in_cs, out_cs, ns) && tr_ready(h, h->tr);
+    const bool tsplit = span >= MIN_TSPLIT_SPAN && (2L * span >= ns || stretch);
+    if (tsplit && ns > span) return Route{PATH_SPLIT, span};
     // Programs of the general interpreter run on their translated kernel once it exists (fx8010_translate.inc).
     // FX8010_TR_RECUR (developer switch): bit 0 = self recurrences (cfg4), bit 1 = delay lines (cfg3) take the translated serial kernel
     const bool tr_recur = h->sl_ok && h->sl_serial && (((h->tr_recurrences & 1) && !h->sl_tram) || ((h->tr_recurrences & 2) && h->sl_tram));
-    if (!h->stateless && (tr_recur || (!(h->sl_ok && h->use_sl) && !use_short_kernel(h))) && !h->trace_mode && tr_ready(h, h->tr) && tr_aligned(h, h->tr, ins, outs, n_blk, in_cs, out_cs, n_samples, nullptr)) {
-        for (int b = 0; b < n_blk; ++b) {
-            const int rc = tr_launch(h, h->tr, ins[b], outs[b], in_cs, out_cs, n_samples, st, nullptr);
+    if (!h->stateless && (tr_recur || (!(h->sl_ok && h->use_sl) && !use_short_kernel(h))) && !h->trace_mode && tr_ready(h, h->tr) &&
+        io_aligned(h, (size_t)h->tr.lanes * 4, ins, outs, n_blk, in_cs, out_cs, ns))
+        return Route{PATH_TR_SERIAL, ns};
+    // A stateless program, or a delay line cut along time, runs on the translated streaming kernel once that exists: 4 adjacent
+    // instances per thread, so the instance count and every buffer must allow 16-byte accesses.
+    const bool tr_sl = (h->stateless || (tsplit && tr_kind(h, h->tr) == 2)) && !h->trace_mode && h->N % 4 == 0 &&
+                       io_aligned(h, 16, ins, outs, n_blk, in_cs, out_cs, ns) && tr_ready(h, h->tr);
+    const bool fuse = (h->sl_ok && h->use_sl && !h->trace_mode && !h->sl_serial && h->use_fuse) || (tr_sl && h->stateless);
+    return Route{tr_sl ? PATH_TR_STREAM : PATH_INTERP, ns, fuse ? MAX_FUSED_BLOCKS : 1, tsplit};
+}
+
+// Cuts the ns periods of every block into pieces of at most len and hands each to run(in, out, periods, s0, own_prev), blocks in
+// order; every piece but the first follows this handle's own launch.
+template <class Run> int split_periods(const fx8010_gpu* h, const float* const* ins, float* const* outs, int n_blk, int ns, int len, bool own_prev, Run run) {
+    for (int b = 0; b < n_blk; ++b)
+        for (int s0 = 0; s0 < ns; s0 += len) {
+            const float* in = ins[b] ? ins[b] + (size_t)s0 * h->N : nullptr;
+            float* out = outs[b] + (size_t)s0 * h->N;
+            const int rc = run(in, out, std::min(len, ns - s0), s0, own_prev || b > 0 || s0 > 0);
             if (rc) return rc;
-            h->tram_periods += (unsigned long long)n_samples;
+        }
+    return FX8010_OK;
+}
+
+// Books one launch on `path` with geometry L over nb blocks of ns periods: the TRAM periods, the chain of late-waiting launches and
+// h->info.  `sp`: the buffers the launch touches (plain interpreter and streaming launches join the chain; the other launches wait at
+// their start and leave it empty).  `tma` < 0 leaves info.last_tma as it was.  Known discrepancies, kept as they are:
+//   * a fused launch of the streaming kernel reports last_grid = grid_x * n_seg, without its nb blocks;
+//   * bit 32 (short-program kernel) is set by M == 0 && use_short_kernel(h) for a plain launch of the streaming kernel too;
+//   * a launch of the general interpreter or the short-program kernel leaves last_tma as the launch before it set it.
+void record_launch(fx8010_gpu* h, Path path, const Launch& L, int nb, int ns, int late_wait, int tma, bool curves, const fx8010_gpu::Span* sp,
+                   cudaStream_t st) {
+    const bool translated = path == PATH_TR_SERIAL || path == PATH_TR_STREAM;
+    const bool lean = L.M == 0 && (path == PATH_INTERP || (path == PATH_TR_STREAM && !curves)) && use_short_kernel(h);
+    const bool pairs = L.M > 0 && std::any_of(h->sl_fuse.begin(), h->sl_fuse.end(), [](uint8_t f) { return f != 0; });
+    h->tram_periods += (unsigned long long)ns * nb;
+    if (!late_wait) h->chain.clear();          // this launch waited at its start: everything before it is complete
+    if (sp) { h->chain.push_back(*sp); h->chain_stream = st; }
+    h->info.kernel_launches++;
+    h->info.last_grid = L.grid_x * L.n_seg * (path == PATH_TR_STREAM ? 1 : nb); h->info.last_block = L.B * L.P; h->info.last_time_split = L.n_seg;
+    h->info.last_smem_bytes = (int)L.smem;
+    h->info.last_late_wait = late_wait; h->info.last_fused_blocks = nb;
+    if (tma >= 0) h->info.last_tma = tma;
+    h->info.kernel_variant = (h->has_skip ? 1 : 0) | (h->has_ext ? 2 : 0) | (h->stateless ? 4 : 0) | (L.M > 0 ? 8 : 0) | (curves ? 16 : 0) | (lean ? 32 : 0) |
+                             (pairs ? 64 : 0) | (translated ? 128 : 0) | (L.K << 8) | (L.M << 16);
+}
+
+// The runtime-API launch of an interpreter kernel: grid = instance groups x (time segments x nb blocks), programmatic dependent
+// launch when enabled.
+template <class Fn, class P> int interp_drive(fx8010_gpu* h, Fn fn, const Launch& L, int nb, cudaStream_t st, const P& p) {
+    const int rc = smem_optin_for(h, fn);
+    if (rc) return rc;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(L.grid_x, L.n_seg * nb); cfg.blockDim = dim3(L.B * L.P); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
+    cudaLaunchAttribute attrs[1];
+    attrs[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attrs[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attrs; cfg.numAttrs = h->use_pdl ? 1 : 0;
+    FX_CUDA(h, cudaLaunchKernelEx(&cfg, fn, p));
+    return FX8010_OK;
+}
+
+// nb consecutive blocks on the instruction-major kernel (geometry L from plan_stateless; tsplit as routed).  `tma`: whether its
+// input stage uses bulk tensor copies.
+int sl_launch(fx8010_gpu* h, const Launch& L, const float* const* ins, float* const* outs, int nb, size_t in_cs, size_t out_cs, int ns, bool tsplit,
+              int late_wait, cudaStream_t st, int& tma) {
+    SLParams p = {};
+    p.gpr = h->d_gpr; p.acc = h->d_acc; p.latch = h->d_latch; p.counts = h->d_counts; p.rt_flags = h->d_flags;
+    p.tabs = h->d_tabs; p.load_list = h->d_sl_load; p.wb_list = h->d_sl_wb;
+    p.n_blk = nb;
+    for (int b = 0; b < nb; ++b) { p.blk_in[b] = ins[b]; p.blk_out[b] = outs[b]; }
+    p.in_cstride = in_cs; p.out_cstride = out_cs;
+    p.n_samples = ns; p.seg_len = L.seg_len; p.n_seg = L.n_seg;
+    p.N = h->N; p.C = h->C; p.n_instrs = (int)h->instrs.size(); p.n_exec = h->n_exec; p.prog_off = h->arena_off;
+    p.n_load = (int)h->sl_load.size(); p.n_wb = (int)h->sl_wb.size();
+    p.M = L.M;
+    p.stage0 = (uint32_t)L.B * L.K * 4u * (uint32_t)(h->sl_n_ro + h->sl_n_wo + h->sl_n_rw * L.M);
+    p.n_smem_tabs = h->n_smem_tabs;
+    for (int t = 0; t < MAX_SMEM_TABLES; ++t) p.smem_tab_id[t] = h->smem_tab_id[t];
+    p.acc_writer = h->acc_writer ? 1 : 0;
+    p.ccr_live = h->sl_ccr_live ? 1 : 0;
+    p.ptrs = h->d_ptrs; p.itram = h->d_itram; p.xtram = h->d_xtram; p.itram_size = h->itram_size; p.xtram_size = h->xtram_size;
+    p.has_tram = h->sl_tram ? 1 : 0; p.n_tr = h->sl_n_tr; p.P = L.P;
+    for (int j = 0; j < 4; ++j) p.tr_ops[j] = 0;
+    for (const fx8010_instr& ins_ : h->instrs) {         // pointer j (iw, ir, xw, xr) moves once per sample period per executed op
+        const Uop u = uop_of(h, ins_);
+        if (u == U_IWRITE) p.tr_ops[0]++; else if (u == U_IREAD) p.tr_ops[1]++;
+        else if (u == U_XWRITE) p.tr_ops[2]++; else if (u == U_XREAD) p.tr_ops[3]++;
+    }
+    p.tr_on[0] = p.tr_on[1] = 0;
+    for (int q = 0; q < h->sl_n_tr; ++q) {
+        const fx8010_gpu::TramStream& t = h->sl_tr[q];
+        const int x = t.isx;                             // the kernel indexes streams by TRAM: 0 = iTRAM, 1 = xTRAM
+        p.tr_on[x] = 1;
+        p.tr_stage[x] = sl_word(h, t.reg, L.B, L.K, L.M) & SL_OFF_MASK;
+        p.tr_y[x] = sl_word(h, t.yreg, L.B, L.K, L.M) & SL_OFF_MASK;
+        p.tr_wy[x] = t.w_yreg >= 0 ? (sl_word(h, t.w_yreg, L.B, L.K, L.M) & SL_OFF_MASK) : 0xffffffffu;
+        p.tr_wfirst[x] = t.w_first;
+    }
+    // cut along time (the pointers are as load_program left them and have moved once per period launched since — known_tram_span):
+    // every segment starts from the host's copy of the pointers, not from the array the last segment's owner rewrites
+    p.tr_base_valid = 0;
+    if (h->sl_tram && tsplit && L.n_seg > 1 && h->tram_ptrs_pristine) {
+        p.tr_base_valid = 1;
+        for (int j = 0; j < 4; ++j) {
+            const int size = j < 2 ? h->itram_size : h->xtram_size;
+            p.tr_base[j] = (size > 0 && p.tr_ops[j]) ? (int)(h->tram_periods * (unsigned long long)p.tr_ops[j] % (unsigned long long)size) : 0;
+        }
+    }
+    p.pdl_late_wait = late_wait;
+    p.use_tma = 0;
+    // Bulk tensor copies (TMA) for the input stage: one instruction per batch and channel instead of one cp.async per thread and
+    // sample row.  Pays where the per-batch overhead is serial with a recurrence (cfg4 at 8 192 instances: 67 -> 59 us, at 65 536:
+    // 125 -> 121 us); a time-split launch loses a little to the block-wide barrier per batch (cfg2 per launch: 8.5 -> 8.6 us) and keeps cp.async.
+    if ((h->use_tma == 2 || (h->use_tma == 1 && L.n_seg == 1 && h->sl_serial)) && !h->sl_tram && nb == 1 && ins[0] && L.P == 1 && in_cs % (size_t)h->N == 0) {
+        const size_t rpc = in_cs / (size_t)h->N;
+        if (make_input_map(ins[0], (size_t)h->N, (size_t)(h->C - 1) * rpc + (size_t)ns, L.B * L.K, L.M, &p.in_map)) { p.use_tma = 1; p.tma_rows_per_channel = (int)rpc; }
+    }
+    tma = p.use_tma;
+    return interp_drive(h, sl_kernel(L.K, h->sl_tram), L, nb, st, p);
+}
+
+// One block on the general interpreter, or on the short-program kernel when the program is short enough (geometry L from plan_launch).
+int generic_launch(fx8010_gpu* h, const Launch& L, const float* in, float* out, size_t in_cs, size_t out_cs, int ns, int late_wait, cudaStream_t st) {
+    Params p = {};
+    p.gpr = h->d_gpr; p.acc = h->d_acc; p.lfsr = h->d_lfsr; p.latch = h->d_latch; p.ptrs = h->d_ptrs;
+    p.itram = h->d_itram; p.xtram = h->d_xtram; p.counts = h->d_counts; p.rt_flags = h->d_flags;
+    p.reg_map = h->d_reg_map; p.load_rows = h->d_load_rows; p.wb_regs = h->d_wb; p.latch_ch = h->d_latch_ch; p.tabs = h->d_tabs;
+    p.in = in; p.out = out; p.in_cstride = in_cs; p.out_cstride = out_cs;
+    p.n_samples = ns; p.seg_len = L.seg_len; p.n_seg = L.n_seg;
+    p.N = h->N; p.C = h->C; p.n_regs = (int)h->reg_map.size(); p.n_instrs = (int)h->instrs.size();
+    p.n_wb = (int)h->wb.size(); p.prog_off = h->arena_off;
+    p.n_exec = h->n_exec; p.n_latch_ch = (int)h->latch_ch.size(); p.n_unpred = h->n_unpred;
+    p.n_load = (int)h->load_rows.size(); p.load_latch = h->load_latch; p.load_acc = h->load_acc;
+    p.itram_size = h->itram_size; p.xtram_size = h->xtram_size;
+    p.n_smem_tabs = h->n_smem_tabs;
+    for (int t = 0; t < MAX_SMEM_TABLES; ++t) p.smem_tab_id[t] = h->smem_tab_id[t];
+    p.chunk = L.chunk;
+    p.pdl_late_wait = late_wait;
+    const bool kskip = h->has_skip || h->trace_mode, kext = h->has_ext || h->trace_mode;
+    p.trace = h->trace_mode ? h->d_trace : nullptr; p.trace_inst = h->trace_inst;
+    return interp_drive(h, use_short_kernel(h) ? short_kernel(L.K, kext, h->n_exec) : generic_kernel(L.K, kskip, kext), L, 1, st, p);
+}
+
+// The driver-API launch of translated kernel T (it lives in an NVRTC module): grid = L.grid_x x (L.n_seg x nb blocks), programmatic
+// dependent launch when enabled.
+int tr_drive(fx8010_gpu* h, const Translation& T, const Launch& L, int nb, cudaStream_t st, void** args) {
+    const DriverApi& d = driver_api();
+    CUlaunchConfig cfg = {};
+    cfg.gridDimX = (unsigned)L.grid_x; cfg.gridDimY = (unsigned)(L.n_seg * nb); cfg.gridDimZ = 1;
+    cfg.blockDimX = (unsigned)L.B; cfg.blockDimY = 1; cfg.blockDimZ = 1;
+    cfg.sharedMemBytes = (unsigned)L.smem; cfg.hStream = (CUstream)st;
+    CUlaunchAttribute attr[1];
+    attr[0].id = CU_LAUNCH_ATTRIBUTE_PROGRAMMATIC_STREAM_SERIALIZATION;
+    attr[0].value.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr; cfg.numAttrs = h->use_pdl ? 1 : 0;
+    const CUresult rc = d.launchKernelEx(&cfg, (CUfunction)T.fn, args, nullptr);
+    if (rc == CUDA_SUCCESS) return FX8010_OK;
+    const char* msg = nullptr;
+    if (d.getErrorString) d.getErrorString(rc, &msg);
+    return fail(h, FX8010_ERR_CUDA, std::string("translated kernel launch: ") + (msg ? msg : "driver error"));
+}
+
+// One block on the translated serial kernel.  Same ordering rules as the interpreter launch that waits at its start.  `cv`: the
+// call's control curves (the automated translation only).  L: the geometry it ran with.
+int tr_launch(fx8010_gpu* h, const Translation& T, const float* in, float* out, size_t in_cs, size_t out_cs, int ns, cudaStream_t st, const CurveBlock* cv,
+              Launch& L) {
+    const DriverApi& d = driver_api();
+    const int N = h->N;
+    // block size: one warp per block until every SM holds a few; the kernel's registers bound residency anyway
+    int B = 32;
+    if ((long)N / T.lanes >= (long)h->num_sms * 32 * 16) B = 64;
+    if ((long)N / T.lanes >= (long)h->num_sms * 32 * 64) B = 128;
+    if (h->tune_B) B = h->tune_B;
+    while (B > 32 && (size_t)T.ring_floats * B * 4 > h->smem_optin) B >>= 1;
+    const unsigned smem = (unsigned)(T.ring_floats * B * 4);       // the input ring (<= 64 periods x 128 threads x 4 B per row)
+    if (smem > 48 * 1024 &&                                        // beyond the default dynamic shared-memory limit: opt in
+        (!d.funcSetAttribute || d.funcSetAttribute((CUfunction)T.fn, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, (int)h->smem_optin) != CUDA_SUCCESS))
+        return fail(h, FX8010_ERR_CAPACITY, "the translated kernel's input ring does not fit in shared memory");
+    void* gpr = h->d_gpr; void* acc = h->d_acc; void* lfsr = h->d_lfsr; void* latch = h->d_latch; void* ptrs = h->d_ptrs;
+    void* itram = h->d_itram; void* xtram = h->d_xtram; void* counts = h->d_counts; void* flags = h->d_flags; void* tabs = h->d_tabs;
+    const void* inp = in; void* outp = out;
+    int ns_ = ns, N_ = N, isz = h->itram_size, xsz = h->xtram_size;
+    CurveBlock cvb = cv ? *cv : CurveBlock{};
+    void* args[] = {&gpr, &acc, &lfsr, &latch, &ptrs, &itram, &xtram, &counts, &flags, &tabs, &inp, &outp, &in_cs, &out_cs, &ns_, &N_, &isz, &xsz, &cvb};
+    L.K = T.lanes; L.B = B; L.P = 1; L.grid_x = (N / T.lanes + B - 1) / B; L.n_seg = 1; L.seg_len = ns; L.smem = smem;
+    return tr_drive(h, T, L, 1, st, args);
+}
+
+// nb consecutive blocks of a stateless program (or one stretch of a delay line) on its translated streaming kernel (late_wait as
+// launch_blocks computes it).  `cv`: the call's control curves (the automated translation only; nb == 1).  L: the geometry it ran with.
+int tr_sl_launch(fx8010_gpu* h, const Translation& T, const float* const* ins, float* const* outs, int nb, size_t in_cs, size_t out_cs, int ns, cudaStream_t st,
+                 int late_wait, Launch& L, const CurveBlock* cv) {
+    const int N = h->N, K = 4;
+    struct { const float* in[32]; float* out[32]; } io = {};
+    for (int b = 0; b < nb; ++b) { io.in[b] = ins[b]; io.out[b] = outs[b]; }
+    int B = 128;
+    if (h->tune_B) B = h->tune_B;
+    const int gx = (N / K + B - 1) / B;
+    // time segments: every thread takes `seg_len` samples (whole 4-sample load groups).  Short segments mean more threads — a lone
+    // block ramps up faster (cfg2, one block per call: 11 us at 8 samples, 15-19 at 16-32) — long ones amortise the per-thread
+    // start-up once the launch holds a couple of waves anyway (cfg2, 20 blocks per launch: 6.3 us per block at 8, 5.9 at 32):
+    // the shortest power of two that keeps the launch within about 2.5 full waves of warps.
+    int seg_len = 8;
+    const long warps_per_row = ((long)gx * B + 31) / 32;
+    while (seg_len < ns && warps_per_row * ((ns + seg_len - 1) / seg_len) * nb > (long)h->num_sms * 64 * 5 / 2) seg_len <<= 1;
+    if (env_int("FX8010_TUNE_SEGLEN") > 0) seg_len = env_int("FX8010_TUNE_SEGLEN");
+    int n_seg = (ns + seg_len - 1) / seg_len;
+    while ((long)n_seg * nb > 65535) { seg_len <<= 1; n_seg = (ns + seg_len - 1) / seg_len; }
+    void* gpr = h->d_gpr; void* acc = h->d_acc; void* latch = h->d_latch; void* counts = h->d_counts; void* flags = h->d_flags; void* tabs = h->d_tabs;
+    int ns_ = ns, nb_ = nb, N_ = N, lw = late_wait, isz = h->itram_size, xsz = h->xtram_size;
+    void* ptrs = h->d_ptrs; void* itram = h->d_itram; void* xtram = h->d_xtram;
+    // ring pointers at this launch's first period (delay lines only: every pointer of a ring that has the instruction has moved once per period since load_program)
+    int base[4] = {0, 0, 0, 0};
+    if (T.kind == 2) {
+        const unsigned long long done = h->tram_periods;
+        if (h->itram_size > 0) base[0] = base[1] = (int)(done % (unsigned long long)h->itram_size);
+        if (h->xtram_size > 0) base[2] = base[3] = (int)(done % (unsigned long long)h->xtram_size);
+    }
+    CurveBlock cvb = cv ? *cv : CurveBlock{};
+    void* args[] = {&io, &gpr, &acc, &latch, &counts, &flags, &tabs, &in_cs, &out_cs, &ns_, &seg_len, &n_seg, &nb_, &N_, &lw, &ptrs, &itram, &xtram, &isz, &xsz,
+                    &base[0], &base[1], &base[2], &base[3], &cvb};
+    L.K = K; L.B = B; L.P = 1; L.M = 0; L.grid_x = gx; L.n_seg = n_seg; L.seg_len = seg_len; L.smem = 0; L.chunk = 0;
+    return tr_drive(h, T, L, nb, st, args);
+}
+
+// Launches n_blk consecutive sample blocks of ns samples each (block b: ins[b] -> outs[b]) the way route() decides.  A time-split
+// (stateless) program runs up to MAX_FUSED_BLOCKS of them in ONE launch — its work items are (block, time segment, instance group)
+// and all are independent; everything else runs block after block.  `own_prev`: the operation right before this one on
+// `st` is known to be this handle's own launch (or nothing that signals programmatic completion early).
+int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, int n_blk, size_t in_cs, size_t out_cs, int ns, cudaStream_t st, bool own_prev) {
+    if (ns == 0 || n_blk == 0) return FX8010_OK;
+    {
+        const int rc = order_on(h, st);
+        if (rc) return rc;
+    }
+    const Route r = route(h, ins, outs, n_blk, in_cs, out_cs, ns, nullptr);
+    // (known discrepancy: PATH_SPLIT and PATH_TR_SERIAL accept a call whose blocks mix NULL and non-NULL inputs; the loop below refuses it)
+    if (r.path == PATH_SPLIT)
+        return split_periods(h, ins, outs, n_blk, ns, r.len, own_prev, [&](const float* in, float* out, int k, int, bool own) {
+            return launch_blocks(h, &in, &out, 1, in_cs, out_cs, k, st, own);
+        });
+    if (r.path == PATH_TR_SERIAL) {
+        for (int b = 0; b < n_blk; ++b) {
+            Launch L = {};
+            const int rc = tr_launch(h, h->tr, ins[b], outs[b], in_cs, out_cs, ns, st, nullptr, L);
+            if (rc) return rc;
+            record_launch(h, r.path, L, 1, ns, 0, 0, false, nullptr, st);
         }
         return FX8010_OK;
     }
-    const int ns = n_samples;
-    const bool fusable = h->sl_ok && h->use_sl && !h->trace_mode && !h->sl_serial && h->use_fuse;
-    // A stateless program runs on its translated streaming kernel once that exists (fx8010_translate.inc): 4 adjacent instances
-    // per thread, so the instance count and every buffer must allow 16-byte accesses.
-    const bool tr_delay = !h->stateless && tsplit && ns <= span && tr_kind(h) == 2;       // a time-cut launch of a delay line
-    bool tr_sl = (h->stateless || tr_delay) && !h->trace_mode && h->N % 4 == 0 && (in_cs * 4) % 16 == 0 && (out_cs * 4) % 16 == 0 && ((size_t)ns * h->N * 4) % 16 == 0;
-    for (int b = 0; b < n_blk && tr_sl; ++b) tr_sl = (((uintptr_t)ins[b] | (uintptr_t)outs[b]) & 15u) == 0;
-    tr_sl = tr_sl && tr_ready(h, h->tr);
+    const bool tr_sl = r.path == PATH_TR_STREAM, tsplit = r.tsplit;
     for (int b0 = 0; b0 < n_blk;) {
-        const int nb = (fusable || (tr_sl && h->stateless)) ? std::min(n_blk - b0, MAX_FUSED_BLOCKS) : 1;
+        const int nb = std::min(n_blk - b0, r.fuse);
         if (h->encode_dirty && !tr_sl) { select_tables(h); h->plan_key.ns = -1; }
         Launch L = {};
         // the plan depends on the batch length and on how far the buffers are aligned
@@ -1234,110 +1503,12 @@ int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, in
             if (ins[b]) { sp.in_lo = std::min(sp.in_lo, i_lo); sp.in_hi = std::max(sp.in_hi, i_hi); }
         }
         const int late_wait = (may_overlap && disjoint) ? 1 : 0;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(L.grid_x, L.n_seg * (L.M > 0 ? nb : 1)); cfg.blockDim = dim3(L.B * L.P); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
-        cudaLaunchAttribute attrs[1];
-        attrs[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attrs[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attrs; cfg.numAttrs = h->use_pdl ? 1 : 0;
-        const float* in = ins[b0]; float* out = outs[b0];
-        if (tr_sl) {
-            const int rc = tr_sl_launch(h, h->tr, ins + b0, outs + b0, nb, in_cs, out_cs, ns, st, late_wait, L, nullptr);
-            if (rc) return rc;
-            h->info.last_tma = 0;
-        } else if (L.M > 0) {
-            SLParams p = {};
-            p.gpr = h->d_gpr; p.acc = h->d_acc; p.latch = h->d_latch; p.counts = h->d_counts; p.rt_flags = h->d_flags;
-            p.tabs = h->d_tabs; p.load_list = h->d_sl_load; p.wb_list = h->d_sl_wb;
-            p.n_blk = nb;
-            for (int b = 0; b < nb; ++b) { p.blk_in[b] = ins[b0 + b]; p.blk_out[b] = outs[b0 + b]; }
-            p.in_cstride = in_cs; p.out_cstride = out_cs;
-            p.n_samples = ns; p.seg_len = L.seg_len; p.n_seg = L.n_seg;
-            p.N = h->N; p.C = h->C; p.n_instrs = (int)h->instrs.size(); p.n_exec = h->n_exec; p.prog_off = h->arena_off;
-            p.n_load = (int)h->sl_load.size(); p.n_wb = (int)h->sl_wb.size();
-            p.M = L.M;
-            p.stage0 = (uint32_t)L.B * L.K * 4u * (uint32_t)(h->sl_n_ro + h->sl_n_wo + h->sl_n_rw * L.M);
-            p.n_smem_tabs = h->n_smem_tabs;
-            for (int t = 0; t < MAX_SMEM_TABLES; ++t) p.smem_tab_id[t] = h->smem_tab_id[t];
-            p.acc_writer = h->acc_writer ? 1 : 0;
-            p.ccr_live = h->sl_ccr_live ? 1 : 0;
-            p.ptrs = h->d_ptrs; p.itram = h->d_itram; p.xtram = h->d_xtram; p.itram_size = h->itram_size; p.xtram_size = h->xtram_size;
-            p.has_tram = h->sl_tram ? 1 : 0; p.n_tr = h->sl_n_tr; p.P = L.P;
-            for (int j = 0; j < 4; ++j) p.tr_ops[j] = 0;
-            for (const fx8010_instr& ins_ : h->instrs) {         // pointer j (iw, ir, xw, xr) moves once per sample period per executed op
-                const Uop u = uop_of(h, ins_);
-                if (u == U_IWRITE) p.tr_ops[0]++; else if (u == U_IREAD) p.tr_ops[1]++;
-                else if (u == U_XWRITE) p.tr_ops[2]++; else if (u == U_XREAD) p.tr_ops[3]++;
-            }
-            p.tr_on[0] = p.tr_on[1] = 0;
-            for (int q = 0; q < h->sl_n_tr; ++q) {
-                const fx8010_gpu::TramStream& t = h->sl_tr[q];
-                const int x = t.isx;                             // the kernel indexes streams by TRAM: 0 = iTRAM, 1 = xTRAM
-                p.tr_on[x] = 1;
-                p.tr_stage[x] = sl_word(h, t.reg, L.B, L.K, L.M) & SL_OFF_MASK;
-                p.tr_y[x] = sl_word(h, t.yreg, L.B, L.K, L.M) & SL_OFF_MASK;
-                p.tr_wy[x] = t.w_yreg >= 0 ? (sl_word(h, t.w_yreg, L.B, L.K, L.M) & SL_OFF_MASK) : 0xffffffffu;
-                p.tr_wfirst[x] = t.w_first;
-            }
-            // cut along time (the pointers are as load_program left them and have moved once per period launched since — known_tram_span):
-            // every segment starts from the host's copy of the pointers, not from the array the last segment's owner rewrites
-            p.tr_base_valid = 0;
-            if (h->sl_tram && tsplit && L.n_seg > 1 && h->tram_ptrs_pristine) {
-                p.tr_base_valid = 1;
-                for (int j = 0; j < 4; ++j) {
-                    const int size = j < 2 ? h->itram_size : h->xtram_size;
-                    p.tr_base[j] = (size > 0 && p.tr_ops[j]) ? (int)(h->tram_periods * (unsigned long long)p.tr_ops[j] % (unsigned long long)size) : 0;
-                }
-            }
-            p.pdl_late_wait = late_wait;
-            p.use_tma = 0;
-            // Bulk tensor copies (TMA) for the input stage: one instruction per batch and channel instead of one cp.async per thread and
-            // sample row.  Pays where the per-batch overhead is serial with a recurrence (cfg4 at 8 192 instances: 67 -> 59 us, at 65 536:
-            // 125 -> 121 us); a time-split launch loses a little to the block-wide barrier per batch (cfg2 per launch: 8.5 -> 8.6 us) and keeps cp.async.
-            if ((h->use_tma == 2 || (h->use_tma == 1 && L.n_seg == 1 && h->sl_serial)) && !h->sl_tram && nb == 1 && in && L.P == 1 && in_cs % (size_t)h->N == 0) {
-                const size_t rpc = in_cs / (size_t)h->N;
-                if (make_input_map(in, (size_t)h->N, (size_t)(h->C - 1) * rpc + (size_t)ns, L.B * L.K, L.M, &p.in_map)) { p.use_tma = 1; p.tma_rows_per_channel = (int)rpc; }
-            }
-            h->info.last_tma = p.use_tma;
-            SLKernelFn fn = pick_sl_kernel(L.K, h->sl_tram);
-            bool& attr = h->sl_attr_set[h->sl_tram ? 1 : 0][L.K == 4 ? 2 : (L.K == 2 ? 1 : 0)];
-            if (!attr) { FX_CUDA(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin)); attr = true; }
-            FX_CUDA(h, cudaLaunchKernelEx(&cfg, fn, p));
-        } else {
-            Params p = {};
-            p.gpr = h->d_gpr; p.acc = h->d_acc; p.lfsr = h->d_lfsr; p.latch = h->d_latch; p.ptrs = h->d_ptrs;
-            p.itram = h->d_itram; p.xtram = h->d_xtram; p.counts = h->d_counts; p.rt_flags = h->d_flags;
-            p.reg_map = h->d_reg_map; p.load_rows = h->d_load_rows; p.wb_regs = h->d_wb; p.latch_ch = h->d_latch_ch; p.tabs = h->d_tabs;
-            p.in = in; p.out = out; p.in_cstride = in_cs; p.out_cstride = out_cs;
-            p.n_samples = ns; p.seg_len = L.seg_len; p.n_seg = L.n_seg;
-            p.N = h->N; p.C = h->C; p.n_regs = (int)h->reg_map.size(); p.n_instrs = (int)h->instrs.size();
-            p.n_wb = (int)h->wb.size(); p.prog_off = h->arena_off;
-            p.n_exec = h->n_exec; p.n_latch_ch = (int)h->latch_ch.size(); p.n_unpred = h->n_unpred;
-            p.n_load = (int)h->load_rows.size(); p.load_latch = h->load_latch; p.load_acc = h->load_acc;
-            p.itram_size = h->itram_size; p.xtram_size = h->xtram_size;
-            p.n_smem_tabs = h->n_smem_tabs;
-            for (int t = 0; t < MAX_SMEM_TABLES; ++t) p.smem_tab_id[t] = h->smem_tab_id[t];
-            p.chunk = L.chunk;
-            p.pdl_late_wait = late_wait;
-            const bool kskip = h->has_skip || h->trace_mode, kext = h->has_ext || h->trace_mode;
-            p.trace = h->trace_mode ? h->d_trace : nullptr; p.trace_inst = h->trace_inst;
-            const bool lean = use_short_kernel(h);
-            KernelFn fn = lean ? pick_short_kernel(L.K, kext, h->n_exec) : pick_kernel(L.K, kskip, kext);
-            bool& attr = lean ? h->short_attr_set[L.K == 4 ? 2 : (L.K == 2 ? 1 : 0)][kext ? 1 : 0][h->n_exec - 1]
-                              : h->attr_set[L.K == 4 ? 2 : (L.K == 2 ? 1 : 0)][kskip ? 1 : 0][kext ? 1 : 0];
-            if (!attr) { FX_CUDA(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_optin)); attr = true; }
-            FX_CUDA(h, cudaLaunchKernelEx(&cfg, fn, p));
-        }
-        bool pairs = false;
-        if (L.M > 0 && !tr_sl) for (uint8_t f : h->sl_fuse) pairs = pairs || f;
-        h->tram_periods += (unsigned long long)ns * nb;
-        if (!late_wait) h->chain.clear();          // this launch waited at its start: everything before it is complete
-        h->chain.push_back(sp); h->chain_stream = st;
-        h->info.kernel_launches++;
-        h->info.last_grid = L.grid_x * L.n_seg * (L.M > 0 ? nb : 1); h->info.last_block = L.B * L.P; h->info.last_time_split = L.n_seg;
-        h->info.last_smem_bytes = (int)L.smem;
-        h->info.last_late_wait = late_wait; h->info.last_fused_blocks = nb;
-        h->info.kernel_variant = (h->has_skip ? 1 : 0) | (h->has_ext ? 2 : 0) | (h->stateless ? 4 : 0) | (L.M > 0 ? 8 : 0) | ((L.M == 0 && use_short_kernel(h)) ? 32 : 0) | (pairs ? 64 : 0) | (tr_sl ? 128 : 0) | (L.K << 8) | (L.M << 16);
+        int tma = -1, rc;
+        if (tr_sl) { rc = tr_sl_launch(h, h->tr, ins + b0, outs + b0, nb, in_cs, out_cs, ns, st, late_wait, L, nullptr); tma = 0; }
+        else if (L.M > 0) rc = sl_launch(h, L, ins + b0, outs + b0, nb, in_cs, out_cs, ns, tsplit, late_wait, st, tma);
+        else rc = generic_launch(h, L, ins[b0], outs[b0], in_cs, out_cs, ns, late_wait, st);
+        if (rc) return rc;
+        record_launch(h, r.path, L, nb, ns, late_wait, tma, false, &sp, st);
         b0 += nb;
     }
     return FX8010_OK;
@@ -1374,36 +1545,33 @@ __global__ void fx_curve_rows_kernel(float* __restrict__ gpr, const CurveRows ro
         dst[i] = rows.cv.bcast[j] ? p[s] : p[(size_t)s * N + i];
 }
 
-// n_samples periods with the curves `cb` on the automated translation (returns 1 when the launch does not qualify: nothing queued).
-int curves_translated(fx8010_gpu* h, const float* d_in, float* d_out, size_t cs, int ns, const CurveBlock& cb, int n, cudaStream_t st) {
-    Translation& T = h->tr_cv;
+// ns periods of one block with the curves of `rows`, the way route() decides.
+int launch_curves(fx8010_gpu* h, const float* d_in, float* d_out, size_t cs, int ns, const CurveRows& rows, cudaStream_t st) {
     const size_t N = (size_t)h->N;
-    if (T.kind == 0) {
-        if (!tr_aligned(h, T, &d_in, &d_out, 1, cs, cs, ns, &cb)) return 1;
-        const int rc = tr_launch(h, T, d_in, d_out, cs, cs, ns, st, &cb);
+    const Route r = route(h, &d_in, &d_out, 1, cs, cs, ns, &rows.cv);
+    if (r.path == PATH_SPLIT)
+        return split_periods(h, &d_in, &d_out, 1, ns, r.len, false, [&](const float* in, float* out, int k, int s0, bool) {
+            CurveRows piece = rows;
+            piece.cv = curves_from(rows.cv, rows.n, (size_t)s0, N);
+            return launch_curves(h, in, out, cs, k, piece, st);
+        });
+    if (r.path == PATH_TR_SERIAL || r.path == PATH_TR_STREAM) {
+        Launch L = {};
+        const int rc = r.path == PATH_TR_SERIAL ? tr_launch(h, h->tr_cv, d_in, d_out, cs, cs, ns, st, &rows.cv, L)
+                                                : tr_sl_launch(h, h->tr_cv, &d_in, &d_out, 1, cs, cs, ns, st, 0, L, &rows.cv);
         if (rc) return rc;
-        h->tram_periods += (unsigned long long)ns;
+        record_launch(h, r.path, L, 1, ns, 0, 0, true, nullptr, st);
         return FX8010_OK;
     }
-    // the streaming kernel: 16-byte accesses at i0 to the samples and to the per-instance curves; a delay line is cut along time
-    bool ok = ((((uintptr_t)d_in | (uintptr_t)d_out) & 15u) == 0) && (cs * 4) % 16 == 0;
-    for (int j = 0; j < n; ++j) ok = ok && (cb.bcast[j] || ((uintptr_t)cb.p[j] & 15u) == 0);
-    const int span = T.kind == 2 ? known_tram_span(h) : ns;
-    if (!ok || span < std::min(ns, MIN_TSPLIT_SPAN)) return 1;
-    for (int s0 = 0; s0 < ns; s0 += span) {
-        const int k = std::min(span, ns - s0);
-        const float* in = d_in ? d_in + (size_t)s0 * N : nullptr;
-        float* out = d_out + (size_t)s0 * N;
-        const CurveBlock cv = curves_from(cb, n, (size_t)s0, N);
-        Launch L = {};
-        const int rc = tr_sl_launch(h, T, &in, &out, 1, cs, cs, k, st, 0, L, &cv);
-        if (rc) return rc;
-        h->tram_periods += (unsigned long long)k;
-        h->chain.clear();
+    // Per-period path (correctness, not speed): no translated kernel for this curve set, or the launch does not qualify.  Each period
+    // is one copy of the curves' values into the register rows and one ordinary one-period launch.
+    for (int s = 0; s < ns; ++s) {
+        fx_curve_rows_kernel<<<dim3((unsigned)std::min<size_t>(1024, (N + 255) / 256), (unsigned)rows.n), 256, 0, st>>>(h->d_gpr, rows, s, (int)N);
         h->info.kernel_launches++;
-        h->info.last_grid = L.grid_x * L.n_seg; h->info.last_block = L.B; h->info.last_time_split = L.n_seg; h->info.last_smem_bytes = 0;
-        h->info.last_late_wait = 0; h->info.last_fused_blocks = 1; h->info.last_tma = 0;
-        h->info.kernel_variant = (h->has_skip ? 1 : 0) | (h->has_ext ? 2 : 0) | (h->stateless ? 4 : 0) | 16 | 128 | (L.K << 8);
+        FX_CUDA(h, cudaGetLastError());
+        h->chain.clear();
+        const int rc = launch_block(h, d_in ? d_in + (size_t)s * N : nullptr, d_out + (size_t)s * N, cs, cs, 1, st);
+        if (rc) return rc;
     }
     return FX8010_OK;
 }
@@ -1807,40 +1975,7 @@ int fx8010_gpu_process_batch_curves(fx8010_gpu* h, const float* d_in, float* d_o
         tr_reset(h, h->tr_cv);
         h->tr_cv.cv_reg = regs; h->tr_cv.cv_bcast = bc; h->tr_cv.serial = false;
     }
-    // per-launch executed-instruction counters are 32-bit: very long batches in pieces (as launch_blocks does)
-    const long long per_sample = (long long)h->instrs.size() * FX8010_MAX_PASSES;
-    const int max_samples = (int)std::max<long long>(1, std::min<long long>(0x7fffffffLL, 0xffffffffLL / per_sample));
-    for (int s0 = 0; s0 < n_samples; s0 += max_samples) {
-        const int ns = std::min(max_samples, n_samples - s0);
-        const float* in = d_in ? d_in + (size_t)s0 * N : nullptr;
-        float* out = d_out + (size_t)s0 * N;
-        const CurveBlock cv = curves_from(rows.cv, n_curves, (size_t)s0, N);
-        if (!h->trace_mode && tr_ready(h, h->tr_cv)) {
-            int rc = curves_translated(h, in, out, cs, ns, cv, n_curves, st);
-            if (rc == 1 && h->tr_cv.kind != 0) {
-                // The streaming kernel does not fit this launch (a buffer not 16-byte aligned, a delay line whose span is no longer known):
-                // from now on this curve set takes the serial kernel, which does not need either.
-                h->tr_cv.serial = true;
-                tr_reset(h, h->tr_cv);
-                rc = tr_ready(h, h->tr_cv) ? curves_translated(h, in, out, cs, ns, cv, n_curves, st) : 1;
-            }
-            if (rc == FX8010_OK) continue;
-            if (rc != 1) return rc;
-        }
-        // Per-period path (correctness, not speed): no translated kernel for this curve set, or the launch does not qualify.  Each period
-        // is one copy of the curves' values into the register rows and one ordinary one-period launch.
-        CurveRows r1 = rows;
-        r1.cv = cv;
-        for (int s = 0; s < ns; ++s) {
-            fx_curve_rows_kernel<<<dim3((unsigned)std::min<size_t>(1024, (N + 255) / 256), (unsigned)n_curves), 256, 0, st>>>(h->d_gpr, r1, s, (int)N);
-            h->info.kernel_launches++;
-            FX_CUDA(h, cudaGetLastError());
-            h->chain.clear();
-            const int rc = launch_block(h, in ? in + (size_t)s * N : nullptr, out + (size_t)s * N, cs, cs, 1, st);
-            if (rc) return rc;
-        }
-    }
-    return FX8010_OK;
+    return launch_curves(h, d_in, d_out, cs, n_samples, rows, st);
 }
 
 // [C][rows][cols] -> [C][cols][rows], 32 x 32 tiles through shared memory (coalesced on both sides)
@@ -2185,9 +2320,8 @@ int fx8010_gpu_translate_status_curves(fx8010_gpu* h, int* state, int* regs_per_
 
 // Needs no device: analyses the image as load_program would and generates the CUDA source of its translated kernel (for control curves
 // on cregs[n_curves] when n_curves > 0) into `src`.  0, -1 for a bad image or curve list, -2 when the program is not eligible.
-// For a freshly loaded image this is the source a handle generates at its first launch on a B200 (148 SMs), with one exception: a delay
-// line whose known span is below MIN_TSPLIT_SPAN gets the serial kernel here, where a handle runs the interpreter kernels and never asks;
-// and the developer switches a handle reads when it is created (FX8010_NO_STATELESS, FX8010_NO_TSPLIT, FX8010_TR_RECUR) are not applied.
+// For a freshly loaded image this is the source a handle generates at its first launch on a B200 (148 SMs), except that the developer
+// switches a handle reads when it is created (FX8010_NO_STATELESS, FX8010_NO_TSPLIT, FX8010_TR_RECUR) are not applied.
 static int translate_source_gen(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
                                 int n_curves, std::string& src) {
     if (!im || !im->instrs || !im->regs || im->n_instrs <= 0 || im->n_regs <= 0 || n_channels <= 0 || n_instances <= 0) return -1;
@@ -2211,7 +2345,7 @@ static int translate_source_gen(const fx8010_program_image* im, int n_instances,
     for (int r : T.cv_reg) tmp.reg_uniform[r] = 0;            // (as fx8010_gpu_process_batch_curves leaves them)
     tmp.tr_volatile.assign(im->n_regs, 0);
     analyse(&tmp);
-    const int kind = n_curves ? tr_kind_curves(&tmp, T) : ((tr_kind(&tmp) == 2 && known_tram_span(&tmp) < MIN_TSPLIT_SPAN) ? 0 : tr_kind(&tmp));
+    const int kind = tr_kind(&tmp, T);
     tmp.tr_gen = n_curves ? &T : nullptr;
     if (kind == 0 && !tr_eligible(&tmp)) return -2;
     std::vector<uint8_t> folded;
