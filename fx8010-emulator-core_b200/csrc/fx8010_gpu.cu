@@ -1412,7 +1412,6 @@ int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, in
         if (rc) return rc;
     }
     const Route r = route(h, ins, outs, n_blk, in_cs, out_cs, ns, nullptr);
-    // (known discrepancy: PATH_SPLIT and PATH_TR_SERIAL accept a call whose blocks mix NULL and non-NULL inputs; the loop below refuses it)
     if (r.path == PATH_SPLIT)
         return split_periods(h, ins, outs, n_blk, ns, r.len, own_prev, [&](const float* in, float* out, int k, int, bool own) {
             return launch_blocks(h, &in, &out, 1, in_cs, out_cs, k, st, own);
@@ -1433,12 +1432,8 @@ int launch_blocks(fx8010_gpu* h, const float* const* ins, float* const* outs, in
         Launch L = {};
         // the plan depends on the batch length and on how far the buffers are aligned
         unsigned align = 0;
-        bool any_in = false, all_in = true;
-        for (int b = b0; b < b0 + nb; ++b) {
-            align |= (unsigned)(((uintptr_t)ins[b] | (uintptr_t)outs[b]) & 15u);
-            any_in = any_in || ins[b]; all_in = all_in && ins[b];
-        }
-        if (any_in != all_in) return fail(h, FX8010_ERR_ARG, "either every block of a call has an input buffer or none has");
+        for (int b = b0; b < b0 + nb; ++b) align |= (unsigned)(((uintptr_t)ins[b] | (uintptr_t)outs[b]) & 15u);
+        const bool any_in = ins[b0] != nullptr;                   // (fx8010_gpu_process_blocks refuses a list that mixes NULL and non-NULL inputs)
         align |= (unsigned)(((uintptr_t)(in_cs * 4) | (uintptr_t)(out_cs * 4)) & 15u) | (any_in ? 16u : 0u);
         const int deep = ((h->sl_ok && h->sl_tram) ? (known_tram_distance(h) > 2 * SL_MAX_M ? 1 : 0) : 0) | (tsplit ? 2 : 0);
         // a launch that may overlap its neighbours (late wait) is planned as half a wave; one that waits at its start fills the SMs
@@ -1852,6 +1847,8 @@ int fx8010_gpu_process_blocks(fx8010_gpu* h, const float* const* d_in, float* co
     FX_NEED_PROGRAM(h);
     if (!d_out || n_samples < 0 || n_blocks < 0) return fail(h, FX8010_ERR_ARG, "d_out is NULL or a count is negative");
     for (int b = 0; b < n_blocks; ++b) if (!d_out[b]) return fail(h, FX8010_ERR_ARG, "d_out holds a NULL block");
+    for (int b = 1; d_in && b < n_blocks; ++b)
+        if (!d_in[b] != !d_in[0]) return fail(h, FX8010_ERR_ARG, "either every block of a call has an input buffer or none has");
     const size_t cs = (size_t)n_samples * h->N;
     std::vector<const float*> no_in;
     if (!d_in) { no_in.assign((size_t)std::max(1, n_blocks), nullptr); d_in = no_in.data(); }

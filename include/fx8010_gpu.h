@@ -160,7 +160,8 @@ FX8010_API int fx8010_gpu_process_batch(fx8010_gpu* h, const float* d_in, float*
                                         int n_samples, void* stream);
 /* n_blocks consecutive blocks of n_samples each in one call: block b reads d_in[b] and writes d_out[b] (arrays of
  * DEVICE pointers, each block laid out as above; d_in may be NULL, or all of its entries NULL, when the program has no
- * INPUT operand).  Equivalent to n_blocks fx8010_gpu_process_batch calls in order; a program without state across sample
+ * INPUT operand).  A d_in whose entries are neither all NULL nor all non-NULL is refused with FX8010_ERR_ARG before
+ * anything is queued.  Equivalent to n_blocks fx8010_gpu_process_batch calls in order; a program without state across sample
  * periods runs up to 32 blocks per kernel launch, and the library knows that its own launches follow one another
  * on the stream (see FX8010_OPT_STREAM_EXCLUSIVE). */
 FX8010_API int fx8010_gpu_process_blocks(fx8010_gpu* h, const float* const* d_in, float* const* d_out, int n_blocks,

@@ -111,6 +111,27 @@ def impulse_noise(n_instances: int, n_samples: int, rng: np.random.Generator) ->
     return x
 
 
+# LOG / EXP input values outside the tables' domain, where rule U6 defines the result (index clamped, FX8010_RT_TABLE_RANGE set):
+# |A| > 1 up to the largest finite value, signed zeros, subnormals, and a NaN.  The NaN is quiet, positive and carries every payload
+# bit: the one NaN an IEEE operation produces on the GPU and propagates unchanged on the CPU.  (Infinities are left out: where a table
+# row is flat, its zero slope times an infinite distance is an invalid operation, whose NaN is 0xffc00000 on x86 and 0x7fffffff on
+# the GPU.)
+TABLE_EDGE_BITS = [0x3f800001, 0xbf800001, 0x3fc00000, 0xbfc00000, 0x40000000, 0xc0000000, 0x7149f2ca, 0xf149f2ca, 0x7f7fffff, 0xff7fffff,
+                   0x00000000, 0x80000000, 0x00000001, 0x80000001, 0x007fffff, 0x807fffff, 0x00400000, 0x80012345,
+                   0x7fffffff]
+
+
+def table_sweep_grid(n: int, rng: np.random.Generator) -> np.ndarray:
+    """n float32 LOG / EXP inputs: every table boundary of [-1, 1] and both of its float32 neighbours, the U6 edge values above,
+    then uniform values in [-1, 1)."""
+    k = np.arange(64)
+    bounds = (-1.0 + k * (2.0 / 63)).astype(np.float32)
+    near = np.concatenate([np.nextafter(bounds, np.float32(-2)), bounds, np.nextafter(bounds, np.float32(2))]).astype(np.float32)
+    edge = np.array(TABLE_EDGE_BITS, dtype=np.uint32).view(np.float32)
+    head = np.concatenate([near, edge]).astype(np.float32)
+    return np.concatenate([head, (2 * rng.random(n - head.size) - 1).astype(np.float32)]).astype(np.float32)
+
+
 # ---- random programs -----------------------------------------------------------------------------
 
 SAT_OPS = ["macs", "macsn", "macints", "acc3", "interp"]

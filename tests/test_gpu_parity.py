@@ -238,23 +238,30 @@ def test_device_pointers_and_streams(fx, po):
 
 
 def test_table_sweep_all_selectors(fx, po):
-    """LOG and EXP over a dense grid of inputs (incl. every table boundary neighbourhood) for all 32
-    selectors, against the oracle's single-evaluation entry point."""
-    rng = np.random.default_rng(8)
+    """LOG and EXP over a dense grid of inputs (every table boundary and its neighbours, and the U6 inputs: |A| > 1, signed zeros,
+    subnormals, NaN) for each of the 32 selectors and for a per-instance selector held in a control, on the interpreter (translate
+    mode 0) and on the translated streaming kernel (mode 2: the programs are stateless and 4 096 instances allow its 16-byte
+    accesses).  The runtime flags follow the oracle's."""
     n = 4096
-    k = np.arange(64)
-    bounds = (-1.0 + k * (2.0 / 63)).astype(np.float32)
-    near = np.concatenate([np.nextafter(bounds, np.float32(-2)), bounds, np.nextafter(bounds, np.float32(2))]).astype(np.float32)
-    near = near[np.abs(near) <= 1]
-    grid = np.concatenate([near, (2 * rng.random(n - near.size) - 1).astype(np.float32)]).astype(np.float32)
-    for op in ("log", "exp"):
-        for sel in (0, 1, 3, 7, 31):
-            text = f"static a\ninput in_l 0\noutput out_l 0\n{op} a, in_l, {sel}, 0\nmacs out_l, 0, a, 1.0\nend"
-            run_case(fx, po, text, n, [2], rng, stimulus=lambda a, s: np.tile(grid, (s, 1)).reshape(1, s, n), what=f"{op} {sel}")
-    # dynamic selector (a control, per instance) goes through the global-memory table path
-    text = "static a\ninput in_l 0\ncontrol sel = 3\noutput out_l 0\nlog a, in_l, sel, 0\nexp out_l, a, sel, 0\nend"
-    sel = rng.integers(0, 32, n).astype(np.float32)
-    run_case(fx, po, text, n, [3], rng, controls={"sel": sel}, stimulus=lambda a, s: np.tile(grid, (s, 1)).reshape(1, s, n), what="dynamic selector")
+    grid = progs.table_sweep_grid(n, np.random.default_rng(8))
+    x = np.tile(grid, (3, 1)).reshape(1, 3, n)
+    dynamic = "static a\ninput in_l 0\ncontrol sel = 3\noutput out_l 0\nlog a, in_l, sel, 0\nexp out_l, a, sel, 0\nend"
+    texts = [f"static a\ninput in_l 0\noutput out_l 0\n{op} a, in_l, {sel}, 0\nmacs out_l, 0, a, 1.0\nend" for sel in range(32) for op in ("log", "exp")]
+    for mode in (0, 2):
+        for text in texts + [dynamic]:
+            what = f"{text.split(chr(10))[-3]}, mode {mode}"
+            prog, img, orc, gpu = make_pair(fx, po, text, n)
+            try:
+                gpu.set_option(fx.OPT_TRANSLATE, mode)
+                if text is dynamic:         # the selector is a control, per instance: the global-memory table path
+                    v = np.random.default_rng(9).integers(0, 32, n).astype(np.float32)
+                    gpu.set_controls(prog.reg_index("sel"), v); orc.set_register("sel", v)
+                assert_bits_equal(gpu.process_host(x), orc.process(x), what + " outputs")
+                compare_state(gpu, orc, img, what, (0, 200, n - 1))
+                assert orc.flags & fx.RT_TABLE_RANGE and gpu.flags() == orc.flags, (what, gpu.flags(), orc.flags)
+                assert bool(gpu.launch_info().kernel_variant & 128) == (mode == 2), (what, hex(gpu.launch_info().kernel_variant))
+            finally:
+                gpu.close()
 
 
 @pytest.mark.parametrize("k,b", [(1, 32), (2, 64), (4, 128), (4, 32)])

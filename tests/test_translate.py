@@ -200,6 +200,35 @@ def test_delay_lines_streaming_kernel(po, name):
     assert "fx_translated_sl" in ht.src and "#define FXT_NTR 0" not in ht.src
 
 
+@pytest.mark.parametrize("sel", [*range(32), "dynamic"])
+def test_table_sweep_all_selectors(po, sel):
+    """The sweep of test_gpu_parity.py::test_table_sweep_all_selectors on the generated streaming kernel: LOG and EXP at every table
+    boundary, its neighbours and the U6 inputs (|A| > 1, signed zeros, subnormals, NaN), per selector; the range flag as the oracle's."""
+    rng = np.random.default_rng(8)
+    n = 512
+    grid = progs.table_sweep_grid(n, rng)
+    x = np.tile(grid, (3, 1)).reshape(1, 3, n)
+    if sel == "dynamic":
+        texts = ["static a\ninput in_l 0\ncontrol sel = 3\noutput out_l 0\nlog a, in_l, sel, 0\nexp out_l, a, sel, 0\nend"]
+    else:
+        texts = [f"static a\ninput in_l 0\noutput out_l 0\n{op} a, in_l, {sel}, 0\nmacs out_l, 0, a, 1.0\nend" for op in ("log", "exp")]
+    for text in texts:
+        prog = fx.Program(text)
+        assert prog.loaded, prog.errors()
+        img = po.Image(prog.instructions(), prog.registers(), prog.itram_size, prog.xtram_size, prog.controls(), prog.tables())
+        orc = po.Oracle(img, n, 1)
+        ht = HostTranslated(prog, n, 1)
+        assert "fx_translated_sl" in ht.src
+        if sel == "dynamic":
+            v = rng.integers(0, 32, n).astype(np.float32)
+            orc.set_register("sel", v); ht.registers[prog.reg_index("sel"), :] = v
+        what = text.split("\n")[-3]
+        assert_bits_equal(ht.process(x), orc.process(x), what + " outputs")
+        assert_bits_equal(ht.registers, orc.registers, what + " registers")
+        assert_bits_equal(ht.counts, orc.counts, what + " counters")
+        assert orc.flags & fx.RT_TABLE_RANGE and int(ht.flags[0]) == orc.flags, (what, int(ht.flags[0]), orc.flags)
+
+
 @pytest.mark.parametrize("name", ["cfg5", "random"])
 def test_source_compiles_for_sm_100a(name):
     """NVRTC (no device needed) turns the generated source into an sm_100a CUBIN."""
