@@ -64,6 +64,10 @@ class CControlCurve(C.Structure):
     _fields_ = [("reg_index", C.c_int32), ("broadcast", C.c_int32), ("d_values", C.c_void_p)]
 
 
+class CHostCurve(C.Structure):
+    _fields_ = [("reg_index", C.c_int32), ("broadcast", C.c_int32), ("values", C.c_void_p)]
+
+
 MAX_CONTROL_CURVES = 8
 VARIANT_CURVES = 16        # fx8010_launch_info.kernel_variant: the last launch read control curves inside the kernel
 
@@ -132,6 +136,7 @@ GPU_SYMBOLS = {
     "fx8010_gpu_process_batch_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "fx8010_translate_source_curves": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_char_p, C.c_size_t,
                                                       C.c_int, C.POINTER(C.c_int)]),
+    "fx8010_gpu_process_batch_host_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_size_t, C.c_int]),
     "fx8010_kernel_cache_set_dir": (C.c_int, [C.c_char_p]),
     "fx8010_kernel_cache_precompile": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
     "fx8010_kernel_cache_get_stats": (C.c_int, [C.POINTER(CKernelCacheStats)]),
@@ -149,6 +154,8 @@ MULTI_SYMBOLS = {
     "fx8010_multi_process_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "fx8010_multi_process_batch_host_async": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "fx8010_multi_process_batch_host_broadcast": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int]),
+    "fx8010_multi_process_batch_host_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int]),
+    "fx8010_multi_shard_curves": (None, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fx8010_multi_synchronize": (C.c_int, [C.c_void_p]),
     "fx8010_multi_set_option": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "fx8010_multi_get_instruction_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_ulonglong)]),
@@ -193,6 +200,8 @@ HOST_SYMBOLS = {
     "fx8010_host_gpu": (C.c_void_p, [C.c_void_p]),
     "fx8010_host_process_block_device_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_char_p), C.c_void_p,
                                                           C.c_void_p, C.c_int, C.c_void_p]),
+    "fx8010_host_process_block_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_char_p), C.c_void_p,
+                                                   C.c_void_p, C.c_int]),
 }
 
 
@@ -231,6 +240,29 @@ def _ptr(a):
     if hasattr(a, "data_ptr"):          # torch tensor
         return a.data_ptr()
     raise TypeError(type(a))
+
+
+def _host_block(a, rows: int, cols: int, host_instances: int):
+    """A host buffer of `rows` rows of `cols` instances for the host-curve calls: a float32 array (copied to a C-contiguous one when it is
+    not), or with host_instances a view of `cols` columns of a C-contiguous array `host_instances` wide (its rows stay where they are)."""
+    if a is None or isinstance(a, int):
+        return a
+    if not host_instances:
+        return np.ascontiguousarray(a, dtype=np.float32).reshape(rows, cols)
+    assert a.dtype == np.float32 and a.shape[-1] == cols and a.strides[-1] == 4 and a.size == rows * cols, "not float32 columns of a wider block"
+    assert all(st == 4 * host_instances * int(np.prod(a.shape[k + 1:-1])) for k, st in enumerate(a.strides[:-1])), "rows not host_instances apart"
+    return a
+
+
+def _host_curves(curves, s: int, n: int, host_instances: int):
+    """[(register index, ndarray, broadcast)] -> (fx8010_host_curve array, the float32 arrays it points into)."""
+    arr = (CHostCurve * max(1, len(curves)))()
+    keep = []
+    for i, (reg, vals, bc) in enumerate(curves):
+        v = np.ascontiguousarray(vals, dtype=np.float32).reshape(s) if bc else _host_block(vals, s, n, host_instances)
+        keep.append(v)
+        arr[i].reg_index, arr[i].broadcast, arr[i].values = int(reg), 1 if bc else 0, v.ctypes.data
+    return arr, keep
 
 
 class Program:
@@ -373,6 +405,22 @@ class Program:
         bc = (C.c_int32 * max(1, n))(*[1 if c[2] else 0 for c in curves])
         self._check(self.L.fx8010_host_process_block_device_curves(self.h, _ptr(d_in), _ptr(d_out), n_samples, names, ptrs, bc, n, stream),
                     "processBlockDeviceWithCurves")
+
+    def process_block_curves(self, x, curves, n_samples=None) -> np.ndarray:
+        """FX8010::processBlockWithCurves: x [C][S][N] (None: no input) -> [C][S][N]; curves = [(register name, ndarray, broadcast)], each
+        [S][N] float32, or [S] with broadcast.  On one device or, with `devices`, on several."""
+        if x is not None:
+            x = np.ascontiguousarray(x, dtype=np.float32).reshape(self.channels, -1, self.instances)
+            n_samples = x.shape[1]
+        out = np.zeros((self.channels, n_samples, self.instances), dtype=np.float32)
+        vals = [np.ascontiguousarray(v, dtype=np.float32).reshape(n_samples) if bc else
+                np.ascontiguousarray(v, dtype=np.float32).reshape(n_samples, self.instances) for _, v, bc in curves]
+        n = len(curves)
+        names = (C.c_char_p * max(1, n))(*[c[0].encode() for c in curves])
+        ptrs = (C.c_void_p * max(1, n))(*[v.ctypes.data for v in vals])
+        bc = (C.c_int * max(1, n))(*[1 if c[2] else 0 for c in curves])
+        self._check(self.L.fx8010_host_process_block_curves(self.h, _ptr(x), out.ctypes.data, n_samples, names, ptrs, bc, n), "processBlockWithCurves")
+        return out
 
     def process_block(self, x, n_samples=None) -> np.ndarray:
         """Batched path with host buffers: x [C][S][N] -> [C][S][N]."""
@@ -586,12 +634,33 @@ class Gpu:
         self._keep_bcast = x
         return out
 
+    def process_host_curves(self, x, curves, out=None, wait: bool = True, host_instances: int = 0, n_samples=None) -> np.ndarray:
+        """fx8010_gpu_process_batch_host_curves: x [C][S][N] (None: no input) -> out [C][S][N]; curves = [(reg_index, ndarray, broadcast)],
+        each [S][N] float32, or [S] with broadcast.  With host_instances, x, out and the per-instance curves are views of N columns of
+        C-contiguous arrays host_instances wide (e.g. big[..., lo:lo + N]).  wait=False queues the work; the arrays are kept until
+        synchronize()."""
+        if x is not None:
+            n_samples = x.shape[1]
+        x = _host_block(x, self.c * n_samples, self.n, host_instances)
+        if out is None:
+            out = np.zeros((self.c, n_samples, self.n), dtype=np.float32)
+        if host_instances:
+            _host_block(out, self.c * n_samples, self.n, host_instances)
+        else:
+            assert out.dtype == np.float32 and out.flags.c_contiguous and out.size == self.c * n_samples * self.n
+        arr, keep = _host_curves(curves, n_samples, self.n, host_instances)
+        self._check(self.L.fx8010_gpu_process_batch_host_curves(self.h, _ptr(x), _ptr(out), n_samples, C.addressof(arr), len(curves),
+                                                                host_instances, 1 if wait else 0))
+        self._pending = [] if wait else getattr(self, "_pending", []) + [(x, out, arr, keep)]
+        return out
+
     def process_host_ptr(self, in_ptr: int, out_ptr: int, n_samples: int, wait: bool = True):
         f = self.L.fx8010_gpu_process_batch_host if wait else self.L.fx8010_gpu_process_batch_host_async
         self._check(f(self.h, in_ptr, out_ptr, n_samples))
 
     def synchronize(self, stream=None):
         self._check(self.L.fx8010_gpu_synchronize(self.h, stream))
+        self._pending = []
 
     def registers(self) -> np.ndarray:
         out = np.zeros((self.dims().n_regs, self.n), dtype=np.float32)
@@ -720,8 +789,25 @@ class MultiGpu:
         self._keep_bcast = x
         return out
 
+    def process_host_curves(self, x, curves, out=None, wait: bool = True, n_samples=None) -> np.ndarray:
+        """fx8010_multi_process_batch_host_curves: x [C][S][N] over all instances (None: no input) -> out [C][S][N]; curves =
+        [(reg_index, ndarray, broadcast)], each [S][N] float32, or [S] with broadcast.  wait=False queues the work; the arrays are
+        kept until synchronize()."""
+        if x is not None:
+            x = np.ascontiguousarray(x, dtype=np.float32).reshape(self.c, -1, self.n)
+            n_samples = x.shape[1]
+        if out is None:
+            out = np.zeros((self.c, n_samples, self.n), dtype=np.float32)
+        assert out.dtype == np.float32 and out.flags.c_contiguous and out.size == self.c * n_samples * self.n
+        arr, keep = _host_curves(curves, n_samples, self.n, 0)
+        self._check(self.L.fx8010_multi_process_batch_host_curves(self.h, _ptr(x), _ptr(out), n_samples, C.addressof(arr), len(curves),
+                                                                  1 if wait else 0))
+        self._pending = [] if wait else getattr(self, "_pending", []) + [(x, out, arr, keep)]
+        return out
+
     def synchronize(self):
         self._check(self.L.fx8010_multi_synchronize(self.h))
+        self._pending = []
 
     def set_option(self, option: int, value: int):
         self._check(self.L.fx8010_multi_set_option(self.h, option, value))

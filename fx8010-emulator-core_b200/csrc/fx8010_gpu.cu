@@ -182,6 +182,7 @@ struct fx8010_gpu {
     float* d_stage_in[HOST_PIPE_BUFS] = {}; float* d_stage_out[HOST_PIPE_BUFS] = {};
     float* d_bcast[HOST_PIPE_BUFS] = {}; size_t bcast_floats = 0;     // [C][sub] staging of a broadcast input (process_batch_host_broadcast)
     size_t stage_floats = 0;
+    float* d_curve_stage[HOST_PIPE_BUFS] = {}; size_t curve_floats = 0;   // host control curves: [sub][N] per per-instance curve, then [sub] per broadcast one
     unsigned long long pipe_seq = 0;             // sub-blocks pushed through the staging buffers so far
     // tuning overrides (0 = heuristic)
     int tune_K = 0, tune_B = 0, tune_seg = 0, tune_sub = 0, tune_P = 0, use_split = 1;
@@ -1531,6 +1532,41 @@ CurveBlock curves_from(const CurveBlock& cb, int n, size_t s0, size_t N) {
     return r;
 }
 struct CurveRows { CurveBlock cv; int reg[FX8010_MAX_CONTROL_CURVES]; int n; };
+
+// The preamble of both curve calls (device and host values): checks the list and copies it into rows — FX8010_ERR_ARG changes and
+// queues nothing.  `arm`: the call will run periods.  While it runs the automated registers hold no one value: nothing may fold them
+// (interpreter encoding, plain translation — a folded STATIC voids it, once).  Afterwards they hold the last period's values, which
+// the host does not know: still not uniform.  h->tr_cv is keyed to this curve set.
+template <class Curve>
+int curves_begin(fx8010_gpu* h, const Curve* curves, int n_curves, const float* const Curve::*values, bool arm, CurveRows& rows) {
+    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && !curves))
+        return fail(h, FX8010_ERR_ARG, "the curve list is NULL or the curve count outside 0..8");
+    std::vector<int> regs((size_t)n_curves);
+    std::vector<uint8_t> bc((size_t)n_curves);
+    rows = {};
+    rows.n = n_curves;
+    for (int j = 0; j < n_curves; ++j) {
+        if (!(curves[j].*values)) return fail(h, FX8010_ERR_ARG, "control curve: the values pointer is NULL");
+        regs[j] = rows.reg[j] = curves[j].reg_index;
+        bc[j] = curves[j].broadcast ? 1 : 0;
+        rows.cv.p[j] = curves[j].*values; rows.cv.bcast[j] = bc[j];
+    }
+    {
+        std::string why;
+        if (!curves_valid(h->regs, regs, why)) return fail(h, FX8010_ERR_ARG, why);
+    }
+    if (!arm || n_curves == 0) return FX8010_OK;
+    for (int r : regs) {
+        h->reg_uniform[r] = 0;
+        if (h->enc_sensitive[r]) h->encode_dirty = true;
+        tr_touch(h, r);
+    }
+    if (h->tr_cv.cv_reg != regs || h->tr_cv.cv_bcast != bc) {
+        tr_reset(h, h->tr_cv);
+        h->tr_cv.cv_reg = regs; h->tr_cv.cv_bcast = bc; h->tr_cv.serial = false;
+    }
+    return FX8010_OK;
+}
 // Period s of every curve into its register row: the per-period path of fx8010_gpu_process_batch_curves (grid.y = curve).
 __global__ void fx_curve_rows_kernel(float* __restrict__ gpr, const CurveRows rows, int s, int N) {
     const int j = blockIdx.y;
@@ -1661,7 +1697,7 @@ void fx8010_gpu_destroy(fx8010_gpu* h) {
     if (h->ev_events) cudaEventDestroy(h->ev_events);
     if (h->ev_order) cudaEventDestroy(h->ev_order);
     for (int i = 0; i < HOST_PIPE_BUFS; ++i) {
-        cudaFree(h->d_stage_in[i]); cudaFree(h->d_stage_out[i]); cudaFree(h->d_bcast[i]);
+        cudaFree(h->d_stage_in[i]); cudaFree(h->d_stage_out[i]); cudaFree(h->d_bcast[i]); cudaFree(h->d_curve_stage[i]);
         if (h->ev_h2d[i]) cudaEventDestroy(h->ev_h2d[i]);
         if (h->ev_comp[i]) cudaEventDestroy(h->ev_comp[i]);
         if (h->ev_d2h[i]) cudaEventDestroy(h->ev_d2h[i]);
@@ -1936,21 +1972,11 @@ int fx8010_gpu_process_batch_events(fx8010_gpu* h, const float* d_in, float* d_o
 int fx8010_gpu_process_batch_curves(fx8010_gpu* h, const float* d_in, float* d_out, int n_samples,
                                     const fx8010_control_curve* curves, int n_curves, void* stream) {
     FX_NEED_PROGRAM(h);
-    if (!d_out || n_samples < 0 || n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && !curves))
-        return fail(h, FX8010_ERR_ARG, "d_out or the curve list is NULL, n_samples negative, or the curve count outside 0..8");
-    std::vector<int> regs((size_t)n_curves);
-    std::vector<uint8_t> bc((size_t)n_curves);
-    CurveRows rows = {};
-    rows.n = n_curves;
-    for (int j = 0; j < n_curves; ++j) {
-        if (!curves[j].d_values) return fail(h, FX8010_ERR_ARG, "control curve: d_values is NULL");
-        regs[j] = rows.reg[j] = curves[j].reg_index;
-        bc[j] = curves[j].broadcast ? 1 : 0;
-        rows.cv.p[j] = curves[j].d_values; rows.cv.bcast[j] = bc[j];
-    }
+    if (!d_out || n_samples < 0) return fail(h, FX8010_ERR_ARG, "d_out is NULL or n_samples negative");
+    CurveRows rows;
     {
-        std::string why;
-        if (!curves_valid(h->regs, regs, why)) return fail(h, FX8010_ERR_ARG, why);
+        const int rc = curves_begin(h, curves, n_curves, &fx8010_control_curve::d_values, n_samples > 0, rows);
+        if (rc) return rc;
     }
     if (n_samples == 0) return FX8010_OK;
     cudaStream_t st = (cudaStream_t)stream;
@@ -1961,17 +1987,6 @@ int fx8010_gpu_process_batch_curves(fx8010_gpu* h, const float* d_in, float* d_o
         if (rc) return rc;
     }
     h->chain.clear();                 // every launch of the call waits for its predecessor at its start: a curve may be earlier work's output
-    // While the call runs the automated registers hold no one value: nothing may fold them (interpreter encoding, plain translation — a
-    // folded STATIC voids it, once).  Afterwards they hold the last period's values, which the host does not know: still not uniform.
-    for (int r : regs) {
-        h->reg_uniform[r] = 0;
-        if (h->enc_sensitive[r]) h->encode_dirty = true;
-        tr_touch(h, r);
-    }
-    if (h->tr_cv.cv_reg != regs || h->tr_cv.cv_bcast != bc) {
-        tr_reset(h, h->tr_cv);
-        h->tr_cv.cv_reg = regs; h->tr_cv.cv_bcast = bc; h->tr_cv.serial = false;
-    }
     return launch_curves(h, d_in, d_out, cs, n_samples, rows, st);
 }
 
@@ -2034,15 +2049,20 @@ static __global__ void fx_broadcast_kernel(const float* __restrict__ src, float*
 
 // host_n: instances per row of the HOST buffers (>= N: this handle's columns are a slice of a wider [channel][sample][instance] block)
 // bcast: `in` holds ONE value per channel and sample period ([channel][sample]); it is copied as it is and spread over the instances on the device
-static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_samples, bool wait, size_t host_n = 0, bool bcast = false) {
+// cv: control curves in HOST memory (curves_begin has checked and armed them): a per-instance curve is [n_samples][host_n] from this handle's
+// first column, a broadcast one [n_samples]; each sub-block's rows are staged like its inputs and the sub-block runs launch_curves
+static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_samples, bool wait, size_t host_n = 0, bool bcast = false,
+                             const CurveRows* cv = nullptr) {
     FX_NEED_PROGRAM(h);
     if (!out || n_samples < 0) return fail(h, FX8010_ERR_ARG, "out is NULL or n_samples negative");
     if (n_samples == 0) return FX8010_OK;
     const size_t N = (size_t)h->N, C = (size_t)h->C;
     if (host_n == 0) host_n = N;
     if (host_n < N) return fail(h, FX8010_ERR_ARG, "host row length below the instance count");
-    // sub-block: ~16 MiB of samples per channel set
-    long sub = h->tune_sub ? h->tune_sub : (long)((16u << 20) / (4 * N * C));     // (cfg2 end to end: 256-sample sub-blocks 0.446 ms per block, 512 0.396, 1 024 0.380)
+    size_t n_pi = 0, n_bc = 0;                   // per-instance and broadcast curves
+    for (int j = 0; cv && j < cv->n; ++j) ++(cv->cv.bcast[j] ? n_bc : n_pi);
+    // sub-block: ~16 MiB of samples and per-instance curve values per buffer set
+    long sub = h->tune_sub ? h->tune_sub : (long)((16u << 20) / (4 * N * (C + n_pi)));     // (cfg2 end to end: 256-sample sub-blocks 0.446 ms per block, 512 0.396, 1 024 0.380)
     sub = std::max<long>(8, sub / 8 * 8);
     sub = std::min<long>(sub, n_samples);
     const size_t need = C * (size_t)sub * N;
@@ -2067,10 +2087,27 @@ static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_s
         for (int i = 0; i < HOST_PIPE_BUFS; ++i) FX_CUDA(h, cudaMalloc(&h->d_bcast[i], sizeof(float) * C * sub));
         h->bcast_floats = (size_t)(C * sub);
     }
+    // Curve j's staging in each buffer set: the per-instance curves at k * sub * N floats (16-byte aligned whenever N % 4 == 0, as the
+    // streaming kernels need; route() takes any other launch to the serial kernel or period by period), then the broadcast ones.
+    size_t cv_off[FX8010_MAX_CONTROL_CURVES] = {};
+    if (cv) {
+        size_t k_pi = 0, k_bc = 0;
+        for (int j = 0; j < cv->n; ++j) cv_off[j] = cv->cv.bcast[j] ? n_pi * sub * N + (k_bc++) * sub : (k_pi++) * sub * N;
+        const size_t cv_need = (size_t)sub * (n_pi * N + n_bc);
+        if (cv_need > h->curve_floats) {
+            const int rc = sync_all(h);
+            if (rc) return rc;
+            for (int i = 0; i < HOST_PIPE_BUFS; ++i) { cudaFree(h->d_curve_stage[i]); h->d_curve_stage[i] = nullptr; }
+            h->curve_floats = 0;
+            for (int i = 0; i < HOST_PIPE_BUFS; ++i) FX_CUDA(h, cudaMalloc(&h->d_curve_stage[i], sizeof(float) * cv_need));
+            h->curve_floats = cv_need;
+        }
+    }
     {   // earlier device-side batches come first
         const int rc = order_on(h, h->s_comp);
         if (rc) return rc;
     }
+    if (cv) h->chain.clear();       // every curve launch waits for its predecessor at its start (as in fx8010_gpu_process_batch_curves)
     // pipe_seq counts sub-blocks over the life of the staging buffers, so that asynchronous calls chain:
     // sub-block q reuses the buffers of sub-block q - HOST_PIPE_BUFS once those have been consumed / drained
     for (long s0 = 0; s0 < n_samples; s0 += sub, ++h->pipe_seq) {
@@ -2089,6 +2126,22 @@ static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_s
                     FX_CUDA(h, cudaMemcpy2DAsync(h->d_stage_in[buf] + c * (size_t)sub * N, sizeof(float) * N, in + (c * (size_t)n_samples + s0) * host_n,
                                                  sizeof(float) * host_n, sizeof(float) * N, (size_t)len, cudaMemcpyHostToDevice, h->s_h2d));
             }
+        CurveRows staged = {};
+        if (cv) {                   // this sub-block's rows of every curve, on the stream and behind the same events as its inputs
+            staged = *cv;
+            for (int j = 0; j < cv->n; ++j) {
+                float* dst = h->d_curve_stage[buf] + cv_off[j];
+                const float* src = cv->cv.p[j];
+                staged.cv.p[j] = dst;
+                if (cv->cv.bcast[j])
+                    FX_CUDA(h, cudaMemcpyAsync(dst, src + s0, sizeof(float) * len, cudaMemcpyHostToDevice, h->s_h2d));
+                else if (host_n == N)
+                    FX_CUDA(h, cudaMemcpyAsync(dst, src + (size_t)s0 * N, sizeof(float) * len * N, cudaMemcpyHostToDevice, h->s_h2d));
+                else
+                    FX_CUDA(h, cudaMemcpy2DAsync(dst, sizeof(float) * N, src + (size_t)s0 * host_n, sizeof(float) * host_n, sizeof(float) * N, (size_t)len,
+                                                 cudaMemcpyHostToDevice, h->s_h2d));
+            }
+        }
         FX_CUDA(h, cudaEventRecord(h->ev_h2d[buf], h->s_h2d));
         FX_CUDA(h, cudaStreamWaitEvent(h->s_comp, h->ev_h2d[buf], 0));
         if (h->pipe_seq >= HOST_PIPE_BUFS) FX_CUDA(h, cudaStreamWaitEvent(h->s_comp, h->ev_d2h[buf], 0));    // stage_out[buf] drained
@@ -2100,7 +2153,9 @@ static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_s
             }
             FX_CUDA(h, cudaGetLastError());
         }
-        const int rc = launch_block(h, in ? h->d_stage_in[buf] : nullptr, h->d_stage_out[buf], (size_t)sub * N, (size_t)sub * N, (int)len, h->s_comp, true);   // (the internal stream carries this handle's launches only)
+        const float* d_in = in ? h->d_stage_in[buf] : nullptr;
+        const int rc = cv ? launch_curves(h, d_in, h->d_stage_out[buf], (size_t)sub * N, (int)len, staged, h->s_comp)
+                          : launch_block(h, d_in, h->d_stage_out[buf], (size_t)sub * N, (size_t)sub * N, (int)len, h->s_comp, true);   // (the internal stream carries this handle's launches only)
         if (rc) return rc;
         FX_CUDA(h, cudaEventRecord(h->ev_comp[buf], h->s_comp));
         FX_CUDA(h, cudaStreamWaitEvent(h->s_d2h, h->ev_comp[buf], 0));
@@ -2129,6 +2184,16 @@ int fx8010_gpu_process_batch_host_slice(fx8010_gpu* h, const float* in, float* o
 }
 int fx8010_gpu_process_batch_host_broadcast(fx8010_gpu* h, const float* in, float* out, int n_samples, size_t host_instances, int wait) {
     return process_host_impl(h, in, out, n_samples, wait != 0, host_instances, true);
+}
+int fx8010_gpu_process_batch_host_curves(fx8010_gpu* h, const float* in, float* out, int n_samples, const fx8010_host_curve* curves, int n_curves,
+                                         size_t host_instances, int wait) {
+    FX_NEED_PROGRAM(h);
+    if (!out || n_samples < 0) return fail(h, FX8010_ERR_ARG, "out is NULL or n_samples negative");
+    if (host_instances != 0 && host_instances < (size_t)h->N) return fail(h, FX8010_ERR_ARG, "host row length below the instance count");
+    CurveRows rows;
+    const int rc = curves_begin(h, curves, n_curves, &fx8010_host_curve::values, n_samples > 0, rows);
+    if (rc) return rc;
+    return process_host_impl(h, in, out, n_samples, wait != 0, host_instances, false, n_curves > 0 ? &rows : nullptr);
 }
 
 int fx8010_gpu_synchronize(fx8010_gpu* h, void* stream) {

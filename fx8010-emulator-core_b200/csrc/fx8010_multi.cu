@@ -19,7 +19,7 @@
 namespace {
 
 struct Shard {
-    int device = 0, lo = 0, hi = 0;
+    int g = 0, device = 0, lo = 0, hi = 0;
     fx8010_gpu* h = nullptr;
     std::thread th;
     // job hand-off
@@ -101,7 +101,7 @@ int fx8010_multi_create(const int* devices, int n_devices, int n_instances, int 
     m->N = n_instances; m->C = n_channels;
     for (int g = 0; g < n_devices; ++g) {
         Shard* s = new Shard();
-        s->device = devices[g];
+        s->g = g; s->device = devices[g];
         fx8010_multi_shard_range(n_instances, g, n_devices, &s->lo, &s->hi);
         const int rc = fx8010_gpu_create(s->device, s->hi - s->lo, n_channels, &s->h);
         if (rc) {
@@ -170,6 +170,28 @@ int fx8010_multi_process_batch_host_broadcast(fx8010_multi* m, const float* in, 
     if (!m || !out || n_samples < 0) return FX8010_ERR_ARG;
     const size_t N = (size_t)m->N;
     return run_all(m, [=](Shard& s) { return fx8010_gpu_process_batch_host_broadcast(s.h, in, out + s.lo, n_samples, N, wait); });
+}
+
+void fx8010_multi_shard_curves(const fx8010_host_curve* curves, int n_curves, int n_total, int g, int G, fx8010_host_curve* out) {
+    int lo = 0;
+    fx8010_multi_shard_range(n_total, g, G, &lo, nullptr);
+    for (int j = 0; j < n_curves; ++j) {
+        out[j] = curves[j];
+        if (!curves[j].broadcast && curves[j].values) out[j].values = curves[j].values + lo;
+    }
+}
+
+int fx8010_multi_process_batch_host_curves(fx8010_multi* m, const float* in, float* out, int n_samples, const fx8010_host_curve* curves, int n_curves,
+                                           int wait) {
+    if (!m || !out || n_samples < 0 || n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && !curves)) return FX8010_ERR_ARG;
+    const size_t N = (size_t)m->N;
+    const int G = (int)m->shards.size();
+    // Every shard checks the list before it queues anything, against the same program: a list one shard refuses, all refuse.
+    return run_all(m, [=](Shard& s) {
+        fx8010_host_curve mine[FX8010_MAX_CONTROL_CURVES];
+        fx8010_multi_shard_curves(curves, n_curves, m->N, s.g, G, mine);
+        return fx8010_gpu_process_batch_host_curves(s.h, in ? in + s.lo : nullptr, out + s.lo, n_samples, mine, n_curves, N, wait);
+    });
 }
 
 int fx8010_multi_set_option(fx8010_multi* m, int option, int value) {

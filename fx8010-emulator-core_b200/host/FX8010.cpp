@@ -134,6 +134,18 @@ void FX8010::processBlockDeviceWithCurves(const float* d_in, float* d_out, int n
     check(fx8010_gpu_process_batch_curves(gpu_, d_in, d_out, n_samples, cv.data(), (int)cv.size(), stream), "process_batch_curves");
 }
 
+void FX8010::processBlockWithCurves(const float* in, float* out, int n_samples, const std::vector<HostCurve>& curves) {
+    ensureUploaded();
+    std::vector<fx8010_host_curve> cv;
+    for (const HostCurve& c : curves) {
+        const int reg = front_.findRegister(c.key);
+        if (reg < 0) throw std::runtime_error("FX8010: unknown register '" + c.key + "'");
+        cv.push_back(fx8010_host_curve{reg, c.broadcast ? 1 : 0, c.values});
+    }
+    if (multi_) check(fx8010_multi_process_batch_host_curves(multi_, in, out, n_samples, cv.data(), (int)cv.size(), 1), "process_batch_host_curves");
+    else check(fx8010_gpu_process_batch_host_curves(gpu_, in, out, n_samples, cv.data(), (int)cv.size(), 0, 1), "process_batch_host_curves");
+}
+
 void FX8010::processBlockDevicePlanar(const float* d_in, float* d_out, int n_samples, void* stream) {
     ensureUploaded();
     if (multi_) throw std::runtime_error("FX8010 (B200): device-pointer members need a single device");

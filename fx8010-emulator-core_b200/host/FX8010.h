@@ -52,8 +52,8 @@ public:
     // ---- batched extension ------------------------------------------------------------------------
     FX8010(int numChannels, int numInstances, int device);
     // numInstances spread over several GPUs of one box (contiguous instance ranges, include/fx8010_multi.h): the host-buffer
-    // members (process, processBlock, set/getRegisterValue(s), the counters) work as on one device and gather into the
-    // caller's buffers; the device-pointer members have no single device to refer to and throw
+    // members (process, processBlock, processBlockWithCurves, set/getRegisterValue(s), the counters) work as on one device and
+    // gather into the caller's buffers; the device-pointer members have no single device to refer to and throw
     FX8010(int numChannels, int numInstances, const std::vector<int>& devices);
     bool loadText(const std::string& source);
     void setRelaxedSyntax(bool on) { front_.setRelaxed(on); }   // accept the README's forms too (see fx8010_frontend.h)
@@ -76,6 +76,12 @@ public:
     // sample period s; DEVICE buffers, asynchronous on `stream`; throws on an unknown name
     struct Curve { std::string key; const float* d_values; bool broadcast; };
     void processBlockDeviceWithCurves(const float* d_in, float* d_out, int n_samples, const std::vector<Curve>& curves, void* stream);
+    // the same automation with HOST buffers, on one device or several: `key` takes values[s] (broadcast, values[n_samples]) or
+    // values[s * numInstances + i] (values[n_samples][numInstances]) right before sample period s; in / out as in processBlock; each
+    // pipelined sub-block copies its rows of the curves to the device with its inputs (include/fx8010_gpu.h,
+    // fx8010_gpu_process_batch_host_curves); returns when `out` is complete; throws on an unknown name
+    struct HostCurve { std::string key; const float* values; bool broadcast; };
+    void processBlockWithCurves(const float* in, float* out, int n_samples, const std::vector<HostCurve>& curves);
     // DEVICE buffers laid out [channel][instance][sample] (planar audio), asynchronous on `stream`
     void processBlockDevicePlanar(const float* d_in, float* d_out, int n_samples, void* stream);
     // program translator (include/fx8010_gpu.h, FX8010_OPT_TRANSLATE): 0 interpreter kernels only, 1 compile in the background and switch

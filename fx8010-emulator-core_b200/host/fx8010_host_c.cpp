@@ -128,6 +128,14 @@ int fx8010_host_process_block_device_curves(fx8010_host* h, const float* d_in, f
         h->fx.processBlockDeviceWithCurves(d_in, d_out, n_samples, cv, stream);
     });
 }
+int fx8010_host_process_block_curves(fx8010_host* h, const float* in, float* out, int n_samples, const char* const* names, const float* const* values,
+                                     const int* broadcast, int n_curves) {
+    return guarded(h, [&] {
+        std::vector<Klangraum::FX8010::HostCurve> cv;
+        for (int j = 0; j < n_curves; ++j) cv.push_back(Klangraum::FX8010::HostCurve{names[j], values[j], broadcast[j] != 0});
+        h->fx.processBlockWithCurves(in, out, n_samples, cv);
+    });
+}
 int fx8010_host_instruction_counter(fx8010_host* h) {
     int v = 0;
     guarded(h, [&] { v = h->fx.getInstructionCounter(); });

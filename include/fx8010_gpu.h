@@ -232,6 +232,24 @@ typedef struct fx8010_control_curve {
 FX8010_API int fx8010_gpu_process_batch_curves(fx8010_gpu* h, const float* d_in, float* d_out, int n_samples,
                                                const fx8010_control_curve* curves, int n_curves, void* stream);
 
+/* The same automation for the host-buffer path: curve values in HOST memory (pageable or page-locked, float32). */
+typedef struct fx8010_host_curve {
+    int32_t reg_index;     /* a CONTROL or STATIC register                                                                       */
+    int32_t broadcast;     /* 0: values is [n_samples][host_instances], this handle's first column at `values`;                  */
+                           /* != 0: [n_samples], one value for every instance                                                    */
+    const float* values;   /* HOST pointer                                                                                       */
+} fx8010_host_curve;
+/* fx8010_gpu_process_batch_host_slice with control curves: bit for bit, in outputs and in the whole final state, what
+ * fx8010_gpu_process_batch_curves gives on device copies of the same buffers (the same definition: set_controls(reg_j, curve_j[s]) before
+ * every period s).  `in`, `out` and host_instances (0 = n_instances) mean what they mean in the _slice form.  Each sub-block of the
+ * pipeline copies its rows of every curve host->device together with its inputs and runs the curve kernels on them, so a per-instance
+ * curve adds 4 * n_instances bytes per period to the PCIe traffic (a broadcast one 4 bytes) and shortens the sub-blocks to keep about
+ * 16 MiB of staging per buffer set.  wait == 0 queues the work like the _async form: `in`, `out` and every `values` array must then stay
+ * untouched until fx8010_gpu_synchronize(h, NULL).  FX8010_ERR_ARG, with nothing queued, for the lists fx8010_gpu_process_batch_curves
+ * refuses and for host_instances below n_instances.  With n_curves == 0 it is fx8010_gpu_process_batch_host_slice. */
+FX8010_API int fx8010_gpu_process_batch_host_curves(fx8010_gpu* h, const float* in, float* out, int n_samples,
+                                                    const fx8010_host_curve* curves, int n_curves, size_t host_instances, int wait);
+
 /* fx8010_gpu_process_batch for PLANAR audio buffers, as an audio host keeps them: DEVICE pointers,
  * [n_channels][n_instances][n_samples] float32 (one contiguous block of samples per instance and channel).
  * The [sample][instance] layout the interpreter streams is produced and undone by tiled transposes on `stream`. */

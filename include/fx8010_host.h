@@ -66,6 +66,10 @@ FX8010_API int fx8010_host_process_block(fx8010_host* h, const float* in, float*
 /* processBlockDeviceWithCurves(): DEVICE buffers, curve j drives register names[j] (d_values[j], broadcast[j]: see fx8010_gpu_process_batch_curves) */
 FX8010_API int fx8010_host_process_block_device_curves(fx8010_host* h, const float* d_in, float* d_out, int n_samples, const char* const* names,
                                                        const float* const* d_values, const int* broadcast, int n_curves, void* stream);
+/* processBlockWithCurves(): host buffers as in processBlock, curve j drives register names[j] (values[j]: HOST pointer, broadcast[j]: see
+ * fx8010_gpu_process_batch_host_curves); on one device or several */
+FX8010_API int fx8010_host_process_block_curves(fx8010_host* h, const float* in, float* out, int n_samples, const char* const* names,
+                                                const float* const* values, const int* broadcast, int n_curves);
 FX8010_API int fx8010_host_instruction_counter(fx8010_host* h);                 /* getInstructionCounter */
 FX8010_API unsigned long long fx8010_host_instruction_counter_total(fx8010_host* h);
 FX8010_API fx8010_gpu* fx8010_host_gpu(fx8010_host* h);                          /* NULL on failure */

@@ -50,6 +50,16 @@ FX8010_API int fx8010_multi_process_batch_host(fx8010_multi* m, const float* in,
 FX8010_API int fx8010_multi_process_batch_host_async(fx8010_multi* m, const float* in, float* out, int n_samples);
 /* One input signal for all instances: `in` is [n_channels][n_samples] (fx8010_gpu_process_batch_host_broadcast per shard). */
 FX8010_API int fx8010_multi_process_batch_host_broadcast(fx8010_multi* m, const float* in, float* out, int n_samples, int wait);
+/* Sample-accurate control curves from host memory (fx8010_gpu_process_batch_host_curves per shard): in / out as for
+ * fx8010_multi_process_batch_host; a per-instance curve is [n_samples][n_instances] over ALL instances, and shard g reads its own
+ * columns through a strided copy; a broadcast curve ([n_samples]) goes to every shard as it is.  The same curve list reaches every
+ * shard, all with the same program, and each checks it before queuing: a refused list (FX8010_ERR_ARG) leaves every shard untouched.
+ * wait == 0 queues the work: in, out and every values array stay untouched until fx8010_multi_synchronize. */
+FX8010_API int fx8010_multi_process_batch_host_curves(fx8010_multi* m, const float* in, float* out, int n_samples,
+                                                      const fx8010_host_curve* curves, int n_curves, int wait);
+/* The curve list shard g of G (over n_total instances) passes to its handle: a per-instance curve's values moved to the shard's first
+ * column (fx8010_multi_shard_range), a broadcast one as it is.  out: n_curves entries.  Pure function, no device needed. */
+FX8010_API void fx8010_multi_shard_curves(const fx8010_host_curve* curves, int n_curves, int n_total, int g, int G, fx8010_host_curve* out);
 FX8010_API int fx8010_multi_synchronize(fx8010_multi* m);
 /* fx8010_gpu_set_option on every shard (FX8010_OPT_STREAM_EXCLUSIVE, FX8010_OPT_TRANSLATE). */
 FX8010_API int fx8010_multi_set_option(fx8010_multi* m, int option, int value);
