@@ -140,6 +140,13 @@ GPU_SYMBOLS = {
     "fx8010_kernel_cache_set_dir": (C.c_int, [C.c_char_p]),
     "fx8010_kernel_cache_precompile": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
     "fx8010_kernel_cache_get_stats": (C.c_int, [C.POINTER(CKernelCacheStats)]),
+    "fx8010_chain_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
+    "fx8010_chain_destroy": (None, [C.c_void_p]),
+    "fx8010_chain_process_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "fx8010_chain_status": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_ulonglong), C.POINTER(C.c_int),
+                                      C.POINTER(C.c_int), C.c_char_p, C.c_size_t]),
+    "fx8010_chain_last_error": (C.c_char_p, [C.c_void_p]),
+    "fx8010_translate_source_chain": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_char_p, C.c_size_t, C.c_int, C.POINTER(C.c_int)]),
 }
 
 MULTI_SYMBOLS = {
@@ -202,6 +209,10 @@ HOST_SYMBOLS = {
                                                           C.c_void_p, C.c_int, C.c_void_p]),
     "fx8010_host_process_block_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_char_p), C.c_void_p,
                                                    C.c_void_p, C.c_int]),
+    "fx8010_host_chain_create": (C.c_void_p, [C.c_void_p, C.c_int]),
+    "fx8010_host_chain_destroy": (None, [C.c_void_p]),
+    "fx8010_host_chain_process_block_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "fx8010_host_chain_last_error": (C.c_char_p, [C.c_void_p]),
 }
 
 
@@ -431,6 +442,11 @@ class Program:
         self._check(self.L.fx8010_host_process_block(self.h, _ptr(x), out.ctypes.data, n_samples), "processBlock")
         return out
 
+    def chain(self, later):
+        """Klangraum::FX8010Chain of this object followed by the Programs `later`: a callable (d_in, d_out, n_samples, stream=None) that runs
+        processBlockDevice, with .close().  Close it before the objects."""
+        return ProgramChain([self] + list(later))
+
     @property
     def instruction_counter(self) -> int:
         return self.L.fx8010_host_instruction_counter(self.h)
@@ -438,6 +454,29 @@ class Program:
     @property
     def instruction_counter_total(self) -> int:
         return self.L.fx8010_host_instruction_counter_total(self.h)
+
+
+class ProgramChain:
+    """Klangraum::FX8010Chain through include/fx8010_host.h (see Program.chain)."""
+
+    def __init__(self, programs):
+        self.L = host_lib()
+        self.programs = list(programs)
+        arr = (C.c_void_p * max(1, len(self.programs)))(*[p.h for p in self.programs])
+        self.h = self.L.fx8010_host_chain_create(arr, len(self.programs))
+        if not self.h:
+            raise FxError(1, self.L.fx8010_host_chain_last_error(None).decode())
+
+    def __call__(self, d_in, d_out, n_samples: int, stream=None):
+        if self.L.fx8010_host_chain_process_block_device(self.h, _ptr(d_in), _ptr(d_out), n_samples, stream):
+            raise FxError(2, self.L.fx8010_host_chain_last_error(self.h).decode())
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.fx8010_host_chain_destroy(self.h)
+            self.h = None
+
+    __del__ = close
 
 
 def translate_source(prog: "Program", channels: int = 1, compile_check: bool = False, instances: int = 1):
@@ -466,6 +505,22 @@ def translate_source_curves(prog: "Program", curves, channels: int = 1, compile_
     buf = C.create_string_buffer(int(n) + 1)
     cub = C.c_int(0)
     L.fx8010_translate_source_curves(prog.image_ptr(), instances, channels, regs, bc, k, buf, int(n) + 1, 1 if compile_check else 0, C.byref(cub))
+    return buf.value.decode(), (cub.value if compile_check else None)
+
+
+def translate_source_chain(progs, channels: int = 1, compile_check: bool = False, instances: int = 1):
+    """The source of the fused kernel of a chain of the decoded programs `progs` (fx8010_translate_source_chain; no device needed).
+    Returns (source or None when some stage is not stateless, CUBIN size when compile_check else None)."""
+    L = gpu_lib()
+    imgs = (C.c_void_p * max(1, len(progs)))(*[p.image_ptr() for p in progs])
+    n = L.fx8010_translate_source_chain(imgs, len(progs), instances, channels, None, 0, 0, None)
+    if n == -1:
+        raise ValueError("bad image list")
+    if n < 0:
+        return None, None
+    buf = C.create_string_buffer(int(n) + 1)
+    cub = C.c_int(0)
+    L.fx8010_translate_source_chain(imgs, len(progs), instances, channels, buf, int(n) + 1, 1 if compile_check else 0, C.byref(cub))
     return buf.value.decode(), (cub.value if compile_check else None)
 
 
@@ -721,6 +776,43 @@ class Gpu:
         i = CLaunchInfo()
         self._check(self.L.fx8010_gpu_get_launch_info(self.h, C.byref(i)))
         return i
+
+
+MAX_CHAIN_STAGES = 8
+
+
+class Chain:
+    """Several Gpu handles run one after another within every sample period (include/fx8010_gpu.h, fx8010_chain_*).  Close it before
+    the handles."""
+
+    def __init__(self, stages):
+        self.L = gpu_lib()
+        self.stages = list(stages)
+        arr = (C.c_void_p * max(1, len(self.stages)))(*[g.h.value for g in self.stages])
+        h = C.c_void_p()
+        rc = self.L.fx8010_chain_create(arr, len(self.stages), C.byref(h))
+        if rc != 0:
+            raise FxError(rc, self.L.fx8010_chain_last_error(None).decode())
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.fx8010_chain_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+    def process_batch(self, d_in, d_out, n: int, stream=None):
+        rc = self.L.fx8010_chain_process_batch(self.h, _ptr(d_in), _ptr(d_out), n, stream)
+        if rc != 0:
+            raise FxError(rc, self.L.fx8010_chain_last_error(self.h).decode())
+
+    def status(self) -> dict:
+        st, fused, regs, loc, launches = C.c_int(0), C.c_int(0), C.c_int(0), C.c_int(0), C.c_ulonglong(0)
+        msg = C.create_string_buffer(4096)
+        self.L.fx8010_chain_status(self.h, C.byref(st), C.byref(fused), C.byref(launches), C.byref(regs), C.byref(loc), msg, 4096)
+        return {"state": st.value, "fused_last": fused.value, "launches": int(launches.value), "regs_per_thread": regs.value,
+                "local_bytes": loc.value, "message": msg.value.decode(errors="replace")}
 
 
 class MultiGpu:

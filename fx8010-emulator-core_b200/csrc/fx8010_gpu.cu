@@ -77,7 +77,8 @@ struct Translation {
     void* fn = nullptr;                          // CUfunction of the translated kernel
     KernelDigest key{}; bool attached = false;   // its entry in the per-process kernel cache (reference-counted)
     int regs = 0, local = 0;                     // its registers per thread / local-memory bytes (spills)
-    int kind = 0;                                // 0 serial kernel, 1 streaming kernel (stateless program), 2 streaming kernel with TRAM (time-cut delay line)
+    int kind = 0;                                // 0 serial kernel, 1 streaming kernel (stateless program), 2 streaming kernel with TRAM (time-cut delay line),
+                                                 // 3 streaming kernel of a program chain (fx8010_chain)
     int lanes = 1;                               // (serial kernel) instances per thread
     int ring_floats = 0;                         // (serial kernel) floats of the shared-memory input ring per thread
     std::shared_ptr<void> job;                   // the running compilation
@@ -193,6 +194,7 @@ struct fx8010_gpu {
     Translation tr_cv;                           // the translation for the most recent set of control curves (fx8010_gpu_process_batch_curves)
     const Translation* tr_gen = nullptr;         // the translation being generated: its curve registers are never folded
     std::vector<uint8_t> tr_volatile;            // per register: the host changed it after load — never folded again
+    unsigned long long tr_epoch = 0;             // bumped whenever both translations are voided (load_program): chains over this handle regenerate
     std::string kc_env_dir;                      // FX8010_KERNEL_CACHE when the handle was created (the disk store; "" = none)
     std::string err;
     fx8010_launch_info info = {};
@@ -1365,6 +1367,20 @@ int tr_launch(fx8010_gpu* h, const Translation& T, const float* in, float* out, 
     return tr_drive(h, T, L, 1, st, args);
 }
 
+// Time segments of a launch of a translated streaming kernel (fx_translated_sl, fx_translated_chain) over nb blocks of ns periods, gx thread
+// blocks of B threads per segment row: every thread takes `seg_len` samples (whole 4-sample load groups).  Short segments mean more threads — a
+// lone block ramps up faster (cfg2, one block per call: 11 us at 8 samples, 15-19 at 16-32) — long ones amortise the per-thread start-up once
+// the launch holds a couple of waves anyway (cfg2, 20 blocks per launch: 6.3 us per block at 8, 5.9 at 32): the shortest power of two that
+// keeps the launch within about 2.5 full waves of warps.
+void sl_segments(const fx8010_gpu* h, int gx, int B, int ns, int nb, int& seg_len, int& n_seg) {
+    seg_len = 8;
+    const long warps_per_row = ((long)gx * B + 31) / 32;
+    while (seg_len < ns && warps_per_row * ((ns + seg_len - 1) / seg_len) * nb > (long)h->num_sms * 64 * 5 / 2) seg_len <<= 1;
+    if (env_int("FX8010_TUNE_SEGLEN") > 0) seg_len = env_int("FX8010_TUNE_SEGLEN");
+    n_seg = (ns + seg_len - 1) / seg_len;
+    while ((long)n_seg * nb > 65535) { seg_len <<= 1; n_seg = (ns + seg_len - 1) / seg_len; }
+}
+
 // nb consecutive blocks of a stateless program (or one stretch of a delay line) on its translated streaming kernel (late_wait as
 // launch_blocks computes it).  `cv`: the call's control curves (the automated translation only; nb == 1).  L: the geometry it ran with.
 int tr_sl_launch(fx8010_gpu* h, const Translation& T, const float* const* ins, float* const* outs, int nb, size_t in_cs, size_t out_cs, int ns, cudaStream_t st,
@@ -1375,16 +1391,8 @@ int tr_sl_launch(fx8010_gpu* h, const Translation& T, const float* const* ins, f
     int B = 128;
     if (h->tune_B) B = h->tune_B;
     const int gx = (N / K + B - 1) / B;
-    // time segments: every thread takes `seg_len` samples (whole 4-sample load groups).  Short segments mean more threads — a lone
-    // block ramps up faster (cfg2, one block per call: 11 us at 8 samples, 15-19 at 16-32) — long ones amortise the per-thread
-    // start-up once the launch holds a couple of waves anyway (cfg2, 20 blocks per launch: 6.3 us per block at 8, 5.9 at 32):
-    // the shortest power of two that keeps the launch within about 2.5 full waves of warps.
-    int seg_len = 8;
-    const long warps_per_row = ((long)gx * B + 31) / 32;
-    while (seg_len < ns && warps_per_row * ((ns + seg_len - 1) / seg_len) * nb > (long)h->num_sms * 64 * 5 / 2) seg_len <<= 1;
-    if (env_int("FX8010_TUNE_SEGLEN") > 0) seg_len = env_int("FX8010_TUNE_SEGLEN");
-    int n_seg = (ns + seg_len - 1) / seg_len;
-    while ((long)n_seg * nb > 65535) { seg_len <<= 1; n_seg = (ns + seg_len - 1) / seg_len; }
+    int seg_len, n_seg;
+    sl_segments(h, gx, B, ns, nb, seg_len, n_seg);
     void* gpr = h->d_gpr; void* acc = h->d_acc; void* latch = h->d_latch; void* counts = h->d_counts; void* flags = h->d_flags; void* tabs = h->d_tabs;
     int ns_ = ns, nb_ = nb, N_ = N, lw = late_wait, isz = h->itram_size, xsz = h->xtram_size;
     void* ptrs = h->d_ptrs; void* itram = h->d_itram; void* xtram = h->d_xtram;
@@ -1624,7 +1632,218 @@ int sync_all(fx8010_gpu* h) {
 
 }  // namespace
 
+// A chain of stages (fx8010_chain_*): handles of one device, instance count and channel count whose programs run one after another within
+// every sample period.  Stateless stages run fused in one translated kernel (fx_translated_chain); anything else runs stage by stage through
+// the chain's own intermediate blocks, which is the definition of a chain call.
+struct fx8010_chain {
+    std::vector<fx8010_gpu*> st;
+    int device = 0;
+    Translation tr;                                  // the fused kernel (kind 3) ...
+    std::vector<unsigned long long> epoch;           // ... generated while each stage had this tr_epoch ...
+    std::vector<std::vector<uint8_t>> folded;        // ... folding these registers of each stage ...
+    std::vector<std::vector<float>> fold_value;      // ... with these values
+    float* d_mid[2] = {nullptr, nullptr};            // [C][S][N] intermediate blocks of the stage-by-stage path, used alternately
+    size_t mid_floats = 0;
+    cudaEvent_t ev = nullptr;                        // orders a stage-by-stage call after the previous one's use of d_mid on another stream
+    cudaStream_t last_stream = nullptr; bool has_last = false;
+    unsigned long long launches = 0;                 // fused launches
+    int fused_last = 0;
+    std::string why;                                 // why the last call did not run fused ("" when it did)
+    std::string err;
+};
+
+namespace {
+
+int chain_fail(fx8010_chain* c, int code, const std::string& msg) {
+    c->err = msg;
+    return code;
+}
+
+// The fused kernel still computes what its stages would: no stage reloaded, every folded register still holds its folded value in every
+// instance.  A register that no longer does is never folded again (as tr_touch decides for a handle's own translation).
+bool chain_current(fx8010_chain* c) {
+    for (size_t j = 0; j < c->st.size(); ++j) {
+        fx8010_gpu* h = c->st[j];
+        if (h->tr_epoch != c->epoch[j]) return false;
+        if (j >= c->folded.size()) continue;
+        for (size_t r = 0; r < c->folded[j].size(); ++r) {
+            if (!c->folded[j][r]) continue;
+            uint32_t a, b;
+            memcpy(&a, &c->fold_value[j][r], 4); memcpy(&b, &h->reg_value[r], 4);
+            if (h->reg_uniform[r] && a == b) continue;
+            h->tr_volatile[r] = 1;
+            return false;
+        }
+    }
+    return true;
+}
+
+// Whether the fused kernel is loaded for the chain's current stages (tr_obtain in stage 0's translation mode); c->why says why not.
+bool chain_ready(fx8010_chain* c, bool may_wait) {
+    fx8010_gpu* h0 = c->st[0];
+    if (!chain_current(c)) {
+        tr_reset(c->device, c->tr);
+        c->folded.clear(); c->fold_value.clear();
+        for (size_t j = 0; j < c->st.size(); ++j) c->epoch[j] = c->st[j]->tr_epoch;
+    }
+    if (h0->use_translate == 0) { c->why = "translation is off on stage 0 (FX8010_OPT_TRANSLATE 0)"; return false; }
+    if (c->tr.state == 0)
+        for (size_t j = 0; j < c->st.size(); ++j)
+            if (!c->st[j]->stateless) { c->tr.state = -1; c->tr.error = "stage " + std::to_string(j) + " carries state across sample periods"; break; }
+    const bool ok = tr_obtain(c->device, h0->use_translate, h0->kc_env_dir, c->tr, [&](std::string& src, std::string&) {
+        src = tr_generate_chain(std::vector<const fx8010_gpu*>(c->st.begin(), c->st.end()), c->folded);
+        c->fold_value.clear();
+        for (fx8010_gpu* h : c->st) c->fold_value.push_back(h->reg_value);
+        return true;
+    }, may_wait);
+    c->why = ok ? "" : (c->tr.state == 1 ? "the chain kernel is compiling" : c->tr.error);
+    return ok;
+}
+
+// One launch of the fused kernel: every stage's earlier work comes first (order_on), and the kernel waits at its start and never lets a
+// later launch start early, so afterwards no stage has a late-waiting launch outstanding (each one's chain is empty).
+int chain_launch(fx8010_chain* c, const float* d_in, float* d_out, int n, cudaStream_t stream) {
+    for (fx8010_gpu* h : c->st) {
+        const int rc = order_on(h, stream);
+        if (rc) return chain_fail(c, rc, h->err);
+    }
+    fx8010_gpu* h0 = c->st[0];
+    struct Stage { float* gpr; double* acc; float* latch; unsigned long long* counts; unsigned int* flags; const TableEntry* tabs; };
+    struct { Stage s[FX8010_MAX_CHAIN_STAGES]; } stages = {};
+    for (size_t j = 0; j < c->st.size(); ++j) {
+        fx8010_gpu* h = c->st[j];
+        stages.s[j] = Stage{h->d_gpr, h->d_acc, h->d_latch, h->d_counts, h->d_flags, h->d_tabs};
+    }
+    Launch L = {};
+    L.K = 4; L.B = h0->tune_B ? h0->tune_B : 128; L.P = 1;
+    L.grid_x = (h0->N / L.K + L.B - 1) / L.B;
+    sl_segments(h0, L.grid_x, L.B, n, 1, L.seg_len, L.n_seg);
+    size_t cs = (size_t)n * h0->N;
+    const void* inp = d_in; void* outp = d_out;
+    int n_ = n, N_ = h0->N;
+    void* args[] = {&stages, &inp, &outp, &cs, &cs, &n_, &L.seg_len, &N_};
+    const int rc = tr_drive(h0, c->tr, L, 1, stream, args);
+    if (rc) return chain_fail(c, rc, h0->err);
+    for (fx8010_gpu* h : c->st) { h->chain.clear(); h->tram_periods += (unsigned long long)n; }
+    c->launches++;
+    return FX8010_OK;
+}
+
+// Stage by stage: fx8010_gpu_process_batch of every stage on `stream`, stage j writing the intermediate block stage j + 1 reads.
+int chain_sequential(fx8010_chain* c, const float* d_in, float* d_out, int n, cudaStream_t stream) {
+    const size_t ns = c->st.size(), need = (size_t)c->st[0]->C * n * c->st[0]->N;
+    if (ns > 1 && need > c->mid_floats) {                 // (cudaFree waits for the device: no earlier call still uses the old blocks)
+        cudaFree(c->d_mid[0]); cudaFree(c->d_mid[1]); c->d_mid[0] = c->d_mid[1] = nullptr; c->mid_floats = 0;
+        for (int b = 0; b < 2; ++b) {
+            const cudaError_t e = cudaMalloc(&c->d_mid[b], sizeof(float) * need);
+            if (e != cudaSuccess) return chain_fail(c, FX8010_ERR_CUDA, std::string("chain intermediate blocks: ") + cudaGetErrorString(e));
+        }
+        c->mid_floats = need;
+    }
+    if (ns > 1 && c->has_last && c->last_stream != stream) {
+        if (cudaEventRecord(c->ev, c->last_stream) == cudaSuccess) {
+            const cudaError_t e = cudaStreamWaitEvent(stream, c->ev, 0);
+            if (e != cudaSuccess) return chain_fail(c, FX8010_ERR_CUDA, std::string("cudaStreamWaitEvent: ") + cudaGetErrorString(e));
+        } else {
+            cudaGetLastError();                              // that stream no longer exists: everything on the device comes first
+            const cudaError_t e = cudaDeviceSynchronize();
+            if (e != cudaSuccess) return chain_fail(c, FX8010_ERR_CUDA, std::string("cudaDeviceSynchronize: ") + cudaGetErrorString(e));
+        }
+    }
+    for (size_t j = 0; j < ns; ++j) {
+        const float* in = j ? c->d_mid[(j - 1) & 1] : d_in;
+        float* out = j + 1 == ns ? d_out : c->d_mid[j & 1];
+        const int rc = fx8010_gpu_process_batch(c->st[j], in, out, n, stream);
+        if (rc) return chain_fail(c, rc, "stage " + std::to_string(j) + ": " + c->st[j]->err);
+    }
+    c->last_stream = stream; c->has_last = true;
+    return FX8010_OK;
+}
+
+// Some instruction of h's program preloads an INPUT register (reads the call's input).
+bool reads_input(const fx8010_gpu* h) {
+    for (const fx8010_instr& in : h->instrs) {
+        bool pa, px, py; int nz;
+        pre_targets(h, in, pa, px, py, nz);
+        if (pa || px || py) return true;
+    }
+    return false;
+}
+
+}  // namespace
+
 extern "C" {
+
+int fx8010_chain_create(fx8010_gpu* const* stages, int n_stages, fx8010_chain** out) {
+    if (!out) return fail(nullptr, FX8010_ERR_ARG, "out is NULL");
+    *out = nullptr;
+    if (!stages || n_stages < 1 || n_stages > FX8010_MAX_CHAIN_STAGES) return fail(nullptr, FX8010_ERR_ARG, "the stage count must be 1..FX8010_MAX_CHAIN_STAGES");
+    for (int j = 0; j < n_stages; ++j) {
+        if (!stages[j]) return fail(nullptr, FX8010_ERR_ARG, "stage " + std::to_string(j) + " is NULL");
+        for (int k = 0; k < j; ++k) if (stages[k] == stages[j]) return fail(nullptr, FX8010_ERR_ARG, "a handle appears twice in the chain");
+        if (stages[j]->device != stages[0]->device || stages[j]->N != stages[0]->N || stages[j]->C != stages[0]->C)
+            return fail(nullptr, FX8010_ERR_ARG, "the stages differ in device, instance count or channel count");
+    }
+    cudaError_t e = cudaSetDevice(stages[0]->device);
+    fx8010_chain* c = new fx8010_chain();
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&c->ev, cudaEventDisableTiming);
+    if (e != cudaSuccess) { delete c; return fail(nullptr, FX8010_ERR_CUDA, std::string("chain: ") + cudaGetErrorString(e)); }
+    c->st.assign(stages, stages + n_stages);
+    c->device = stages[0]->device;
+    c->tr.kind = 3;
+    for (fx8010_gpu* h : c->st) c->epoch.push_back(h->tr_epoch);
+    *out = c;
+    return FX8010_OK;
+}
+
+void fx8010_chain_destroy(fx8010_chain* c) {
+    if (!c) return;
+    cudaSetDevice(c->device);
+    cudaFree(c->d_mid[0]); cudaFree(c->d_mid[1]);            // (waits for the device)
+    if (c->ev) cudaEventDestroy(c->ev);
+    tr_detach(c->device, c->tr);
+    delete c;
+}
+
+int fx8010_chain_process_batch(fx8010_chain* c, const float* d_in, float* d_out, int n_samples, void* stream) {
+    if (!c) return FX8010_ERR_ARG;
+    for (size_t j = 0; j < c->st.size(); ++j)
+        if (!c->st[j]->loaded) return chain_fail(c, FX8010_ERR_NO_PROGRAM, "stage " + std::to_string(j) + " has no program");
+    if (!d_out || n_samples < 0) return chain_fail(c, FX8010_ERR_ARG, "d_out is NULL or n_samples negative");
+    if (!d_in && reads_input(c->st[0])) return chain_fail(c, FX8010_ERR_ARG, "d_in is NULL but stage 0 reads an input");
+    if (cudaSetDevice(c->device) != cudaSuccess) return chain_fail(c, FX8010_ERR_CUDA, "cudaSetDevice failed");
+    if (n_samples == 0) return FX8010_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    fx8010_gpu* h0 = c->st[0];
+    const size_t cs = (size_t)n_samples * h0->N;
+    bool fused = false;
+    if (c->st.size() == 1) c->why = "a chain of one stage is that stage's process_batch";
+    else if (h0->N % 4) c->why = "the instance count is not a multiple of 4";
+    else if (!io_aligned(h0, 16, &d_in, &d_out, 1, cs, cs, n_samples)) c->why = "a buffer is not 16-byte aligned";
+    else fused = chain_ready(c, true);
+    c->fused_last = fused ? 1 : 0;
+    return fused ? chain_launch(c, d_in, d_out, n_samples, st) : chain_sequential(c, d_in, d_out, n_samples, st);
+}
+
+int fx8010_chain_status(fx8010_chain* c, int* state, int* fused_last, unsigned long long* launches, int* regs_per_thread, int* local_bytes,
+                        char* message, size_t message_cap) {
+    if (!c) return FX8010_ERR_ARG;
+    if (c->tr.state == 1 && cudaSetDevice(c->device) == cudaSuccess) {     // pick up a finished background compilation
+        bool loaded = true;
+        for (fx8010_gpu* h : c->st) loaded = loaded && h->loaded;
+        if (loaded) chain_ready(c, false);
+    }
+    if (state) *state = c->tr.state;
+    if (fused_last) *fused_last = c->fused_last;
+    if (launches) *launches = c->launches;
+    if (regs_per_thread) *regs_per_thread = c->tr.regs;
+    if (local_bytes) *local_bytes = c->tr.local;
+    const std::string& m = c->fused_last ? std::string() : c->why;
+    if (message && message_cap) { strncpy(message, m.c_str(), message_cap - 1); message[message_cap - 1] = 0; }
+    return FX8010_OK;
+}
+
+const char* fx8010_chain_last_error(fx8010_chain* c) { return c ? c->err.c_str() : g_create_error.c_str(); }
 
 int fx8010_gpu_create(int device, int n_instances, int n_channels, fx8010_gpu** out) {
     if (!out) return fail(nullptr, FX8010_ERR_ARG, "out is NULL");
@@ -2384,11 +2603,10 @@ int fx8010_gpu_translate_status_curves(fx8010_gpu* h, int* state, int* regs_per_
 // on cregs[n_curves] when n_curves > 0) into `src`.  0, -1 for a bad image or curve list, -2 when the program is not eligible.
 // For a freshly loaded image this is the source a handle generates at its first launch on a B200 (148 SMs), except that the developer
 // switches a handle reads when it is created (FX8010_NO_STATELESS, FX8010_NO_TSPLIT, FX8010_TR_RECUR) are not applied.
-static int translate_source_gen(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
-                                int n_curves, std::string& src) {
+// The host-side analysis of image `im` as load_program would leave it (the registers of cv_reg automated, hence not uniform) in tmp.
+// 0, or -1 for a bad image or curve list.
+static int image_handle(const fx8010_program_image* im, int n_instances, int n_channels, const std::vector<int>& cv_reg, fx8010_gpu& tmp) {
     if (!im || !im->instrs || !im->regs || im->n_instrs <= 0 || im->n_regs <= 0 || n_channels <= 0 || n_instances <= 0) return -1;
-    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && (!cregs || !cbcast))) return -1;
-    fx8010_gpu tmp;
     tmp.C = n_channels; tmp.N = n_instances;
     tmp.instrs.assign(im->instrs, im->instrs + im->n_instrs);
     tmp.regs.assign(im->regs, im->regs + im->n_regs);
@@ -2396,17 +2614,29 @@ static int translate_source_gen(const fx8010_program_image* im, int n_instances,
         if (in.opcode < 0 || in.opcode >= FX_NUM_OPCODES || in.r < 0 || in.r >= im->n_regs || in.a < 0 || in.a >= im->n_regs ||
             in.x < 0 || in.x >= im->n_regs || in.y < 0 || in.y >= im->n_regs) return -1;
     for (const fx8010_reg& r : tmp.regs) if (r.io_index < 0 || r.io_index >= n_channels) return -1;
-    Translation T;
-    for (int j = 0; j < n_curves; ++j) { T.cv_reg.push_back(cregs[j]); T.cv_bcast.push_back(cbcast[j] ? 1 : 0); }
     std::string why;
-    if (!curves_valid(tmp.regs, T.cv_reg, why)) return -1;
+    if (!curves_valid(tmp.regs, cv_reg, why)) return -1;
     tmp.itram_size = im->itram_size; tmp.xtram_size = im->xtram_size;
     tmp.reg_uniform.assign(im->n_regs, 1);
     tmp.reg_value.resize(im->n_regs);
     for (int r = 0; r < im->n_regs; ++r) tmp.reg_value[r] = im->regs[r].init_value;
-    for (int r : T.cv_reg) tmp.reg_uniform[r] = 0;            // (as fx8010_gpu_process_batch_curves leaves them)
+    for (int r : cv_reg) tmp.reg_uniform[r] = 0;              // (as fx8010_gpu_process_batch_curves leaves them)
     tmp.tr_volatile.assign(im->n_regs, 0);
     analyse(&tmp);
+    return 0;
+}
+
+// Needs no device: analyses the image as load_program would and generates the CUDA source of its translated kernel (for control curves
+// on cregs[n_curves] when n_curves > 0) into `src`.  0, -1 for a bad image or curve list, -2 when the program is not eligible.
+// For a freshly loaded image this is the source a handle generates at its first launch on a B200 (148 SMs), except that the developer
+// switches a handle reads when it is created (FX8010_NO_STATELESS, FX8010_NO_TSPLIT, FX8010_TR_RECUR) are not applied.
+static int translate_source_gen(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
+                                int n_curves, std::string& src) {
+    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && (!cregs || !cbcast))) return -1;
+    Translation T;
+    for (int j = 0; j < n_curves; ++j) { T.cv_reg.push_back(cregs[j]); T.cv_bcast.push_back(cbcast[j] ? 1 : 0); }
+    fx8010_gpu tmp;
+    if (image_handle(im, n_instances, n_channels, T.cv_reg, tmp)) return -1;
     const int kind = tr_kind(&tmp, T);
     tmp.tr_gen = n_curves ? &T : nullptr;
     if (kind == 0 && !tr_eligible(&tmp)) return -2;
@@ -2415,19 +2645,22 @@ static int translate_source_gen(const fx8010_program_image* im, int n_instances,
     tmp.tr_gen = nullptr;
     return 0;
 }
-static long long translate_source_impl(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
-                                       int n_curves, char* buf, size_t cap, int compile_check, int* regs_or_status) {
-    std::string src;
-    const int g = translate_source_gen(im, n_instances, n_channels, cregs, cbcast, n_curves, src);
-    if (g) return g;
+// Writes `src` to buf (cap bytes with the terminator) and, with compile_check, compiles it with NVRTC: *cubin_bytes = the CUBIN size or -1.
+static long long translate_source_out(const std::string& src, char* buf, size_t cap, int compile_check, int* cubin_bytes) {
     if (buf && cap) { strncpy(buf, src.c_str(), cap - 1); buf[cap - 1] = 0; }
     if (compile_check) {                                     // NVRTC -> sm_100a CUBIN (works without a GPU)
         std::vector<char> cubin; std::string log;
         const bool ok = translate_compile(src, cubin, log);
-        if (regs_or_status) *regs_or_status = ok ? (int)cubin.size() : -1;
+        if (cubin_bytes) *cubin_bytes = ok ? (int)cubin.size() : -1;
         if (!ok) fprintf(stderr, "fx8010_translate_source: %s\n", log.c_str());
     }
     return (long long)src.size();
+}
+static long long translate_source_impl(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* cregs, const int32_t* cbcast,
+                                       int n_curves, char* buf, size_t cap, int compile_check, int* regs_or_status) {
+    std::string src;
+    const int g = translate_source_gen(im, n_instances, n_channels, cregs, cbcast, n_curves, src);
+    return g ? g : translate_source_out(src, buf, cap, compile_check, regs_or_status);
 }
 long long fx8010_translate_source(const fx8010_program_image* im, int n_instances, int n_channels, char* buf, size_t cap, int compile_check, int* regs_or_status) {
     return translate_source_impl(im, n_instances, n_channels, nullptr, nullptr, 0, buf, cap, compile_check, regs_or_status);
@@ -2435,6 +2668,19 @@ long long fx8010_translate_source(const fx8010_program_image* im, int n_instance
 long long fx8010_translate_source_curves(const fx8010_program_image* im, int n_instances, int n_channels, const int32_t* regs, const int32_t* broadcast,
                                          int n_curves, char* buf, size_t cap, int compile_check, int* cubin_bytes) {
     return translate_source_impl(im, n_instances, n_channels, regs, broadcast, n_curves, buf, cap, compile_check, cubin_bytes);
+}
+
+long long fx8010_translate_source_chain(const fx8010_program_image* const* images, int n_stages, int n_instances, int n_channels, char* buf,
+                                        size_t cap, int compile_check, int* cubin_bytes) {
+    if (!images || n_stages < 1 || n_stages > FX8010_MAX_CHAIN_STAGES) return -1;
+    std::vector<fx8010_gpu> tmp((size_t)n_stages);
+    for (int j = 0; j < n_stages; ++j)
+        if (image_handle(images[j], n_instances, n_channels, {}, tmp[j])) return -1;
+    for (const fx8010_gpu& h : tmp) if (!h.stateless) return -2;
+    std::vector<const fx8010_gpu*> hs;
+    for (const fx8010_gpu& h : tmp) hs.push_back(&h);
+    std::vector<std::vector<uint8_t>> folded;
+    return translate_source_out(tr_generate_chain(hs, folded), buf, cap, compile_check, cubin_bytes);
 }
 
 int fx8010_kernel_cache_set_dir(const char* dir) {

@@ -67,6 +67,24 @@ void FX8010::ensureUploaded() {
     }
 }
 
+FX8010Chain::FX8010Chain(const std::vector<FX8010*>& stages) : stages_(stages) {
+    std::vector<fx8010_gpu*> h;
+    for (FX8010* s : stages_) {
+        if (!s) throw std::runtime_error("FX8010Chain (B200): a stage is NULL");
+        h.push_back(s->gpuHandle());                           // (throws for an object spread over several devices)
+    }
+    if (fx8010_chain_create(h.data(), (int)h.size(), &chain_) != FX8010_OK)
+        throw std::runtime_error(std::string("FX8010Chain (B200): ") + fx8010_chain_last_error(nullptr));
+}
+
+FX8010Chain::~FX8010Chain() { fx8010_chain_destroy(chain_); }
+
+void FX8010Chain::processBlockDevice(const float* d_in, float* d_out, int n_samples, void* stream) {
+    for (FX8010* s : stages_) s->gpuHandle();                  // uploads a program loaded since the last block
+    if (fx8010_chain_process_batch(chain_, d_in, d_out, n_samples, stream) != FX8010_OK)
+        throw std::runtime_error(std::string("FX8010Chain (B200): process_batch failed: ") + fx8010_chain_last_error(chain_));
+}
+
 fx8010_gpu* FX8010::gpuHandle() {
     ensureUploaded();
     if (multi_) throw std::runtime_error("FX8010 (B200): this object drives several GPUs; there is no single device handle");

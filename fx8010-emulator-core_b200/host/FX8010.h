@@ -110,6 +110,23 @@ private:
     std::vector<float> in_block_, out_block_;
 };
 
+// Several objects' programs one after another within every sample period (include/fx8010_gpu.h, fx8010_chain_*): output channel c of
+// one stage is input channel c of the next, and a block costs one launch when every stage is stateless.  The objects must drive one
+// device each, the same one, with equal channel and instance counts (the constructor throws otherwise), and outlive the chain.
+class FX8010_CLASS FX8010Chain {
+public:
+    explicit FX8010Chain(const std::vector<FX8010*>& stages);
+    ~FX8010Chain();
+    FX8010Chain(const FX8010Chain&) = delete;
+    FX8010Chain& operator=(const FX8010Chain&) = delete;
+    // n_samples sample periods of every instance through every stage; DEVICE buffers [channel][sample][instance], asynchronous on `stream`
+    void processBlockDevice(const float* d_in, float* d_out, int n_samples, void* stream);
+
+private:
+    std::vector<FX8010*> stages_;
+    fx8010_chain* chain_ = nullptr;
+};
+
 }  // namespace Klangraum
 
 #endif

@@ -14,7 +14,14 @@ struct fx8010_host {
     fx8010_host(int c, int n, const std::vector<int>& devs) : fx(c, n, devs) {}
 };
 
+struct fx8010_host_chain {
+    Klangraum::FX8010Chain chain;
+    std::string err;
+    explicit fx8010_host_chain(const std::vector<Klangraum::FX8010*>& stages) : chain(stages) {}
+};
+
 namespace {
+thread_local std::string g_chain_create_error;
 void copy_out(const std::string& s, char* buf, int cap) {
     if (!buf || cap <= 0) return;
     std::strncpy(buf, s.c_str(), (size_t)cap - 1);
@@ -151,5 +158,19 @@ fx8010_gpu* fx8010_host_gpu(fx8010_host* h) {
     guarded(h, [&] { g = h->fx.gpuHandle(); });
     return g;
 }
+
+fx8010_host_chain* fx8010_host_chain_create(fx8010_host* const* stages, int n_stages) {
+    if (!stages || n_stages <= 0) { g_chain_create_error = "no stages"; return nullptr; }
+    std::vector<Klangraum::FX8010*> v;
+    for (int j = 0; j < n_stages; ++j) v.push_back(stages[j] ? &stages[j]->fx : nullptr);
+    try { return new fx8010_host_chain(v); }
+    catch (const std::exception& e) { g_chain_create_error = e.what(); return nullptr; }
+}
+void fx8010_host_chain_destroy(fx8010_host_chain* c) { delete c; }
+int fx8010_host_chain_process_block_device(fx8010_host_chain* c, const float* d_in, float* d_out, int n_samples, void* stream) {
+    try { c->chain.processBlockDevice(d_in, d_out, n_samples, stream); return 0; }
+    catch (const std::exception& e) { c->err = e.what(); return 1; }
+}
+const char* fx8010_host_chain_last_error(fx8010_host_chain* c) { return c ? c->err.c_str() : g_chain_create_error.c_str(); }
 
 }  // extern "C"

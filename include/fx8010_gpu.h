@@ -337,6 +337,37 @@ FX8010_API long long fx8010_translate_source(const fx8010_program_image* image, 
 FX8010_API long long fx8010_translate_source_curves(const fx8010_program_image* image, int n_instances, int n_channels, const int32_t* regs,
                                                     const int32_t* broadcast, int n_curves, char* buf, size_t cap, int compile_check, int* cubin_bytes);
 
+/* ---- program chains ----------------------------------------------------------------------------------------------------
+ * A chain runs the programs of several handles one after another within every sample period: output channel c of stage j is input
+ * channel c of stage j + 1.  fx8010_chain_process_batch(c, d_in, d_out, n, stream) is, bit for bit in d_out and in every stage's whole
+ * final state, process_batch(stage 0, d_in, t0); process_batch(stage 1, t0, t1); ...; process_batch(stage k-1, t(k-2), d_out).
+ * When every stage is stateless, the instance count is a multiple of 4, both buffers are 16-byte aligned and stage 0's
+ * FX8010_OPT_TRANSLATE is not 0, the chain runs as ONE translated kernel that keeps the intermediate samples in registers (mode 1
+ * compiles it in the background — the calls until then run stage by stage —, mode 2 before the call).  Otherwise it runs stage by stage
+ * through intermediate blocks the chain owns.  The fused launch is booked in fx8010_chain_status, not in the stages' launch info; it
+ * follows every stage's earlier work on any stream, and later work of any stage follows it.  Host-buffer, control-curve and multi-GPU
+ * calls have no chain form. */
+#define FX8010_MAX_CHAIN_STAGES 8
+typedef struct fx8010_chain fx8010_chain;
+/* stages[n_stages] (1..FX8010_MAX_CHAIN_STAGES distinct handles of one device, instance count and channel count; FX8010_ERR_ARG
+ * otherwise).  Programs may be loaded or reloaded after creation: the chain looks at its stages at every call.  Destroy the chain
+ * before any of its handles. */
+FX8010_API int fx8010_chain_create(fx8010_gpu* const* stages, int n_stages, fx8010_chain** out);
+FX8010_API void fx8010_chain_destroy(fx8010_chain* c);
+/* d_in / d_out as in fx8010_gpu_process_batch.  Checks everything before it queues anything: FX8010_ERR_NO_PROGRAM when a stage has no
+ * program, FX8010_ERR_ARG for a NULL d_out, a negative count, or a NULL d_in while stage 0 reads an input. */
+FX8010_API int fx8010_chain_process_batch(fx8010_chain* c, const float* d_in, float* d_out, int n_samples, void* stream);
+/* state: the fused kernel's translation state (values of fx8010_gpu_translate_status); fused_last: the last call ran it; launches: its
+ * launches so far; regs_per_thread / local_bytes: the loaded kernel's; message: why the last call did not run fused ("" when it did).
+ * Any pointer may be NULL. */
+FX8010_API int fx8010_chain_status(fx8010_chain* c, int* state, int* fused_last, unsigned long long* launches, int* regs_per_thread,
+                                   int* local_bytes, char* message, size_t message_cap);
+/* NULL: the last error of fx8010_chain_create on this thread. */
+FX8010_API const char* fx8010_chain_last_error(fx8010_chain* c);
+/* The source of the fused kernel for images[n_stages] (as fx8010_translate_source; -2 when some stage is not stateless). */
+FX8010_API long long fx8010_translate_source_chain(const fx8010_program_image* const* images, int n_stages, int n_instances, int n_channels,
+                                                   char* buf, size_t cap, int compile_check, int* cubin_bytes);
+
 /* ---- kernel cache of the program translator ----------------------------------------------------------------------------
  * A translated kernel is named by SHA-256 over these bytes, concatenated: "fx8010-kernel-v1\n", "sm_100a\n", each NVRTC option
  * followed by "\n" ("--gpu-architecture=sm_100a", "--std=c++17", "--fmad=false", "--ftz=false", "--prec-div=true", "--prec-sqrt=true",

@@ -72,7 +72,17 @@ FX8010_API int fx8010_host_process_block_curves(fx8010_host* h, const float* in,
                                                 const float* const* values, const int* broadcast, int n_curves);
 FX8010_API int fx8010_host_instruction_counter(fx8010_host* h);                 /* getInstructionCounter */
 FX8010_API unsigned long long fx8010_host_instruction_counter_total(fx8010_host* h);
-FX8010_API fx8010_gpu* fx8010_host_gpu(fx8010_host* h);                          /* NULL on failure */
+FX8010_API fx8010_gpu* fx8010_host_gpu(fx8010_host* h);
+
+/* Klangraum::FX8010Chain: the programs of stages[n_stages] one after another within every sample period (fx8010_chain_* of fx8010_gpu.h).
+ * create returns NULL when the objects do not share one device, channel and instance count (fx8010_host_chain_last_error(NULL) says why);
+ * destroy the chain before its objects. */
+typedef struct fx8010_host_chain fx8010_host_chain;
+FX8010_API fx8010_host_chain* fx8010_host_chain_create(fx8010_host* const* stages, int n_stages);
+FX8010_API void fx8010_host_chain_destroy(fx8010_host_chain* c);
+/* processBlockDevice(): DEVICE buffers [channel][sample][instance], asynchronous on `stream` */
+FX8010_API int fx8010_host_chain_process_block_device(fx8010_host_chain* c, const float* d_in, float* d_out, int n_samples, void* stream);
+FX8010_API const char* fx8010_host_chain_last_error(fx8010_host_chain* c);                          /* NULL on failure */
 
 #ifdef __cplusplus
 }
