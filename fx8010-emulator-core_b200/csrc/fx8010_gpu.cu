@@ -1753,6 +1753,9 @@ int chain_sequential(fx8010_chain* c, const float* d_in, float* d_out, int n, cu
     for (size_t j = 0; j < ns; ++j) {
         const float* in = j ? c->d_mid[(j - 1) & 1] : d_in;
         float* out = j + 1 == ns ? d_out : c->d_mid[j & 1];
+        // A stage's launch may postpone its wait only when it follows that handle's own launches (launch_blocks); here it follows the
+        // previous stage, which writes its input, so every stage launch waits at its start (STREAM_EXCLUSIVE set on a stage included).
+        c->st[j]->chain.clear();
         const int rc = fx8010_gpu_process_batch(c->st[j], in, out, n, stream);
         if (rc) return chain_fail(c, rc, "stage " + std::to_string(j) + ": " + c->st[j]->err);
     }

@@ -131,7 +131,8 @@ FX8010_API int fx8010_gpu_load_program(fx8010_gpu* h, const fx8010_program_image
  * events (other handles of this library included).  Consecutive launches of a program without state across sample
  * periods may then overlap on the device (programmatic dependent launch with a postponed wait) whenever their buffers
  * are disjoint from those of every launch that can still be running.  Without the promise every launch waits for
- * its predecessor on the stream at its start.
+ * its predecessor on the stream at its start.  The stage launches a chain queues (fx8010_chain_process_batch) never
+ * postpone their wait, whatever the stages' options: each stage reads what the stage before it has just written.
  *
  * FX8010_OPT_TRANSLATE (default 1; env FX8010_TRANSLATE): programs that need the general interpreter (SKIP, noise, MACMV,
  * state carried between instructions) are translated into one straight-line sm_100a kernel with NVRTC — registers in
@@ -155,7 +156,12 @@ FX8010_API int fx8010_gpu_get_register(fx8010_gpu* h, int reg_index, float* out)
 
 /* d_in / d_out: DEVICE pointers, [n_channels][n_samples][n_instances] float32.  Asynchronous
  * on `stream` (a cudaStream_t, NULL = default stream).  d_in may be NULL when the program has
- * no INPUT operand. */
+ * no INPUT operand.
+ * In place: d_out may equal d_in exactly (same pointer, same layout), and the call then gives the same outputs and the
+ * same final state as with separate buffers.  That holds for every call of this header and of fx8010_multi.h that takes
+ * an input and an output: process_batch, each block of process_blocks (d_out[b] == d_in[b]), process_batch_curves,
+ * process_batch_host with its _async, _slice and _host_curves forms, the fx8010_multi_process_batch_* calls and
+ * fx8010_chain_process_batch.  Any other overlap between an input and an output buffer is undefined. */
 FX8010_API int fx8010_gpu_process_batch(fx8010_gpu* h, const float* d_in, float* d_out,
                                         int n_samples, void* stream);
 /* n_blocks consecutive blocks of n_samples each in one call: block b reads d_in[b] and writes d_out[b] (arrays of
@@ -354,7 +360,7 @@ typedef struct fx8010_chain fx8010_chain;
  * before any of its handles. */
 FX8010_API int fx8010_chain_create(fx8010_gpu* const* stages, int n_stages, fx8010_chain** out);
 FX8010_API void fx8010_chain_destroy(fx8010_chain* c);
-/* d_in / d_out as in fx8010_gpu_process_batch.  Checks everything before it queues anything: FX8010_ERR_NO_PROGRAM when a stage has no
+/* d_in / d_out as in fx8010_gpu_process_batch (d_out may equal d_in).  Checks everything before it queues anything: FX8010_ERR_NO_PROGRAM when a stage has no
  * program, FX8010_ERR_ARG for a NULL d_out, a negative count, or a NULL d_in while stage 0 reads an input. */
 FX8010_API int fx8010_chain_process_batch(fx8010_chain* c, const float* d_in, float* d_out, int n_samples, void* stream);
 /* state: the fused kernel's translation state (values of fx8010_gpu_translate_status); fused_last: the last call ran it; launches: its

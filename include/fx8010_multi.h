@@ -43,7 +43,8 @@ FX8010_API int fx8010_multi_get_register(fx8010_multi* m, int reg_index, float* 
 
 /* FX8010::process x n_samples x N (source/FX8010.cpp:1023-1249): in / out are HOST buffers
  * [n_channels][n_samples][n_instances]; every device moves and computes its own columns concurrently; returns when
- * `out` is complete.  `in` may be NULL when the program has no INPUT operand. */
+ * `out` is complete.  `in` may be NULL when the program has no INPUT operand.  `out` may equal `in` (in place, as in
+ * fx8010_gpu_process_batch, for every call below); any other overlap is undefined. */
 FX8010_API int fx8010_multi_process_batch_host(fx8010_multi* m, const float* in, float* out, int n_samples);
 /* Same, but returns once every device has QUEUED its work (consecutive calls pipeline copies and kernels per
  * device); fx8010_multi_synchronize waits for everything. */

@@ -68,13 +68,17 @@ class HostChain:
         self.n, self.c = n, channels
         self.stages = [StageState(p, n, channels) for p in progs]
 
-    def process(self, x, s=None, seg_len=8, seed=0):
-        """x: [C][S][N] float32 (or None with s) -> out [C][S][N]."""
+    def process(self, x, s=None, seg_len=8, seed=0, inplace=False):
+        """x: [C][S][N] float32 (or None with s) -> out [C][S][N].  With `inplace` the kernel writes its outputs over its inputs (a copy
+        of x: d_out == d_in)."""
         assert self.n % 4 == 0
         if x is not None:
             x = np.ascontiguousarray(x, dtype=np.float32).reshape(self.c, -1, self.n)
             s = x.shape[1]
-        out = np.zeros((self.c, s, self.n), np.float32)
+        if inplace:
+            out = x = x.copy()
+        else:
+            out = np.zeros((self.c, s, self.n), np.float32)
         ch = FxtChain()
         for j, st in enumerate(self.stages):
             ch.s[j] = FxtStage(st.registers.ctypes.data, st.acc.ctypes.data, st.out_latch.ctypes.data, st.counts.ctypes.data,

@@ -16,7 +16,7 @@ from chain_host import HostChain
 fx = importlib.import_module("fx8010-emulator-core_b200")
 
 
-def run_chain(po, name, n, blocks, seg_len, rng, no_input=False):
+def run_chain(po, name, n, blocks, seg_len, rng, no_input=False, inplace=False):
     texts, ch = cc.chain_texts(name)
     prog_list = [fx.Program(t, channels=ch) for t in texts]
     for p in prog_list:
@@ -34,7 +34,7 @@ def run_chain(po, name, n, blocks, seg_len, rng, no_input=False):
     for b, s in enumerate(blocks):
         x = None if no_input else (1.8 * rng.random((ch, s, n)) - 0.9).astype(np.float32)
         want = cc.oracle_chain_stepped(orcs, x, s)
-        got = hc.process(x, s, seg_len=seg_len, seed=b)
+        got = hc.process(x, s, seg_len=seg_len, seed=b, inplace=inplace)
         assert_bits_equal(got, want, f"{name} outputs of block at {start}")
         start += s
     for j, (orc, st) in enumerate(zip(orcs, hc.stages)):
@@ -49,11 +49,13 @@ def run_chain(po, name, n, blocks, seg_len, rng, no_input=False):
     return hc
 
 
-@pytest.mark.parametrize("seg_len", [4, 8, 64])
-@pytest.mark.parametrize("name", cc.CHAINS)
-def test_chain_matches_stages_one_after_another(po, name, seg_len):
+@pytest.mark.parametrize("name,seg_len,inplace", [pytest.param(nm, sl, ip, id=f"{nm}-{sl}" + ("-inplace" if ip else ""))
+                                                  for ip in (False, True) for nm in cc.CHAINS for sl in (4, 8, 64)])
+def test_chain_matches_stages_one_after_another(po, name, seg_len, inplace):
+    """In place (d_out == d_in), the owner of the last period must re-run it through every stage from its input, not from the output it
+    has just stored there."""
     rng = np.random.default_rng(31 + seg_len)
-    hc = run_chain(po, name, 12, [37, 9, 1], seg_len, rng)
+    hc = run_chain(po, name, 12, [37, 9, 1], seg_len, rng, inplace=inplace)
     assert "fx_translated_chain" in hc.src and hc.src.count("FXT_DEV void fxt_period_s") == len(hc.stages)
 
 

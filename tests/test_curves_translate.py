@@ -73,11 +73,16 @@ class HostCurves:
             cb.bcast[j] = 1 if self.bcast[j] else 0
         return cb
 
-    def process(self, x, vals, span=None):
-        """x [C][S][N]; vals: per curve [S][N] (or [S] broadcast) float32 -> out [C][S][N]."""
+    def process(self, x, vals, span=None, inplace=False):
+        """x [C][S][N]; vals: per curve [S][N] (or [S] broadcast) float32 -> out [C][S][N].  With `inplace` the streaming kernel writes its
+        outputs over its inputs (a copy of x: d_out == d_in)."""
         x = np.ascontiguousarray(x, dtype=np.float32)
         s = x.shape[1]
-        out = np.zeros((self.c, s, self.n), np.float32)
+        if inplace:
+            assert not self.serial
+            out = x = x.copy()
+        else:
+            out = np.zeros((self.c, s, self.n), np.float32)
         cs = s * self.n
         if self.serial:
             lanes = int(re.search(r"#define FXT_K (\d+)", self.src).group(1))
@@ -108,7 +113,7 @@ class HostCurves:
         return out
 
 
-def run_case(po, name, n, blocks, want_kind=None, span=None, seed=0):
+def run_case(po, name, n, blocks, want_kind=None, span=None, seed=0, inplace=False):
     text, ch, cv = cc.programs()[name]
     prog = fx.Program(text, channels=ch)
     assert prog.loaded, prog.errors()
@@ -123,7 +128,7 @@ def run_case(po, name, n, blocks, want_kind=None, span=None, seed=0):
     for b, s in enumerate(blocks):
         x = (1.8 * rng.random((ch, s, n)) - 0.9).astype(np.float32)
         vals = [cc.make_curve(name, r, bc, s, n, rng) for r, bc in cv]
-        got = ht.process(x, vals, span=span)
+        got = ht.process(x, vals, span=span, inplace=inplace)
         want = cc.oracle_stepped(orc, x, list(zip(regs, vals, bcast)), s)
         assert_bits_equal(got, want, f"{name} outputs of block {b}")
     assert_bits_equal(ht.registers, orc.registers, name + " registers")
@@ -147,13 +152,18 @@ CASES = [
 ]
 
 
-@pytest.mark.parametrize("name,n,kind", CASES)
-def test_curves_match_the_oracle_stepped_per_period(po, name, n, kind):
+# ... and the cases on the streaming kernel once more with d_out == d_in
+RUNS = ([pytest.param(name, n, kind, False, id=f"{name}-{n}-{kind}") for name, n, kind in CASES] +
+        [pytest.param(name, n, kind, True, id=f"{name}-{n}-{kind}-inplace") for name, n, kind in CASES if kind != 0])
+
+
+@pytest.mark.parametrize("name,n,kind,inplace", RUNS)
+def test_curves_match_the_oracle_stepped_per_period(po, name, n, kind, inplace):
     span = 200 if name == "delay_fb" and kind == 2 else None
     blocks = [37, 9, 1] if name != "cfg5" else [9, 4]
     if name in ("delay_fb", "delay_mod"):
         blocks = [70, 333, 1, 250]
-    run_case(po, name, n, blocks, want_kind=kind, span=span, seed=sum(map(ord, name)) + n)
+    run_case(po, name, n, blocks, want_kind=kind, span=span, seed=sum(map(ord, name)) + n, inplace=inplace)
 
 
 def test_cfg4_four_instances_per_thread(po, monkeypatch):

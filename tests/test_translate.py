@@ -23,7 +23,7 @@ def po():
     return pyoracle
 
 
-def check(po, text, n, blocks, rng, channels=1, controls=None, amp=0.9, what="case", span=None):
+def check(po, text, n, blocks, rng, channels=1, controls=None, amp=0.9, what="case", span=None, inplace=False):
     prog = fx.Program(text, channels=channels)
     assert prog.loaded, prog.errors()
     img = po.Image(prog.instructions(), prog.registers(), prog.itram_size, prog.xtram_size, prog.controls(), prog.tables())
@@ -37,7 +37,7 @@ def check(po, text, n, blocks, rng, channels=1, controls=None, amp=0.9, what="ca
     start = 0
     for s in blocks:
         x = (2 * amp * rng.random((channels, s, n)) - amp).astype(np.float32)
-        assert_bits_equal(ht.process(x), orc.process(x), f"{what} outputs of block at {start}")
+        assert_bits_equal(ht.process(x, inplace=inplace), orc.process(x), f"{what} outputs of block at {start}")
         start += s
     assert_bits_equal(ht.registers, orc.registers, what + " registers")
     assert_bits_equal(ht.acc, orc.acc, what + " accumulator")
@@ -134,9 +134,15 @@ def test_noise_macmv_tram(po):
     check(po, text, 3, [90, 45], rng, what="noise/macmv/tram")
 
 
-@pytest.mark.parametrize("name", ["cfg1", "cfg2", "logtube", "random_stateless"])
-def test_stateless_programs_streaming_kernel(po, name):
-    """Stateless programs translate into the streaming kernel (fx_translated_sl): blocks x time segments x instance groups."""
+def with_inplace(names):
+    """Each case on separate buffers (the case's name) and with d_out == d_in (name-inplace)."""
+    return [pytest.param(nm, False, id=nm) for nm in names] + [pytest.param(nm, True, id=nm + "-inplace") for nm in names]
+
+
+@pytest.mark.parametrize("name,inplace", with_inplace(["cfg1", "cfg2", "logtube", "random_stateless"]))
+def test_stateless_programs_streaming_kernel(po, name, inplace):
+    """Stateless programs translate into the streaming kernel (fx_translated_sl): blocks x time segments x instance groups.  In place,
+    the owner of the last period must re-run it from its input, not from the output it has just stored there."""
     rng = np.random.default_rng(21)
     n = 12
     if name == "random_stateless":
@@ -147,7 +153,7 @@ def test_stateless_programs_streaming_kernel(po, name):
     prog = fx.Program(text)
     assert prog.loaded, prog.errors()
     ctl = {nm: rng.random(n).astype(np.float32) for nm in prog.controls()}
-    ht = check(po, text, n, [37, 8, 1], rng, controls=ctl, what=name)
+    ht = check(po, text, n, [37, 8, 1], rng, controls=ctl, what=name, inplace=inplace)
     assert "fx_translated_sl" in ht.src
     # several blocks in one launch
     img = po.Image(prog.instructions(), prog.registers(), prog.itram_size, prog.xtram_size, prog.controls(), prog.tables())
@@ -156,7 +162,7 @@ def test_stateless_programs_streaming_kernel(po, name):
     for nm, v in ctl.items():
         orc.set_register(prog.reg_index(nm), v); ht.registers[prog.reg_index(nm), :] = v
     xs = [(1.8 * rng.random((1, 21, n)) - 0.9).astype(np.float32) for _ in range(3)]
-    ys = ht.process_blocks(xs, 21, seg_len=4)
+    ys = ht.process_blocks(xs, 21, seg_len=4, inplace=inplace)
     for b in range(3):
         assert_bits_equal(ys[b], orc.process(xs[b]), f"{name} fused block {b}")
     assert_bits_equal(ht.registers, orc.registers, name + " registers after fused blocks")
@@ -175,8 +181,8 @@ def stateless_variant(text: str) -> str:
                       "limit a, b, a, 0.25", "exp b, a, 3, 0", "macsn out_l, b, a, g", "end"])
 
 
-@pytest.mark.parametrize("name", ["cfg3_200", "tap", "two_rings", "xdelay"])
-def test_delay_lines_streaming_kernel(po, name):
+@pytest.mark.parametrize("name,inplace", with_inplace(["cfg3_200", "tap", "two_rings", "xdelay"]))
+def test_delay_lines_streaming_kernel(po, name, inplace):
     """Delay lines whose periods are independent over a stretch (ring positions shared by all instances): the streaming kernel with TRAM
     READs loaded like inputs and WRITEs stored like outputs, one emulated launch per stretch, work items in random order."""
     rng = np.random.default_rng(23)
@@ -196,7 +202,7 @@ def test_delay_lines_streaming_kernel(po, name):
         text = "\n".join(["static a", "static rd", "input in_l 0", "output out_l 0", "xtramsize 2000 ", "xdelay read, rd, at, 0", "macs a, in_l, rd, 0.5",
                           "xdelay write, a, at, 0", "macs out_l, in_l, rd, 0.5", "end"])
         span = 2000
-    ht = check(po, text, n, [70, 400, 33, 1, 250], rng, what=name, span=span)
+    ht = check(po, text, n, [70, 400, 33, 1, 250], rng, what=name, span=span, inplace=inplace)
     assert "fx_translated_sl" in ht.src and "#define FXT_NTR 0" not in ht.src
 
 

@@ -81,8 +81,9 @@ class HostTranslated:
         self.flags = np.zeros(1, np.uint32)
         self.tabs = device_tables(prog.tables())
 
-    def process(self, x):
-        """x: [C][S][N] float32 or (None, S) -> out [C][S][N]."""
+    def process(self, x, inplace=False):
+        """x: [C][S][N] float32 or (None, S) -> out [C][S][N].  With `inplace` the streaming kernel writes its outputs over its inputs
+        (a copy of x: d_out == d_in)."""
         if isinstance(x, tuple):
             x, s = None, x[1]
         else:
@@ -92,13 +93,13 @@ class HostTranslated:
         cs = s * self.n
         if hasattr(self.lib, "fx_translated_sl_host"):
             if "#define FXT_NTR 0" in self.src:
-                return self.process_blocks([x], s)[0]
+                return self.process_blocks([x], s, inplace=inplace)[0]
             # a delay line: one emulated launch per stretch of at most `span` periods (what fx8010_gpu.cu::launch_blocks does)
             assert self.span and x is not None
             outs = []
             for a in range(0, s, self.span):
                 k = min(self.span, s - a)
-                outs.append(self.process_blocks([x[:, a:a + k]], k, seg_len=4)[0])
+                outs.append(self.process_blocks([x[:, a:a + k]], k, seg_len=4, inplace=inplace)[0])
             return np.concatenate(outs, axis=1)
         import re
         lanes = int(re.search(r"#define FXT_K (\d+)", self.src).group(1))
@@ -112,15 +113,21 @@ class HostTranslated:
     def tram(self, which: int, instance: int):
         return (self.itram if which == 0 else self.xtram)[: (self.isz if which == 0 else self.xsz), instance].copy()
 
-    def process_blocks(self, xs, s, seg_len=8):
-        """Stateless programs: consecutive blocks in ONE emulated launch (block x time segment x instance group work items)."""
+    def process_blocks(self, xs, s, seg_len=8, inplace=False):
+        """Stateless programs: consecutive blocks in ONE emulated launch (block x time segment x instance group work items).  With
+        `inplace` every block's output buffer is its input buffer (a copy of xs[b], which stays as it was)."""
         assert self.n % 4 == 0
         nb = len(xs)
         xs = [None if x is None else np.ascontiguousarray(x, dtype=np.float32).reshape(self.c, s, self.n) for x in xs]
-        outs = [np.zeros((self.c, s, self.n), np.float32) for _ in xs]
+        if inplace:
+            assert all(x is not None for x in xs)
+            outs = [x.copy() for x in xs]
+        else:
+            outs = [np.zeros((self.c, s, self.n), np.float32) for _ in xs]
+        ins = outs if inplace else xs
         io = FxtIo()
         for b in range(nb):
-            io.inp[b] = xs[b].ctypes.data if xs[b] is not None else None
+            io.inp[b] = ins[b].ctypes.data if ins[b] is not None else None
             io.out[b] = outs[b].ctypes.data
         cs = s * self.n
         n_seg = -(-s // seg_len)
