@@ -68,6 +68,10 @@ class CHostCurve(C.Structure):
     _fields_ = [("reg_index", C.c_int32), ("broadcast", C.c_int32), ("values", C.c_void_p)]
 
 
+class CChainCurve(C.Structure):
+    _fields_ = [("stage", C.c_int32), ("reg_index", C.c_int32), ("broadcast", C.c_int32), ("reserved", C.c_int32), ("d_values", C.c_void_p)]
+
+
 MAX_CONTROL_CURVES = 8
 VARIANT_CURVES = 16        # fx8010_launch_info.kernel_variant: the last launch read control curves inside the kernel
 
@@ -147,6 +151,10 @@ GPU_SYMBOLS = {
                                       C.POINTER(C.c_int), C.c_char_p, C.c_size_t]),
     "fx8010_chain_last_error": (C.c_char_p, [C.c_void_p]),
     "fx8010_translate_source_chain": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_char_p, C.c_size_t, C.c_int, C.POINTER(C.c_int)]),
+    "fx8010_chain_process_batch_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
+    "fx8010_chain_status_curves": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_char_p, C.c_size_t]),
+    "fx8010_translate_source_chain_curves": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                            C.c_char_p, C.c_size_t, C.c_int, C.POINTER(C.c_int)]),
 }
 
 MULTI_SYMBOLS = {
@@ -213,6 +221,8 @@ HOST_SYMBOLS = {
     "fx8010_host_chain_destroy": (None, [C.c_void_p]),
     "fx8010_host_chain_process_block_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "fx8010_host_chain_last_error": (C.c_char_p, [C.c_void_p]),
+    "fx8010_host_chain_process_block_device_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_char_p),
+                                                                C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
 }
 
 
@@ -471,6 +481,16 @@ class ProgramChain:
         if self.L.fx8010_host_chain_process_block_device(self.h, _ptr(d_in), _ptr(d_out), n_samples, stream):
             raise FxError(2, self.L.fx8010_host_chain_last_error(self.h).decode())
 
+    def process_curves(self, d_in, d_out, n_samples: int, curves, stream=None):
+        """FX8010Chain::processBlockDeviceWithCurves: curves = [(stage, register name, device tensor, broadcast)]."""
+        n = len(curves)
+        stages = (C.c_int * max(1, n))(*[int(c[0]) for c in curves])
+        names = (C.c_char_p * max(1, n))(*[c[1].encode() for c in curves])
+        ptrs = (C.c_void_p * max(1, n))(*[_ptr(c[2]) for c in curves])
+        bc = (C.c_int * max(1, n))(*[1 if c[3] else 0 for c in curves])
+        if self.L.fx8010_host_chain_process_block_device_curves(self.h, _ptr(d_in), _ptr(d_out), n_samples, stages, names, ptrs, bc, n, stream):
+            raise FxError(2, self.L.fx8010_host_chain_last_error(self.h).decode())
+
     def close(self):
         if getattr(self, "h", None):
             self.L.fx8010_host_chain_destroy(self.h)
@@ -521,6 +541,27 @@ def translate_source_chain(progs, channels: int = 1, compile_check: bool = False
     buf = C.create_string_buffer(int(n) + 1)
     cub = C.c_int(0)
     L.fx8010_translate_source_chain(imgs, len(progs), instances, channels, buf, int(n) + 1, 1 if compile_check else 0, C.byref(cub))
+    return buf.value.decode(), (cub.value if compile_check else None)
+
+
+def translate_source_chain_curves(progs, curves, channels: int = 1, compile_check: bool = False, instances: int = 1):
+    """translate_source_chain for the kernel fx8010_chain_process_batch_curves uses: curves = [(stage, register index, broadcast)].
+    Returns (None, None) when some stage is not stateless; raises ValueError for an image or curve list the call refuses."""
+    L = gpu_lib()
+    imgs = (C.c_void_p * max(1, len(progs)))(*[p.image_ptr() for p in progs])
+    k = len(curves)
+    stage = (C.c_int32 * max(1, k))(*[int(c[0]) for c in curves])
+    regs = (C.c_int32 * max(1, k))(*[int(c[1]) for c in curves])
+    bc = (C.c_int32 * max(1, k))(*[1 if c[2] else 0 for c in curves])
+    n = L.fx8010_translate_source_chain_curves(imgs, len(progs), instances, channels, stage, regs, bc, k, None, 0, 0, None)
+    if n == -1:
+        raise ValueError("bad image or curve list")
+    if n < 0:
+        return None, None
+    buf = C.create_string_buffer(int(n) + 1)
+    cub = C.c_int(0)
+    L.fx8010_translate_source_chain_curves(imgs, len(progs), instances, channels, stage, regs, bc, k, buf, int(n) + 1, 1 if compile_check else 0,
+                                           C.byref(cub))
     return buf.value.decode(), (cub.value if compile_check else None)
 
 
@@ -813,6 +854,24 @@ class Chain:
         self.L.fx8010_chain_status(self.h, C.byref(st), C.byref(fused), C.byref(launches), C.byref(regs), C.byref(loc), msg, 4096)
         return {"state": st.value, "fused_last": fused.value, "launches": int(launches.value), "regs_per_thread": regs.value,
                 "local_bytes": loc.value, "message": msg.value.decode(errors="replace")}
+
+    def process_batch_curves(self, d_in, d_out, n: int, curves, stream=None):
+        """fx8010_chain_process_batch_curves: curves = [(stage, register index, device buffer, broadcast)] — [n][N] float32 values, or [n]
+        with broadcast."""
+        curves = list(curves)
+        arr = (CChainCurve * max(1, len(curves)))()
+        for i, (stage, reg, vals, bc) in enumerate(curves):
+            arr[i].stage, arr[i].reg_index, arr[i].broadcast, arr[i].d_values = int(stage), int(reg), 1 if bc else 0, _ptr(vals)
+        rc = self.L.fx8010_chain_process_batch_curves(self.h, _ptr(d_in), _ptr(d_out), n, C.addressof(arr), len(curves), stream)
+        if rc != 0:
+            raise FxError(rc, self.L.fx8010_chain_last_error(self.h).decode())
+
+    def status_curves(self) -> dict:
+        """fx8010_chain_status_curves: the fused kernel of the most recent curve list."""
+        st, regs, loc = C.c_int(0), C.c_int(0), C.c_int(0)
+        msg = C.create_string_buffer(4096)
+        self.L.fx8010_chain_status_curves(self.h, C.byref(st), C.byref(regs), C.byref(loc), msg, 4096)
+        return {"state": st.value, "regs_per_thread": regs.value, "local_bytes": loc.value, "message": msg.value.decode(errors="replace")}
 
 
 class MultiGpu:

@@ -93,6 +93,12 @@ struct Translation {
 // The curves of one call as the kernels take them (a by-value parameter of the automated translated kernels: FxtCurves there).
 struct CurveBlock { const float* p[FX8010_MAX_CONTROL_CURVES]; int bcast[FX8010_MAX_CONTROL_CURVES]; };
 
+// Curve q of a chain call (fx8010_chain_process_batch_curves): register `reg` of stage `stage`; the list keys the chain's curve kernel.
+struct ChainCurve {
+    int stage, reg; uint8_t bcast;
+    bool operator==(const ChainCurve& o) const { return stage == o.stage && reg == o.reg && bcast == o.bcast; }
+};
+
 }  // namespace
 
 struct fx8010_gpu {
@@ -192,7 +198,7 @@ struct fx8010_gpu {
     int use_translate = 1;                       // FX8010_OPT_TRANSLATE: 0 never, 1 background compile + switch when ready, 2 compile before the first launch
     Translation tr;                              // the plain translation
     Translation tr_cv;                           // the translation for the most recent set of control curves (fx8010_gpu_process_batch_curves)
-    const Translation* tr_gen = nullptr;         // the translation being generated: its curve registers are never folded
+    mutable const Translation* tr_gen = nullptr; // the translation being generated: its curve registers are never folded (tr_generate_chain sets it per stage)
     std::vector<uint8_t> tr_volatile;            // per register: the host changed it after load — never folded again
     unsigned long long tr_epoch = 0;             // bumped whenever both translations are voided (load_program): chains over this handle regenerate
     std::string kc_env_dir;                      // FX8010_KERNEL_CACHE when the handle was created (the disk store; "" = none)
@@ -1541,10 +1547,18 @@ CurveBlock curves_from(const CurveBlock& cb, int n, size_t s0, size_t N) {
 }
 struct CurveRows { CurveBlock cv; int reg[FX8010_MAX_CONTROL_CURVES]; int n; };
 
+// While periods with curves on `regs` run, those registers hold no one value: nothing may fold them (interpreter encoding, plain
+// translation — a folded STATIC voids it, once).  Afterwards they hold the last period's values, which the host does not know: still not uniform.
+void curves_arm(fx8010_gpu* h, const std::vector<int>& regs) {
+    for (int r : regs) {
+        h->reg_uniform[r] = 0;
+        if (h->enc_sensitive[r]) h->encode_dirty = true;
+        tr_touch(h, r);
+    }
+}
+
 // The preamble of both curve calls (device and host values): checks the list and copies it into rows — FX8010_ERR_ARG changes and
-// queues nothing.  `arm`: the call will run periods.  While it runs the automated registers hold no one value: nothing may fold them
-// (interpreter encoding, plain translation — a folded STATIC voids it, once).  Afterwards they hold the last period's values, which
-// the host does not know: still not uniform.  h->tr_cv is keyed to this curve set.
+// queues nothing.  `arm`: the call will run periods (curves_arm).  h->tr_cv is keyed to this curve set.
 template <class Curve>
 int curves_begin(fx8010_gpu* h, const Curve* curves, int n_curves, const float* const Curve::*values, bool arm, CurveRows& rows) {
     if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && !curves))
@@ -1564,11 +1578,7 @@ int curves_begin(fx8010_gpu* h, const Curve* curves, int n_curves, const float* 
         if (!curves_valid(h->regs, regs, why)) return fail(h, FX8010_ERR_ARG, why);
     }
     if (!arm || n_curves == 0) return FX8010_OK;
-    for (int r : regs) {
-        h->reg_uniform[r] = 0;
-        if (h->enc_sensitive[r]) h->encode_dirty = true;
-        tr_touch(h, r);
-    }
+    curves_arm(h, regs);
     if (h->tr_cv.cv_reg != regs || h->tr_cv.cv_bcast != bc) {
         tr_reset(h, h->tr_cv);
         h->tr_cv.cv_reg = regs; h->tr_cv.cv_bcast = bc; h->tr_cv.serial = false;
@@ -1630,6 +1640,15 @@ int sync_all(fx8010_gpu* h) {
     return FX8010_OK;
 }
 
+// One fused kernel of a chain and what it was generated from.
+struct ChainKernel {
+    Translation tr;                                  // the fused kernel (kind 3) ...
+    std::vector<ChainCurve> cvs;                     // ... reading these control curves (none: the plain kernel) ...
+    std::vector<unsigned long long> epoch;           // ... generated while each stage had this tr_epoch ...
+    std::vector<std::vector<uint8_t>> folded;        // ... folding these registers of each stage ...
+    std::vector<std::vector<float>> fold_value;      // ... with these values
+};
+
 }  // namespace
 
 // A chain of stages (fx8010_chain_*): handles of one device, instance count and channel count whose programs run one after another within
@@ -1638,17 +1657,15 @@ int sync_all(fx8010_gpu* h) {
 struct fx8010_chain {
     std::vector<fx8010_gpu*> st;
     int device = 0;
-    Translation tr;                                  // the fused kernel (kind 3) ...
-    std::vector<unsigned long long> epoch;           // ... generated while each stage had this tr_epoch ...
-    std::vector<std::vector<uint8_t>> folded;        // ... folding these registers of each stage ...
-    std::vector<std::vector<float>> fold_value;      // ... with these values
+    ChainKernel plain;                               // the fused kernel of fx8010_chain_process_batch
+    ChainKernel cv;                                  // the one of fx8010_chain_process_batch_curves, for its most recent curve list
     float* d_mid[2] = {nullptr, nullptr};            // [C][S][N] intermediate blocks of the stage-by-stage path, used alternately
     size_t mid_floats = 0;
     cudaEvent_t ev = nullptr;                        // orders a stage-by-stage call after the previous one's use of d_mid on another stream
     cudaStream_t last_stream = nullptr; bool has_last = false;
-    unsigned long long launches = 0;                 // fused launches
+    unsigned long long launches = 0;                 // fused launches (plain and with curves)
     int fused_last = 0;
-    std::string why;                                 // why the last call did not run fused ("" when it did)
+    std::string why;                                 // why the last call (plain or with curves) did not run fused ("" when it did)
     std::string err;
 };
 
@@ -1659,17 +1676,17 @@ int chain_fail(fx8010_chain* c, int code, const std::string& msg) {
     return code;
 }
 
-// The fused kernel still computes what its stages would: no stage reloaded, every folded register still holds its folded value in every
+// Fused kernel K still computes what its stages would: no stage reloaded, every folded register still holds its folded value in every
 // instance.  A register that no longer does is never folded again (as tr_touch decides for a handle's own translation).
-bool chain_current(fx8010_chain* c) {
+bool chain_current(fx8010_chain* c, ChainKernel& K) {
     for (size_t j = 0; j < c->st.size(); ++j) {
         fx8010_gpu* h = c->st[j];
-        if (h->tr_epoch != c->epoch[j]) return false;
-        if (j >= c->folded.size()) continue;
-        for (size_t r = 0; r < c->folded[j].size(); ++r) {
-            if (!c->folded[j][r]) continue;
+        if (h->tr_epoch != K.epoch[j]) return false;
+        if (j >= K.folded.size()) continue;
+        for (size_t r = 0; r < K.folded[j].size(); ++r) {
+            if (!K.folded[j][r]) continue;
             uint32_t a, b;
-            memcpy(&a, &c->fold_value[j][r], 4); memcpy(&b, &h->reg_value[r], 4);
+            memcpy(&a, &K.fold_value[j][r], 4); memcpy(&b, &h->reg_value[r], 4);
             if (h->reg_uniform[r] && a == b) continue;
             h->tr_volatile[r] = 1;
             return false;
@@ -1678,31 +1695,32 @@ bool chain_current(fx8010_chain* c) {
     return true;
 }
 
-// Whether the fused kernel is loaded for the chain's current stages (tr_obtain in stage 0's translation mode); c->why says why not.
-bool chain_ready(fx8010_chain* c, bool may_wait) {
+// Whether fused kernel K is loaded for the chain's current stages (tr_obtain in stage 0's translation mode); `why` says why not.
+bool chain_ready(fx8010_chain* c, ChainKernel& K, bool may_wait, std::string& why) {
     fx8010_gpu* h0 = c->st[0];
-    if (!chain_current(c)) {
-        tr_reset(c->device, c->tr);
-        c->folded.clear(); c->fold_value.clear();
-        for (size_t j = 0; j < c->st.size(); ++j) c->epoch[j] = c->st[j]->tr_epoch;
+    if (!chain_current(c, K)) {
+        tr_reset(c->device, K.tr);
+        K.folded.clear(); K.fold_value.clear();
+        for (size_t j = 0; j < c->st.size(); ++j) K.epoch[j] = c->st[j]->tr_epoch;
     }
-    if (h0->use_translate == 0) { c->why = "translation is off on stage 0 (FX8010_OPT_TRANSLATE 0)"; return false; }
-    if (c->tr.state == 0)
+    if (h0->use_translate == 0) { why = "translation is off on stage 0 (FX8010_OPT_TRANSLATE 0)"; return false; }
+    if (K.tr.state == 0)
         for (size_t j = 0; j < c->st.size(); ++j)
-            if (!c->st[j]->stateless) { c->tr.state = -1; c->tr.error = "stage " + std::to_string(j) + " carries state across sample periods"; break; }
-    const bool ok = tr_obtain(c->device, h0->use_translate, h0->kc_env_dir, c->tr, [&](std::string& src, std::string&) {
-        src = tr_generate_chain(std::vector<const fx8010_gpu*>(c->st.begin(), c->st.end()), c->folded);
-        c->fold_value.clear();
-        for (fx8010_gpu* h : c->st) c->fold_value.push_back(h->reg_value);
+            if (!c->st[j]->stateless) { K.tr.state = -1; K.tr.error = "stage " + std::to_string(j) + " carries state across sample periods"; break; }
+    const bool ok = tr_obtain(c->device, h0->use_translate, h0->kc_env_dir, K.tr, [&](std::string& src, std::string&) {
+        src = tr_generate_chain(std::vector<const fx8010_gpu*>(c->st.begin(), c->st.end()), K.folded, K.cvs);
+        K.fold_value.clear();
+        for (fx8010_gpu* h : c->st) K.fold_value.push_back(h->reg_value);
         return true;
     }, may_wait);
-    c->why = ok ? "" : (c->tr.state == 1 ? "the chain kernel is compiling" : c->tr.error);
+    why = ok ? "" : (K.tr.state == 1 ? "the chain kernel is compiling" : K.tr.error);
     return ok;
 }
 
-// One launch of the fused kernel: every stage's earlier work comes first (order_on), and the kernel waits at its start and never lets a
-// later launch start early, so afterwards no stage has a late-waiting launch outstanding (each one's chain is empty).
-int chain_launch(fx8010_chain* c, const float* d_in, float* d_out, int n, cudaStream_t stream) {
+// One launch of fused kernel K (with the call's curves cv for the curve kernel): every stage's earlier work comes first (order_on), and the
+// kernel waits at its start and never lets a later launch start early, so afterwards no stage has a late-waiting launch outstanding (each
+// one's chain is empty).
+int chain_launch(fx8010_chain* c, const ChainKernel& K, const float* d_in, float* d_out, int n, cudaStream_t stream, const CurveBlock* cv = nullptr) {
     for (fx8010_gpu* h : c->st) {
         const int rc = order_on(h, stream);
         if (rc) return chain_fail(c, rc, h->err);
@@ -1721,16 +1739,19 @@ int chain_launch(fx8010_chain* c, const float* d_in, float* d_out, int n, cudaSt
     size_t cs = (size_t)n * h0->N;
     const void* inp = d_in; void* outp = d_out;
     int n_ = n, N_ = h0->N;
-    void* args[] = {&stages, &inp, &outp, &cs, &cs, &n_, &L.seg_len, &N_};
-    const int rc = tr_drive(h0, c->tr, L, 1, stream, args);
+    CurveBlock cvb = cv ? *cv : CurveBlock{};
+    void* args[] = {&stages, &inp, &outp, &cs, &cs, &n_, &L.seg_len, &N_, &cvb};
+    const int rc = tr_drive(h0, K.tr, L, 1, stream, args);
     if (rc) return chain_fail(c, rc, h0->err);
     for (fx8010_gpu* h : c->st) { h->chain.clear(); h->tram_periods += (unsigned long long)n; }
     c->launches++;
     return FX8010_OK;
 }
 
-// Stage by stage: fx8010_gpu_process_batch of every stage on `stream`, stage j writing the intermediate block stage j + 1 reads.
-int chain_sequential(fx8010_chain* c, const float* d_in, float* d_out, int n, cudaStream_t stream) {
+// Stage by stage: fx8010_gpu_process_batch of every stage on `stream`, stage j writing the intermediate block stage j + 1 reads; a stage
+// with curves in `cvs` (per stage, as the chain call lists them) takes fx8010_gpu_process_batch_curves and routes them itself.
+int chain_sequential(fx8010_chain* c, const float* d_in, float* d_out, int n, cudaStream_t stream,
+                     const std::vector<std::vector<fx8010_control_curve>>* cvs = nullptr) {
     const size_t ns = c->st.size(), need = (size_t)c->st[0]->C * n * c->st[0]->N;
     if (ns > 1 && need > c->mid_floats) {                 // (cudaFree waits for the device: no earlier call still uses the old blocks)
         cudaFree(c->d_mid[0]); cudaFree(c->d_mid[1]); c->d_mid[0] = c->d_mid[1] = nullptr; c->mid_floats = 0;
@@ -1756,7 +1777,9 @@ int chain_sequential(fx8010_chain* c, const float* d_in, float* d_out, int n, cu
         // A stage's launch may postpone its wait only when it follows that handle's own launches (launch_blocks); here it follows the
         // previous stage, which writes its input, so every stage launch waits at its start (STREAM_EXCLUSIVE set on a stage included).
         c->st[j]->chain.clear();
-        const int rc = fx8010_gpu_process_batch(c->st[j], in, out, n, stream);
+        const int rc = cvs && !(*cvs)[j].empty()
+                           ? fx8010_gpu_process_batch_curves(c->st[j], in, out, n, (*cvs)[j].data(), (int)(*cvs)[j].size(), stream)
+                           : fx8010_gpu_process_batch(c->st[j], in, out, n, stream);
         if (rc) return chain_fail(c, rc, "stage " + std::to_string(j) + ": " + c->st[j]->err);
     }
     c->last_stream = stream; c->has_last = true;
@@ -1793,8 +1816,10 @@ int fx8010_chain_create(fx8010_gpu* const* stages, int n_stages, fx8010_chain** 
     if (e != cudaSuccess) { delete c; return fail(nullptr, FX8010_ERR_CUDA, std::string("chain: ") + cudaGetErrorString(e)); }
     c->st.assign(stages, stages + n_stages);
     c->device = stages[0]->device;
-    c->tr.kind = 3;
-    for (fx8010_gpu* h : c->st) c->epoch.push_back(h->tr_epoch);
+    for (ChainKernel* K : {&c->plain, &c->cv}) {
+        K->tr.kind = 3;
+        for (fx8010_gpu* h : c->st) K->epoch.push_back(h->tr_epoch);
+    }
     *out = c;
     return FX8010_OK;
 }
@@ -1804,7 +1829,8 @@ void fx8010_chain_destroy(fx8010_chain* c) {
     cudaSetDevice(c->device);
     cudaFree(c->d_mid[0]); cudaFree(c->d_mid[1]);            // (waits for the device)
     if (c->ev) cudaEventDestroy(c->ev);
-    tr_detach(c->device, c->tr);
+    tr_detach(c->device, c->plain.tr);
+    tr_detach(c->device, c->cv.tr);
     delete c;
 }
 
@@ -1823,26 +1849,93 @@ int fx8010_chain_process_batch(fx8010_chain* c, const float* d_in, float* d_out,
     if (c->st.size() == 1) c->why = "a chain of one stage is that stage's process_batch";
     else if (h0->N % 4) c->why = "the instance count is not a multiple of 4";
     else if (!io_aligned(h0, 16, &d_in, &d_out, 1, cs, cs, n_samples)) c->why = "a buffer is not 16-byte aligned";
-    else fused = chain_ready(c, true);
+    else fused = chain_ready(c, c->plain, true, c->why);
     c->fused_last = fused ? 1 : 0;
-    return fused ? chain_launch(c, d_in, d_out, n_samples, st) : chain_sequential(c, d_in, d_out, n_samples, st);
+    return fused ? chain_launch(c, c->plain, d_in, d_out, n_samples, st) : chain_sequential(c, d_in, d_out, n_samples, st);
+}
+
+int fx8010_chain_process_batch_curves(fx8010_chain* c, const float* d_in, float* d_out, int n_samples, const fx8010_chain_curve* curves,
+                                      int n_curves, void* stream) {
+    if (!c) return FX8010_ERR_ARG;
+    if (n_curves == 0) return fx8010_chain_process_batch(c, d_in, d_out, n_samples, stream);
+    for (size_t j = 0; j < c->st.size(); ++j)
+        if (!c->st[j]->loaded) return chain_fail(c, FX8010_ERR_NO_PROGRAM, "stage " + std::to_string(j) + " has no program");
+    if (!d_out || n_samples < 0) return chain_fail(c, FX8010_ERR_ARG, "d_out is NULL or n_samples negative");
+    if (!d_in && reads_input(c->st[0])) return chain_fail(c, FX8010_ERR_ARG, "d_in is NULL but stage 0 reads an input");
+    // The whole list is checked, for every stage, before any stage runs (the stage-by-stage path must not run stage 0 and then refuse stage 2).
+    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || !curves)
+        return chain_fail(c, FX8010_ERR_ARG, "the curve list is NULL or the curve count outside 0..8");
+    const int NS = (int)c->st.size();
+    std::vector<std::vector<fx8010_control_curve>> per_stage((size_t)NS);
+    std::vector<ChainCurve> key;
+    CurveBlock cb = {};
+    for (int q = 0; q < n_curves; ++q) {
+        const fx8010_chain_curve& cv = curves[q];
+        if (cv.stage < 0 || cv.stage >= NS) return chain_fail(c, FX8010_ERR_ARG, "control curve " + std::to_string(q) + ": stage index out of range");
+        per_stage[cv.stage].push_back(fx8010_control_curve{cv.reg_index, cv.broadcast ? 1 : 0, cv.d_values});
+        key.push_back(ChainCurve{cv.stage, cv.reg_index, (uint8_t)(cv.broadcast ? 1 : 0)});
+        cb.p[q] = cv.d_values; cb.bcast[q] = cv.broadcast ? 1 : 0;
+    }
+    for (int j = 0; j < NS; ++j) {
+        CurveRows rows;
+        if (curves_begin(c->st[j], per_stage[j].data(), (int)per_stage[j].size(), &fx8010_control_curve::d_values, false, rows))
+            return chain_fail(c, FX8010_ERR_ARG, "stage " + std::to_string(j) + ": " + c->st[j]->err);
+    }
+    if (cudaSetDevice(c->device) != cudaSuccess) return chain_fail(c, FX8010_ERR_CUDA, "cudaSetDevice failed");
+    if (n_samples == 0) return FX8010_OK;
+    for (int j = 0; j < NS; ++j) {                          // (as fx8010_gpu_process_batch_curves leaves each stage)
+        std::vector<int> regs;
+        for (const fx8010_control_curve& cv : per_stage[j]) regs.push_back(cv.reg_index);
+        curves_arm(c->st[j], regs);
+    }
+    if (c->cv.cvs != key) {                                 // another curve list: another kernel
+        tr_reset(c->device, c->cv.tr);
+        c->cv.folded.clear(); c->cv.fold_value.clear();
+        c->cv.cvs = key;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    fx8010_gpu* h0 = c->st[0];
+    const size_t cs = (size_t)n_samples * h0->N;
+    bool fused = false;
+    if (NS == 1) c->why = "a chain of one stage is that stage's process_batch_curves";
+    else if (h0->N % 4) c->why = "the instance count is not a multiple of 4";
+    else if (!io_aligned(h0, 16, &d_in, &d_out, 1, cs, cs, n_samples)) c->why = "a buffer is not 16-byte aligned";
+    else if (!io_aligned(h0, 16, &d_in, &d_out, 1, cs, cs, n_samples, &cb, n_curves)) c->why = "a curve buffer is not 16-byte aligned";
+    else fused = chain_ready(c, c->cv, true, c->why);
+    c->fused_last = fused ? 1 : 0;
+    return fused ? chain_launch(c, c->cv, d_in, d_out, n_samples, st, &cb) : chain_sequential(c, d_in, d_out, n_samples, st, &per_stage);
 }
 
 int fx8010_chain_status(fx8010_chain* c, int* state, int* fused_last, unsigned long long* launches, int* regs_per_thread, int* local_bytes,
                         char* message, size_t message_cap) {
     if (!c) return FX8010_ERR_ARG;
-    if (c->tr.state == 1 && cudaSetDevice(c->device) == cudaSuccess) {     // pick up a finished background compilation
+    if (c->plain.tr.state == 1 && cudaSetDevice(c->device) == cudaSuccess) {     // pick up a finished background compilation
         bool loaded = true;
         for (fx8010_gpu* h : c->st) loaded = loaded && h->loaded;
-        if (loaded) chain_ready(c, false);
+        if (loaded) chain_ready(c, c->plain, false, c->why);
     }
-    if (state) *state = c->tr.state;
+    if (state) *state = c->plain.tr.state;
     if (fused_last) *fused_last = c->fused_last;
     if (launches) *launches = c->launches;
-    if (regs_per_thread) *regs_per_thread = c->tr.regs;
-    if (local_bytes) *local_bytes = c->tr.local;
+    if (regs_per_thread) *regs_per_thread = c->plain.tr.regs;
+    if (local_bytes) *local_bytes = c->plain.tr.local;
     const std::string& m = c->fused_last ? std::string() : c->why;
     if (message && message_cap) { strncpy(message, m.c_str(), message_cap - 1); message[message_cap - 1] = 0; }
+    return FX8010_OK;
+}
+
+int fx8010_chain_status_curves(fx8010_chain* c, int* state, int* regs_per_thread, int* local_bytes, char* message, size_t message_cap) {
+    if (!c) return FX8010_ERR_ARG;
+    std::string why = c->cv.tr.state == 1 ? "the chain kernel is compiling" : c->cv.tr.error;
+    if (c->cv.tr.state == 1 && cudaSetDevice(c->device) == cudaSuccess) {        // pick up a finished background compilation
+        bool loaded = true;
+        for (fx8010_gpu* h : c->st) loaded = loaded && h->loaded;
+        if (loaded) chain_ready(c, c->cv, false, why);
+    }
+    if (state) *state = c->cv.tr.state;
+    if (regs_per_thread) *regs_per_thread = c->cv.tr.regs;
+    if (local_bytes) *local_bytes = c->cv.tr.local;
+    if (message && message_cap) { strncpy(message, why.c_str(), message_cap - 1); message[message_cap - 1] = 0; }
     return FX8010_OK;
 }
 
@@ -2673,17 +2766,39 @@ long long fx8010_translate_source_curves(const fx8010_program_image* im, int n_i
     return translate_source_impl(im, n_instances, n_channels, regs, broadcast, n_curves, buf, cap, compile_check, cubin_bytes);
 }
 
-long long fx8010_translate_source_chain(const fx8010_program_image* const* images, int n_stages, int n_instances, int n_channels, char* buf,
-                                        size_t cap, int compile_check, int* cubin_bytes) {
+// The chain's fused kernel, with control curves q on register regs[q] of stage stage[q] when n_curves > 0: -1 for a bad image or a curve
+// list fx8010_chain_process_batch_curves refuses, -2 when some stage is not stateless (a program with SKIP never is, so no curve can make a
+// stateless stage ineligible).
+static long long translate_source_chain_impl(const fx8010_program_image* const* images, int n_stages, int n_instances, int n_channels,
+                                             const int32_t* stage, const int32_t* regs, const int32_t* broadcast, int n_curves, char* buf,
+                                             size_t cap, int compile_check, int* cubin_bytes) {
     if (!images || n_stages < 1 || n_stages > FX8010_MAX_CHAIN_STAGES) return -1;
+    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && (!stage || !regs || !broadcast))) return -1;
+    std::vector<ChainCurve> cvs;
+    std::vector<std::vector<int>> per_stage((size_t)n_stages);
+    for (int q = 0; q < n_curves; ++q) {
+        if (stage[q] < 0 || stage[q] >= n_stages) return -1;
+        per_stage[stage[q]].push_back(regs[q]);
+        cvs.push_back(ChainCurve{stage[q], regs[q], (uint8_t)(broadcast[q] ? 1 : 0)});
+    }
     std::vector<fx8010_gpu> tmp((size_t)n_stages);
     for (int j = 0; j < n_stages; ++j)
-        if (image_handle(images[j], n_instances, n_channels, {}, tmp[j])) return -1;
+        if (image_handle(images[j], n_instances, n_channels, per_stage[j], tmp[j])) return -1;
     for (const fx8010_gpu& h : tmp) if (!h.stateless) return -2;
     std::vector<const fx8010_gpu*> hs;
     for (const fx8010_gpu& h : tmp) hs.push_back(&h);
     std::vector<std::vector<uint8_t>> folded;
-    return translate_source_out(tr_generate_chain(hs, folded), buf, cap, compile_check, cubin_bytes);
+    return translate_source_out(tr_generate_chain(hs, folded, cvs), buf, cap, compile_check, cubin_bytes);
+}
+long long fx8010_translate_source_chain(const fx8010_program_image* const* images, int n_stages, int n_instances, int n_channels, char* buf,
+                                        size_t cap, int compile_check, int* cubin_bytes) {
+    return translate_source_chain_impl(images, n_stages, n_instances, n_channels, nullptr, nullptr, nullptr, 0, buf, cap, compile_check, cubin_bytes);
+}
+long long fx8010_translate_source_chain_curves(const fx8010_program_image* const* images, int n_stages, int n_instances, int n_channels,
+                                               const int32_t* stage, const int32_t* regs, const int32_t* broadcast, int n_curves, char* buf,
+                                               size_t cap, int compile_check, int* cubin_bytes) {
+    return translate_source_chain_impl(images, n_stages, n_instances, n_channels, stage, regs, broadcast, n_curves, buf, cap, compile_check,
+                                       cubin_bytes);
 }
 
 int fx8010_kernel_cache_set_dir(const char* dir) {

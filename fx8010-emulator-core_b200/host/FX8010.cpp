@@ -85,6 +85,20 @@ void FX8010Chain::processBlockDevice(const float* d_in, float* d_out, int n_samp
         throw std::runtime_error(std::string("FX8010Chain (B200): process_batch failed: ") + fx8010_chain_last_error(chain_));
 }
 
+void FX8010Chain::processBlockDeviceWithCurves(const float* d_in, float* d_out, int n_samples, const std::vector<Curve>& curves, void* stream) {
+    for (FX8010* s : stages_) s->gpuHandle();                  // uploads a program loaded since the last block
+    std::vector<fx8010_chain_curve> cv;
+    for (const Curve& c : curves) {
+        if (c.stage < 0 || c.stage >= (int)stages_.size())
+            throw std::runtime_error("FX8010Chain (B200): curve stage " + std::to_string(c.stage) + " out of range");
+        const int reg = stages_[c.stage]->frontend().findRegister(c.key);
+        if (reg < 0) throw std::runtime_error("FX8010Chain: unknown register '" + c.key + "' of stage " + std::to_string(c.stage));
+        cv.push_back(fx8010_chain_curve{c.stage, reg, c.broadcast ? 1 : 0, 0, c.d_values});
+    }
+    if (fx8010_chain_process_batch_curves(chain_, d_in, d_out, n_samples, cv.data(), (int)cv.size(), stream) != FX8010_OK)
+        throw std::runtime_error(std::string("FX8010Chain (B200): process_batch_curves failed: ") + fx8010_chain_last_error(chain_));
+}
+
 fx8010_gpu* FX8010::gpuHandle() {
     ensureUploaded();
     if (multi_) throw std::runtime_error("FX8010 (B200): this object drives several GPUs; there is no single device handle");

@@ -121,6 +121,11 @@ public:
     FX8010Chain& operator=(const FX8010Chain&) = delete;
     // n_samples sample periods of every instance through every stage; DEVICE buffers [channel][sample][instance], asynchronous on `stream`
     void processBlockDevice(const float* d_in, float* d_out, int n_samples, void* stream);
+    // the same with sample-accurate automation of any stage's registers (include/fx8010_gpu.h, fx8010_chain_process_batch_curves): register
+    // `key` of stage `stage` takes d_values[s] (broadcast) or d_values[s * numInstances + i] right before that stage's sample period s;
+    // DEVICE buffers, asynchronous on `stream`; throws on a stage out of range or an unknown name
+    struct Curve { int stage; std::string key; const float* d_values; bool broadcast; };
+    void processBlockDeviceWithCurves(const float* d_in, float* d_out, int n_samples, const std::vector<Curve>& curves, void* stream);
 
 private:
     std::vector<FX8010*> stages_;

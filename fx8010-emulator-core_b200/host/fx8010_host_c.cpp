@@ -171,6 +171,16 @@ int fx8010_host_chain_process_block_device(fx8010_host_chain* c, const float* d_
     try { c->chain.processBlockDevice(d_in, d_out, n_samples, stream); return 0; }
     catch (const std::exception& e) { c->err = e.what(); return 1; }
 }
+int fx8010_host_chain_process_block_device_curves(fx8010_host_chain* c, const float* d_in, float* d_out, int n_samples, const int* stages,
+                                                  const char* const* names, const float* const* d_values, const int* broadcast, int n_curves,
+                                                  void* stream) {
+    try {
+        std::vector<Klangraum::FX8010Chain::Curve> cv;
+        for (int j = 0; j < n_curves; ++j) cv.push_back(Klangraum::FX8010Chain::Curve{stages[j], names[j], d_values[j], broadcast[j] != 0});
+        c->chain.processBlockDeviceWithCurves(d_in, d_out, n_samples, cv, stream);
+        return 0;
+    } catch (const std::exception& e) { c->err = e.what(); return 1; }
+}
 const char* fx8010_host_chain_last_error(fx8010_host_chain* c) { return c ? c->err.c_str() : g_chain_create_error.c_str(); }
 
 }  // extern "C"

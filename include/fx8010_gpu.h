@@ -161,7 +161,7 @@ FX8010_API int fx8010_gpu_get_register(fx8010_gpu* h, int reg_index, float* out)
  * same final state as with separate buffers.  That holds for every call of this header and of fx8010_multi.h that takes
  * an input and an output: process_batch, each block of process_blocks (d_out[b] == d_in[b]), process_batch_curves,
  * process_batch_host with its _async, _slice and _host_curves forms, the fx8010_multi_process_batch_* calls and
- * fx8010_chain_process_batch.  Any other overlap between an input and an output buffer is undefined. */
+ * fx8010_chain_process_batch with its _curves form.  Any other overlap between an input and an output buffer is undefined. */
 FX8010_API int fx8010_gpu_process_batch(fx8010_gpu* h, const float* d_in, float* d_out,
                                         int n_samples, void* stream);
 /* n_blocks consecutive blocks of n_samples each in one call: block b reads d_in[b] and writes d_out[b] (arrays of
@@ -351,8 +351,8 @@ FX8010_API long long fx8010_translate_source_curves(const fx8010_program_image* 
  * FX8010_OPT_TRANSLATE is not 0, the chain runs as ONE translated kernel that keeps the intermediate samples in registers (mode 1
  * compiles it in the background — the calls until then run stage by stage —, mode 2 before the call).  Otherwise it runs stage by stage
  * through intermediate blocks the chain owns.  The fused launch is booked in fx8010_chain_status, not in the stages' launch info; it
- * follows every stage's earlier work on any stream, and later work of any stage follows it.  Host-buffer, control-curve and multi-GPU
- * calls have no chain form. */
+ * follows every stage's earlier work on any stream, and later work of any stage follows it.  Control curves on any stage's registers:
+ * fx8010_chain_process_batch_curves.  Host-buffer and multi-GPU calls have no chain form. */
 #define FX8010_MAX_CHAIN_STAGES 8
 typedef struct fx8010_chain fx8010_chain;
 /* stages[n_stages] (1..FX8010_MAX_CHAIN_STAGES distinct handles of one device, instance count and channel count; FX8010_ERR_ARG
@@ -365,14 +365,46 @@ FX8010_API void fx8010_chain_destroy(fx8010_chain* c);
 FX8010_API int fx8010_chain_process_batch(fx8010_chain* c, const float* d_in, float* d_out, int n_samples, void* stream);
 /* state: the fused kernel's translation state (values of fx8010_gpu_translate_status); fused_last: the last call ran it; launches: its
  * launches so far; regs_per_thread / local_bytes: the loaded kernel's; message: why the last call did not run fused ("" when it did).
- * Any pointer may be NULL. */
+ * state, regs_per_thread and local_bytes describe the kernel of fx8010_chain_process_batch; fused_last, launches and message the last chain
+ * call of either kind (with or without curves).  Any pointer may be NULL. */
 FX8010_API int fx8010_chain_status(fx8010_chain* c, int* state, int* fused_last, unsigned long long* launches, int* regs_per_thread,
                                    int* local_bytes, char* message, size_t message_cap);
+
+/* Sample-accurate automation of a chain: control curves on registers of any of its stages, read inside the fused kernel. */
+typedef struct fx8010_chain_curve {
+    int32_t stage;          /* 0 .. n_stages-1                                              */
+    int32_t reg_index;      /* a CONTROL or STATIC register of that stage's program         */
+    int32_t broadcast;      /* 0: d_values is [n_samples][n_instances]; != 0: [n_samples]   */
+    int32_t reserved;
+    const float* d_values;  /* DEVICE pointer, float32                                      */
+} fx8010_chain_curve;
+/* fx8010_chain_process_batch with up to FX8010_MAX_CONTROL_CURVES curves in total, spread over the stages in any way.  Bit for bit in d_out
+ * and in every stage's whole final state it is, stage after stage, fx8010_gpu_process_batch_curves(stage j, t(j-1), t(j), n_samples, the
+ * curves of stage j) — fx8010_gpu_process_batch for a stage without curves: before stage j's period s each automated register of stage j
+ * holds curve[s], and it ends holding its last curve value or what the stage's program wrote to it in the last period.  The chain runs fused
+ * under the conditions of fx8010_chain_process_batch when, in addition, every per-instance curve is 16-byte aligned; the fused kernel loads
+ * each period's curve values with the chain's inputs.  Otherwise it runs stage by stage, every stage with curves routing them as
+ * fx8010_gpu_process_batch_curves does (fx8010_chain_status says why).  Everything is checked, for every stage, before anything is queued:
+ * the rules of fx8010_chain_process_batch, and FX8010_ERR_ARG for a count outside 0..8, a NULL list with a count > 0, a NULL d_values, a
+ * stage out of range, a register out of range for its stage, one (stage, register) named twice, or a register neither CONTROL nor STATIC.
+ * d_out may equal d_in; a curve buffer that overlaps d_out is undefined.  A curve buffer may be the output of earlier work on `stream`.
+ * With n_curves == 0 it is fx8010_chain_process_batch. */
+FX8010_API int fx8010_chain_process_batch_curves(fx8010_chain* c, const float* d_in, float* d_out, int n_samples,
+                                                 const fx8010_chain_curve* curves, int n_curves, void* stream);
+/* The fused kernel of the most recent curve list (stage, register, broadcast) of fx8010_chain_process_batch_curves: its state (values of
+ * fx8010_gpu_translate_status; 0 also before any curve call), registers and local memory, and why it is not in use ("" when it is). */
+FX8010_API int fx8010_chain_status_curves(fx8010_chain* c, int* state, int* regs_per_thread, int* local_bytes, char* message,
+                                          size_t message_cap);
 /* NULL: the last error of fx8010_chain_create on this thread. */
 FX8010_API const char* fx8010_chain_last_error(fx8010_chain* c);
 /* The source of the fused kernel for images[n_stages] (as fx8010_translate_source; -2 when some stage is not stateless). */
 FX8010_API long long fx8010_translate_source_chain(const fx8010_program_image* const* images, int n_stages, int n_instances, int n_channels,
                                                    char* buf, size_t cap, int compile_check, int* cubin_bytes);
+/* The same with control curves q on register regs[q] of stage stage[q] (broadcast[q] as in fx8010_chain_curve).  With n_curves == 0 it is
+ * fx8010_translate_source_chain.  -1 also for a curve list fx8010_chain_process_batch_curves refuses. */
+FX8010_API long long fx8010_translate_source_chain_curves(const fx8010_program_image* const* images, int n_stages, int n_instances,
+                                                          int n_channels, const int32_t* stage, const int32_t* regs, const int32_t* broadcast,
+                                                          int n_curves, char* buf, size_t cap, int compile_check, int* cubin_bytes);
 
 /* ---- kernel cache of the program translator ----------------------------------------------------------------------------
  * A translated kernel is named by SHA-256 over these bytes, concatenated: "fx8010-kernel-v1\n", "sm_100a\n", each NVRTC option

@@ -82,6 +82,11 @@ FX8010_API fx8010_host_chain* fx8010_host_chain_create(fx8010_host* const* stage
 FX8010_API void fx8010_host_chain_destroy(fx8010_host_chain* c);
 /* processBlockDevice(): DEVICE buffers [channel][sample][instance], asynchronous on `stream` */
 FX8010_API int fx8010_host_chain_process_block_device(fx8010_host_chain* c, const float* d_in, float* d_out, int n_samples, void* stream);
+/* processBlockDeviceWithCurves(): curve j drives register names[j] of stage stages[j] (d_values[j], broadcast[j]: see
+ * fx8010_chain_process_batch_curves) */
+FX8010_API int fx8010_host_chain_process_block_device_curves(fx8010_host_chain* c, const float* d_in, float* d_out, int n_samples,
+                                                             const int* stages, const char* const* names, const float* const* d_values,
+                                                             const int* broadcast, int n_curves, void* stream);
 FX8010_API const char* fx8010_host_chain_last_error(fx8010_host_chain* c);                          /* NULL on failure */
 
 #ifdef __cplusplus
