@@ -999,6 +999,8 @@ int plan_stateless(fx8010_gpu* h, const float*, const float*, unsigned align, in
     if (tsplit) while (M > 1 && 2 * M >= known_tram_span(h)) M >>= 1;    // the READs of batch b + 1 are prefetched while batch b runs
     if (serial && M < 2) M = 2;        // a carried operand reads row (m - 1) mod M while row m is written
     while (sl_smem_bytes(h, B, K, M) > h->smem_optin && B > 32) B >>= 1;
+    // (a long program with many registers and shared-memory tables can need fewer instances per thread, like the general interpreter's plan)
+    while (sl_smem_bytes(h, B, K, M) > h->smem_optin && K > 1 && !h->tune_K) K >>= 1;
     if (sl_smem_bytes(h, B, K, M) > h->smem_optin) return fail(h, FX8010_ERR_CAPACITY, "register file does not fit in shared memory");
     // Sample split: a serial program whose only state across sample periods is TRAM (nothing carried in registers) has
     // independent samples inside a batch, so P threads can share one instance column and take M / P samples each — P
