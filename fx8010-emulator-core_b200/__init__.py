@@ -14,6 +14,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import weakref
 
 import numpy as np
 
@@ -70,6 +71,10 @@ class CHostCurve(C.Structure):
 
 class CChainCurve(C.Structure):
     _fields_ = [("stage", C.c_int32), ("reg_index", C.c_int32), ("broadcast", C.c_int32), ("reserved", C.c_int32), ("d_values", C.c_void_p)]
+
+
+class CChainHostCurve(C.Structure):
+    _fields_ = [("stage", C.c_int32), ("reg_index", C.c_int32), ("broadcast", C.c_int32), ("reserved", C.c_int32), ("values", C.c_void_p)]
 
 
 MAX_CONTROL_CURVES = 8
@@ -155,6 +160,9 @@ GPU_SYMBOLS = {
     "fx8010_chain_status_curves": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_char_p, C.c_size_t]),
     "fx8010_translate_source_chain_curves": (C.c_longlong, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                                             C.c_char_p, C.c_size_t, C.c_int, C.POINTER(C.c_int)]),
+    "fx8010_chain_process_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_int]),
+    "fx8010_chain_process_batch_host_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_size_t, C.c_int]),
+    "fx8010_chain_synchronize": (C.c_int, [C.c_void_p]),
 }
 
 MULTI_SYMBOLS = {
@@ -177,6 +185,14 @@ MULTI_SYMBOLS = {
     "fx8010_multi_get_registers": (C.c_int, [C.c_void_p, C.c_void_p]),
     "fx8010_multi_get_runtime_flags": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint), C.c_int]),
     "fx8010_multi_last_error": (C.c_char_p, [C.c_void_p]),
+    "fx8010_multi_chain_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
+    "fx8010_multi_chain_destroy": (None, [C.c_void_p]),
+    "fx8010_multi_chain_process_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int]),
+    "fx8010_multi_chain_process_batch_host_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int]),
+    "fx8010_multi_chain_synchronize": (C.c_int, [C.c_void_p]),
+    "fx8010_multi_chain_shard": (C.c_void_p, [C.c_void_p, C.c_int]),
+    "fx8010_multi_chain_last_error": (C.c_char_p, [C.c_void_p]),
+    "fx8010_multi_shard_chain_curves": (None, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
 }
 
 HOST_SYMBOLS = {
@@ -223,6 +239,9 @@ HOST_SYMBOLS = {
     "fx8010_host_chain_last_error": (C.c_char_p, [C.c_void_p]),
     "fx8010_host_chain_process_block_device_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_char_p),
                                                                 C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "fx8010_host_chain_process_block": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
+    "fx8010_host_chain_process_block_curves": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_char_p),
+                                                         C.c_void_p, C.c_void_p, C.c_int]),
 }
 
 
@@ -275,6 +294,42 @@ def _host_block(a, rows: int, cols: int, host_instances: int):
     return a
 
 
+def _chain_host_curves(curves, s: int, n: int, host_instances: int):
+    """[(stage, register index, ndarray, broadcast)] -> (fx8010_chain_host_curve array, the float32 arrays it points into)."""
+    arr = (CChainHostCurve * max(1, len(curves)))()
+    keep = []
+    for i, (stage, reg, vals, bc) in enumerate(curves):
+        v = np.ascontiguousarray(vals, dtype=np.float32).reshape(s) if bc else _host_block(vals, s, n, host_instances)
+        keep.append(v)
+        arr[i].stage, arr[i].reg_index, arr[i].broadcast, arr[i].values = int(stage), int(reg), 1 if bc else 0, v.ctypes.data
+    return arr, keep
+
+
+def _host_out(out, c: int, s: int, n: int, host_instances: int):
+    """The output block of a host-buffer call: the caller's (checked like its input), or a new one — with host_instances, the first n
+    columns of a new [C][S][host_instances] block, so that every row the call writes lies inside it."""
+    if out is None:
+        return np.zeros((c, s, host_instances or n), dtype=np.float32)[:, :, :n]
+    if host_instances:
+        _host_block(out, c * s, n, host_instances)
+    else:
+        assert out.dtype == np.float32 and out.flags.c_contiguous and out.size == c * s * n
+    return out
+
+
+def _register_chain(chain, stages):
+    """A chain reads its stages when it is destroyed: closing a stage closes the chains over it first."""
+    for st in stages:
+        st.__dict__.setdefault("_chains", []).append(weakref.ref(chain))
+
+
+def _close_chains(obj):
+    for ref in obj.__dict__.pop("_chains", []):
+        c = ref()
+        if c is not None:
+            c.close()
+
+
 def _host_curves(curves, s: int, n: int, host_instances: int):
     """[(register index, ndarray, broadcast)] -> (fx8010_host_curve array, the float32 arrays it points into)."""
     arr = (CHostCurve * max(1, len(curves)))()
@@ -307,6 +362,7 @@ class Program:
             self.loaded = self.load(text=text, path=path)
 
     def close(self):
+        _close_chains(self)
         if getattr(self, "h", None):
             self.L.fx8010_host_destroy(self.h)
             self.h = None
@@ -476,10 +532,40 @@ class ProgramChain:
         self.h = self.L.fx8010_host_chain_create(arr, len(self.programs))
         if not self.h:
             raise FxError(1, self.L.fx8010_host_chain_last_error(None).decode())
+        _register_chain(self, self.programs)
 
     def __call__(self, d_in, d_out, n_samples: int, stream=None):
         if self.L.fx8010_host_chain_process_block_device(self.h, _ptr(d_in), _ptr(d_out), n_samples, stream):
             raise FxError(2, self.L.fx8010_host_chain_last_error(self.h).decode())
+
+    def process_block(self, x, n_samples=None) -> np.ndarray:
+        """FX8010Chain::processBlock: host buffers, x [C][S][N] (None: no input) -> [C][S][N]."""
+        p0 = self.programs[0]
+        if x is not None:
+            x = np.ascontiguousarray(x, dtype=np.float32).reshape(p0.channels, -1, p0.instances)
+            n_samples = x.shape[1]
+        out = np.zeros((p0.channels, n_samples, p0.instances), dtype=np.float32)
+        if self.L.fx8010_host_chain_process_block(self.h, _ptr(x), out.ctypes.data, n_samples):
+            raise FxError(2, self.L.fx8010_host_chain_last_error(self.h).decode())
+        return out
+
+    def process_block_curves(self, x, curves, n_samples=None) -> np.ndarray:
+        """FX8010Chain::processBlockWithCurves: curves = [(stage, register name, ndarray, broadcast)], each [S][N] float32, or [S] with
+        broadcast."""
+        p0 = self.programs[0]
+        if x is not None:
+            x = np.ascontiguousarray(x, dtype=np.float32).reshape(p0.channels, -1, p0.instances)
+            n_samples = x.shape[1]
+        out = np.zeros((p0.channels, n_samples, p0.instances), dtype=np.float32)
+        n = len(curves)
+        vals = [np.ascontiguousarray(c[2], dtype=np.float32) for c in curves]
+        stages = (C.c_int * max(1, n))(*[int(c[0]) for c in curves])
+        names = (C.c_char_p * max(1, n))(*[c[1].encode() for c in curves])
+        ptrs = (C.c_void_p * max(1, n))(*[v.ctypes.data for v in vals])
+        bc = (C.c_int * max(1, n))(*[1 if c[3] else 0 for c in curves])
+        if self.L.fx8010_host_chain_process_block_curves(self.h, _ptr(x), out.ctypes.data, n_samples, stages, names, ptrs, bc, n):
+            raise FxError(2, self.L.fx8010_host_chain_last_error(self.h).decode())
+        return out
 
     def process_curves(self, d_in, d_out, n_samples: int, curves, stream=None):
         """FX8010Chain::processBlockDeviceWithCurves: curves = [(stage, register name, device tensor, broadcast)]."""
@@ -602,6 +688,7 @@ class Gpu:
         self._keep = None
 
     def close(self):
+        _close_chains(self)
         if getattr(self, "h", None):
             self.L.fx8010_gpu_destroy(self.h)
             self.h = None
@@ -823,8 +910,8 @@ MAX_CHAIN_STAGES = 8
 
 
 class Chain:
-    """Several Gpu handles run one after another within every sample period (include/fx8010_gpu.h, fx8010_chain_*).  Close it before
-    the handles."""
+    """Several Gpu handles run one after another within every sample period (include/fx8010_gpu.h, fx8010_chain_*).  It is closed
+    before the handles: closing a handle closes the chains over it first."""
 
     def __init__(self, stages):
         self.L = gpu_lib()
@@ -835,6 +922,7 @@ class Chain:
         if rc != 0:
             raise FxError(rc, self.L.fx8010_chain_last_error(None).decode())
         self.h = h
+        _register_chain(self, self.stages)
 
     def close(self):
         if getattr(self, "h", None):
@@ -849,11 +937,7 @@ class Chain:
             raise FxError(rc, self.L.fx8010_chain_last_error(self.h).decode())
 
     def status(self) -> dict:
-        st, fused, regs, loc, launches = C.c_int(0), C.c_int(0), C.c_int(0), C.c_int(0), C.c_ulonglong(0)
-        msg = C.create_string_buffer(4096)
-        self.L.fx8010_chain_status(self.h, C.byref(st), C.byref(fused), C.byref(launches), C.byref(regs), C.byref(loc), msg, 4096)
-        return {"state": st.value, "fused_last": fused.value, "launches": int(launches.value), "regs_per_thread": regs.value,
-                "local_bytes": loc.value, "message": msg.value.decode(errors="replace")}
+        return _chain_status(self.L, self.h)
 
     def process_batch_curves(self, d_in, d_out, n: int, curves, stream=None):
         """fx8010_chain_process_batch_curves: curves = [(stage, register index, device buffer, broadcast)] — [n][N] float32 values, or [n]
@@ -873,6 +957,42 @@ class Chain:
         self.L.fx8010_chain_status_curves(self.h, C.byref(st), C.byref(regs), C.byref(loc), msg, 4096)
         return {"state": st.value, "regs_per_thread": regs.value, "local_bytes": loc.value, "message": msg.value.decode(errors="replace")}
 
+    def process_host(self, x, n_samples=None, out=None, wait: bool = True, host_instances: int = 0) -> np.ndarray:
+        """fx8010_chain_process_batch_host: x [C][S][N] (None: no input) -> out [C][S][N].  With host_instances, x and out are views of N
+        columns of C-contiguous arrays host_instances wide (as in Gpu.process_host_curves).  wait=False queues the work; the arrays are
+        kept until synchronize()."""
+        return self.process_host_curves(x, [], n_samples=n_samples, out=out, wait=wait, host_instances=host_instances)
+
+    def process_host_curves(self, x, curves, n_samples=None, out=None, wait: bool = True, host_instances: int = 0) -> np.ndarray:
+        """fx8010_chain_process_batch_host_curves: curves = [(stage, register index, ndarray, broadcast)], each [S][N] float32 (N columns of
+        a host_instances-wide array with host_instances), or [S] with broadcast; the rest as in process_host."""
+        g0 = self.stages[0]
+        if x is not None:
+            n_samples = x.shape[1]
+        x = _host_block(x, g0.c * n_samples, g0.n, host_instances)
+        out = _host_out(out, g0.c, n_samples, g0.n, host_instances)
+        arr, keep = _chain_host_curves(curves, n_samples, g0.n, host_instances)
+        rc = self.L.fx8010_chain_process_batch_host_curves(self.h, _ptr(x), _ptr(out), n_samples, C.addressof(arr), len(curves), host_instances,
+                                                           1 if wait else 0)
+        if rc != 0:
+            raise FxError(rc, self.L.fx8010_chain_last_error(self.h).decode())
+        self._pending = [] if wait else getattr(self, "_pending", []) + [(x, out, arr, keep)]
+        return out
+
+    def synchronize(self):
+        rc = self.L.fx8010_chain_synchronize(self.h)
+        if rc != 0:
+            raise FxError(rc, self.L.fx8010_chain_last_error(self.h).decode())
+        self._pending = []
+
+
+def _chain_status(L, h) -> dict:
+    st, fused, regs, loc, launches = C.c_int(0), C.c_int(0), C.c_int(0), C.c_int(0), C.c_ulonglong(0)
+    msg = C.create_string_buffer(4096)
+    L.fx8010_chain_status(h, C.byref(st), C.byref(fused), C.byref(launches), C.byref(regs), C.byref(loc), msg, 4096)
+    return {"state": st.value, "fused_last": fused.value, "launches": int(launches.value), "regs_per_thread": regs.value,
+            "local_bytes": loc.value, "message": msg.value.decode(errors="replace")}
+
 
 class MultiGpu:
     """One program over N instances spread across several GPUs (include/fx8010_multi.h): contiguous instance ranges,
@@ -889,6 +1009,7 @@ class MultiGpu:
         self.h = h
 
     def close(self):
+        _close_chains(self)
         if getattr(self, "h", None):
             self.L.fx8010_multi_destroy(self.h)
             self.h = None
@@ -977,6 +1098,64 @@ class MultiGpu:
         f = C.c_uint(0)
         self._check(self.L.fx8010_multi_get_runtime_flags(self.h, C.byref(f), 1 if clear else 0))
         return int(f.value)
+
+
+class MultiChain:
+    """Several MultiGpu executors run one after another within every sample period (include/fx8010_multi.h, fx8010_multi_chain_*): one
+    chain per shard, driven by the shard threads of the first executor.  It is closed before the executors: closing an executor closes the
+    chains over it first."""
+
+    def __init__(self, stages):
+        self.L = gpu_lib()
+        self.stages = list(stages)
+        arr = (C.c_void_p * max(1, len(self.stages)))(*[m.h.value for m in self.stages])
+        h = C.c_void_p()
+        rc = self.L.fx8010_multi_chain_create(arr, len(self.stages), C.byref(h))
+        if rc != 0:
+            raise FxError(rc, self.L.fx8010_multi_chain_last_error(None).decode())
+        self.h = h
+        _register_chain(self, self.stages)
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.fx8010_multi_chain_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+    def _check(self, rc):
+        if rc != 0:
+            raise FxError(rc, self.L.fx8010_multi_chain_last_error(self.h).decode())
+
+    def process_host(self, x, n_samples=None, out=None, wait: bool = True) -> np.ndarray:
+        """fx8010_multi_chain_process_batch_host: x [C][S][N] over all instances (None: no input) -> out [C][S][N].  wait=False queues
+        the work; the arrays are kept until synchronize()."""
+        return self.process_host_curves(x, [], n_samples=n_samples, out=out, wait=wait)
+
+    def process_host_curves(self, x, curves, n_samples=None, out=None, wait: bool = True) -> np.ndarray:
+        """fx8010_multi_chain_process_batch_host_curves: curves = [(stage, register index, ndarray, broadcast)], each [S][N] float32 over
+        all instances, or [S] with broadcast."""
+        m0 = self.stages[0]
+        if x is not None:
+            x = np.ascontiguousarray(x, dtype=np.float32).reshape(m0.c, -1, m0.n)
+            n_samples = x.shape[1]
+        out = _host_out(out, m0.c, n_samples, m0.n, 0)
+        arr, keep = _chain_host_curves(curves, n_samples, m0.n, 0)
+        self._check(self.L.fx8010_multi_chain_process_batch_host_curves(self.h, _ptr(x), _ptr(out), n_samples, C.addressof(arr), len(curves),
+                                                                        1 if wait else 0))
+        self._pending = [] if wait else getattr(self, "_pending", []) + [(x, out, arr, keep)]
+        return out
+
+    def synchronize(self):
+        self._check(self.L.fx8010_multi_chain_synchronize(self.h))
+        self._pending = []
+
+    def shard_status(self, g: int) -> dict:
+        """fx8010_chain_status of shard g's chain."""
+        c = self.L.fx8010_multi_chain_shard(self.h, g)
+        if not c:
+            raise FxError(1, f"no shard {g}")
+        return _chain_status(self.L, c)
 
 
 def shard_range(n_total: int, rank: int, world: int):

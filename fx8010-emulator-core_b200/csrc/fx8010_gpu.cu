@@ -22,6 +22,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -1798,6 +1799,35 @@ bool reads_input(const fx8010_gpu* h) {
     return false;
 }
 
+// What every chain call checks before it queues anything (device buffers, io = "d_", or host buffers, io = ""): every stage has a program,
+// `out` is given and the count not negative, `in` is given when stage 0 reads an input, and — with n_curves != 0 — the curve list: a count
+// of 0..8, a list, and for every stage its own curves as fx8010_gpu_process_batch_curves checks them.  per_stage gets each stage's curves.
+template <class Curve>
+int chain_check(fx8010_chain* c, const char* io, const float* in, const float* out, int n_samples, const Curve* curves, int n_curves,
+                const float* const Curve::*values, std::vector<std::vector<fx8010_control_curve>>& per_stage) {
+    const int NS = (int)c->st.size();
+    for (int j = 0; j < NS; ++j)
+        if (!c->st[j]->loaded) return chain_fail(c, FX8010_ERR_NO_PROGRAM, "stage " + std::to_string(j) + " has no program");
+    if (!out || n_samples < 0) return chain_fail(c, FX8010_ERR_ARG, std::string(io) + "out is NULL or n_samples negative");
+    if (!in && reads_input(c->st[0])) return chain_fail(c, FX8010_ERR_ARG, std::string(io) + "in is NULL but stage 0 reads an input");
+    per_stage.assign((size_t)NS, {});
+    if (n_curves == 0) return FX8010_OK;
+    // The whole list is checked, for every stage, before any stage runs (the stage-by-stage path must not run stage 0 and then refuse stage 2).
+    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || !curves)
+        return chain_fail(c, FX8010_ERR_ARG, "the curve list is NULL or the curve count outside 0..8");
+    for (int q = 0; q < n_curves; ++q) {
+        const Curve& cv = curves[q];
+        if (cv.stage < 0 || cv.stage >= NS) return chain_fail(c, FX8010_ERR_ARG, "control curve " + std::to_string(q) + ": stage index out of range");
+        per_stage[cv.stage].push_back(fx8010_control_curve{cv.reg_index, cv.broadcast ? 1 : 0, cv.*values});
+    }
+    for (int j = 0; j < NS; ++j) {
+        CurveRows rows;
+        if (curves_begin(c->st[j], per_stage[j].data(), (int)per_stage[j].size(), &fx8010_control_curve::d_values, false, rows))
+            return chain_fail(c, FX8010_ERR_ARG, "stage " + std::to_string(j) + ": " + c->st[j]->err);
+    }
+    return FX8010_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1829,6 +1859,13 @@ int fx8010_chain_create(fx8010_gpu* const* stages, int n_stages, fx8010_chain** 
 void fx8010_chain_destroy(fx8010_chain* c) {
     if (!c) return;
     cudaSetDevice(c->device);
+    // A host-buffer call leaves every stage's latest work on stage 0's compute stream, which dies with stage 0: once it has drained, no
+    // stage refers to it any more, so that the handles may be destroyed in any order.
+    for (fx8010_gpu* h : c->st)
+        if (h != c->st[0] && h->has_last && h->last_stream == c->st[0]->s_comp) {
+            cudaStreamSynchronize(h->last_stream);
+            h->has_last = false;
+        }
     cudaFree(c->d_mid[0]); cudaFree(c->d_mid[1]);            // (waits for the device)
     if (c->ev) cudaEventDestroy(c->ev);
     tr_detach(c->device, c->plain.tr);
@@ -1838,10 +1875,9 @@ void fx8010_chain_destroy(fx8010_chain* c) {
 
 int fx8010_chain_process_batch(fx8010_chain* c, const float* d_in, float* d_out, int n_samples, void* stream) {
     if (!c) return FX8010_ERR_ARG;
-    for (size_t j = 0; j < c->st.size(); ++j)
-        if (!c->st[j]->loaded) return chain_fail(c, FX8010_ERR_NO_PROGRAM, "stage " + std::to_string(j) + " has no program");
-    if (!d_out || n_samples < 0) return chain_fail(c, FX8010_ERR_ARG, "d_out is NULL or n_samples negative");
-    if (!d_in && reads_input(c->st[0])) return chain_fail(c, FX8010_ERR_ARG, "d_in is NULL but stage 0 reads an input");
+    std::vector<std::vector<fx8010_control_curve>> per_stage;
+    const int rc = chain_check(c, "d_", d_in, d_out, n_samples, (const fx8010_chain_curve*)nullptr, 0, &fx8010_chain_curve::d_values, per_stage);
+    if (rc) return rc;
     if (cudaSetDevice(c->device) != cudaSuccess) return chain_fail(c, FX8010_ERR_CUDA, "cudaSetDevice failed");
     if (n_samples == 0) return FX8010_OK;
     cudaStream_t st = (cudaStream_t)stream;
@@ -1860,28 +1896,16 @@ int fx8010_chain_process_batch_curves(fx8010_chain* c, const float* d_in, float*
                                       int n_curves, void* stream) {
     if (!c) return FX8010_ERR_ARG;
     if (n_curves == 0) return fx8010_chain_process_batch(c, d_in, d_out, n_samples, stream);
-    for (size_t j = 0; j < c->st.size(); ++j)
-        if (!c->st[j]->loaded) return chain_fail(c, FX8010_ERR_NO_PROGRAM, "stage " + std::to_string(j) + " has no program");
-    if (!d_out || n_samples < 0) return chain_fail(c, FX8010_ERR_ARG, "d_out is NULL or n_samples negative");
-    if (!d_in && reads_input(c->st[0])) return chain_fail(c, FX8010_ERR_ARG, "d_in is NULL but stage 0 reads an input");
-    // The whole list is checked, for every stage, before any stage runs (the stage-by-stage path must not run stage 0 and then refuse stage 2).
-    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || !curves)
-        return chain_fail(c, FX8010_ERR_ARG, "the curve list is NULL or the curve count outside 0..8");
+    std::vector<std::vector<fx8010_control_curve>> per_stage;
+    const int rc = chain_check(c, "d_", d_in, d_out, n_samples, curves, n_curves, &fx8010_chain_curve::d_values, per_stage);
+    if (rc) return rc;
     const int NS = (int)c->st.size();
-    std::vector<std::vector<fx8010_control_curve>> per_stage((size_t)NS);
     std::vector<ChainCurve> key;
     CurveBlock cb = {};
     for (int q = 0; q < n_curves; ++q) {
         const fx8010_chain_curve& cv = curves[q];
-        if (cv.stage < 0 || cv.stage >= NS) return chain_fail(c, FX8010_ERR_ARG, "control curve " + std::to_string(q) + ": stage index out of range");
-        per_stage[cv.stage].push_back(fx8010_control_curve{cv.reg_index, cv.broadcast ? 1 : 0, cv.d_values});
         key.push_back(ChainCurve{cv.stage, cv.reg_index, (uint8_t)(cv.broadcast ? 1 : 0)});
         cb.p[q] = cv.d_values; cb.bcast[q] = cv.broadcast ? 1 : 0;
-    }
-    for (int j = 0; j < NS; ++j) {
-        CurveRows rows;
-        if (curves_begin(c->st[j], per_stage[j].data(), (int)per_stage[j].size(), &fx8010_control_curve::d_values, false, rows))
-            return chain_fail(c, FX8010_ERR_ARG, "stage " + std::to_string(j) + ": " + c->st[j]->err);
     }
     if (cudaSetDevice(c->device) != cudaSuccess) return chain_fail(c, FX8010_ERR_CUDA, "cudaSetDevice failed");
     if (n_samples == 0) return FX8010_OK;
@@ -2364,12 +2388,18 @@ static __global__ void fx_broadcast_kernel(const float* __restrict__ src, float*
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) d[i] = v;
 }
 
+// The compute step of one sub-block of the host pipeline, queued on h->s_comp: `len` periods from d_in (NULL without input) to d_out, channel
+// stride cs, with `staged` (NULL without curves) pointing at this sub-block's rows of every curve.
+using HostStep = std::function<int(const float* d_in, float* d_out, size_t cs, int len, const CurveRows* staged)>;
+
 // host_n: instances per row of the HOST buffers (>= N: this handle's columns are a slice of a wider [channel][sample][instance] block)
 // bcast: `in` holds ONE value per channel and sample period ([channel][sample]); it is copied as it is and spread over the instances on the device
-// cv: control curves in HOST memory (curves_begin has checked and armed them): a per-instance curve is [n_samples][host_n] from this handle's
-// first column, a broadcast one [n_samples]; each sub-block's rows are staged like its inputs and the sub-block runs launch_curves
-static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_samples, bool wait, size_t host_n = 0, bool bcast = false,
-                             const CurveRows* cv = nullptr) {
+// cv: control curves in HOST memory (checked and armed by the caller): a per-instance curve is [n_samples][host_n] from this handle's first
+// column, a broadcast one [n_samples]; each sub-block's rows are staged like its inputs and handed to `step`
+// packed: a sub-block's staged channels are len * N floats apart ([channel][len][instance], the layout of a device call on len periods);
+// otherwise sub * N
+static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_samples, bool wait, size_t host_n, bool bcast, const CurveRows* cv,
+                             bool packed, const HostStep& step) {
     FX_NEED_PROGRAM(h);
     if (!out || n_samples < 0) return fail(h, FX8010_ERR_ARG, "out is NULL or n_samples negative");
     if (n_samples == 0) return FX8010_OK;
@@ -2430,6 +2460,7 @@ static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_s
     for (long s0 = 0; s0 < n_samples; s0 += sub, ++h->pipe_seq) {
         const int buf = (int)(h->pipe_seq % HOST_PIPE_BUFS);
         const long len = std::min<long>(sub, n_samples - s0);
+        const size_t cs = (size_t)(packed ? len : sub) * N;
         if (h->pipe_seq >= HOST_PIPE_BUFS) FX_CUDA(h, cudaStreamWaitEvent(h->s_h2d, h->ev_comp[buf], 0));     // stage_in[buf] consumed
         if (in && bcast)
             for (size_t c = 0; c < C; ++c)
@@ -2437,10 +2468,10 @@ static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_s
         else if (in)
             for (size_t c = 0; c < C; ++c) {
                 if (host_n == N)
-                    FX_CUDA(h, cudaMemcpyAsync(h->d_stage_in[buf] + c * (size_t)sub * N, in + (c * (size_t)n_samples + s0) * N,
+                    FX_CUDA(h, cudaMemcpyAsync(h->d_stage_in[buf] + c * cs, in + (c * (size_t)n_samples + s0) * N,
                                                sizeof(float) * len * N, cudaMemcpyHostToDevice, h->s_h2d));
                 else
-                    FX_CUDA(h, cudaMemcpy2DAsync(h->d_stage_in[buf] + c * (size_t)sub * N, sizeof(float) * N, in + (c * (size_t)n_samples + s0) * host_n,
+                    FX_CUDA(h, cudaMemcpy2DAsync(h->d_stage_in[buf] + c * cs, sizeof(float) * N, in + (c * (size_t)n_samples + s0) * host_n,
                                                  sizeof(float) * host_n, sizeof(float) * N, (size_t)len, cudaMemcpyHostToDevice, h->s_h2d));
             }
         CurveRows staged = {};
@@ -2465,23 +2496,22 @@ static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_s
         if (in && bcast) {
             for (size_t c = 0; c < C; ++c) {
                 fx_broadcast_kernel<<<dim3((unsigned)std::min<size_t>(64, (N + 255) / 256), (unsigned)len), 256, 0, h->s_comp>>>(
-                    h->d_bcast[buf] + c * (size_t)sub, h->d_stage_in[buf] + c * (size_t)sub * N, (int)len, (int)N);
+                    h->d_bcast[buf] + c * (size_t)sub, h->d_stage_in[buf] + c * cs, (int)len, (int)N);
                 h->info.kernel_launches++;
             }
             FX_CUDA(h, cudaGetLastError());
         }
         const float* d_in = in ? h->d_stage_in[buf] : nullptr;
-        const int rc = cv ? launch_curves(h, d_in, h->d_stage_out[buf], (size_t)sub * N, (int)len, staged, h->s_comp)
-                          : launch_block(h, d_in, h->d_stage_out[buf], (size_t)sub * N, (size_t)sub * N, (int)len, h->s_comp, true);   // (the internal stream carries this handle's launches only)
+        const int rc = step(d_in, h->d_stage_out[buf], cs, (int)len, cv ? &staged : nullptr);
         if (rc) return rc;
         FX_CUDA(h, cudaEventRecord(h->ev_comp[buf], h->s_comp));
         FX_CUDA(h, cudaStreamWaitEvent(h->s_d2h, h->ev_comp[buf], 0));
         for (size_t c = 0; c < C; ++c) {
             if (host_n == N)
-                FX_CUDA(h, cudaMemcpyAsync(out + (c * (size_t)n_samples + s0) * N, h->d_stage_out[buf] + c * (size_t)sub * N,
+                FX_CUDA(h, cudaMemcpyAsync(out + (c * (size_t)n_samples + s0) * N, h->d_stage_out[buf] + c * cs,
                                            sizeof(float) * len * N, cudaMemcpyDeviceToHost, h->s_d2h));
             else
-                FX_CUDA(h, cudaMemcpy2DAsync(out + (c * (size_t)n_samples + s0) * host_n, sizeof(float) * host_n, h->d_stage_out[buf] + c * (size_t)sub * N,
+                FX_CUDA(h, cudaMemcpy2DAsync(out + (c * (size_t)n_samples + s0) * host_n, sizeof(float) * host_n, h->d_stage_out[buf] + c * cs,
                                              sizeof(float) * N, sizeof(float) * N, (size_t)len, cudaMemcpyDeviceToHost, h->s_d2h));
         }
         FX_CUDA(h, cudaEventRecord(h->ev_d2h[buf], h->s_d2h));
@@ -2490,17 +2520,27 @@ static int process_host_impl(fx8010_gpu* h, const float* in, float* out, int n_s
     return FX8010_OK;
 }
 
+// The single-handle host calls: each sub-block runs launch_block, or launch_curves with the call's curves.
+static int process_host_handle(fx8010_gpu* h, const float* in, float* out, int n_samples, bool wait, size_t host_n = 0, bool bcast = false,
+                               const CurveRows* cv = nullptr) {
+    return process_host_impl(h, in, out, n_samples, wait, host_n, bcast, cv, false,
+                             [h](const float* d_in, float* d_out, size_t cs, int len, const CurveRows* staged) {
+        return staged ? launch_curves(h, d_in, d_out, cs, len, *staged, h->s_comp)
+                      : launch_block(h, d_in, d_out, cs, cs, len, h->s_comp, true);   // (the internal stream carries this handle's launches only)
+    });
+}
+
 int fx8010_gpu_process_batch_host(fx8010_gpu* h, const float* in, float* out, int n_samples) {
-    return process_host_impl(h, in, out, n_samples, true);
+    return process_host_handle(h, in, out, n_samples, true);
 }
 int fx8010_gpu_process_batch_host_async(fx8010_gpu* h, const float* in, float* out, int n_samples) {
-    return process_host_impl(h, in, out, n_samples, false);
+    return process_host_handle(h, in, out, n_samples, false);
 }
 int fx8010_gpu_process_batch_host_slice(fx8010_gpu* h, const float* in, float* out, int n_samples, size_t host_instances, int wait) {
-    return process_host_impl(h, in, out, n_samples, wait != 0, host_instances);
+    return process_host_handle(h, in, out, n_samples, wait != 0, host_instances);
 }
 int fx8010_gpu_process_batch_host_broadcast(fx8010_gpu* h, const float* in, float* out, int n_samples, size_t host_instances, int wait) {
-    return process_host_impl(h, in, out, n_samples, wait != 0, host_instances, true);
+    return process_host_handle(h, in, out, n_samples, wait != 0, host_instances, true);
 }
 int fx8010_gpu_process_batch_host_curves(fx8010_gpu* h, const float* in, float* out, int n_samples, const fx8010_host_curve* curves, int n_curves,
                                          size_t host_instances, int wait) {
@@ -2510,7 +2550,69 @@ int fx8010_gpu_process_batch_host_curves(fx8010_gpu* h, const float* in, float* 
     CurveRows rows;
     const int rc = curves_begin(h, curves, n_curves, &fx8010_host_curve::values, n_samples > 0, rows);
     if (rc) return rc;
-    return process_host_impl(h, in, out, n_samples, wait != 0, host_instances, false, n_curves > 0 ? &rows : nullptr);
+    return process_host_handle(h, in, out, n_samples, wait != 0, host_instances, false, n_curves > 0 ? &rows : nullptr);
+}
+
+// fx8010_chain_process_batch_host(_curves): stage 0's host pipeline, each sub-block running the device chain call on its staging buffers
+// (packed, so that they are laid out as the device call's buffers) on stage 0's compute stream.
+static int chain_host(fx8010_chain* c, const float* in, float* out, int n_samples, const fx8010_chain_host_curve* curves, int n_curves,
+                      size_t host_n, bool wait) {
+    if (!c) return FX8010_ERR_ARG;
+    std::vector<std::vector<fx8010_control_curve>> per_stage;
+    int rc = chain_check(c, "", in, out, n_samples, curves, n_curves, &fx8010_chain_host_curve::values, per_stage);
+    if (rc) return rc;
+    fx8010_gpu* h0 = c->st[0];
+    if (host_n != 0 && host_n < (size_t)h0->N) return chain_fail(c, FX8010_ERR_ARG, "host row length below the instance count");
+    if (cudaSetDevice(c->device) != cudaSuccess) return chain_fail(c, FX8010_ERR_CUDA, "cudaSetDevice failed");
+    if (n_samples == 0) return FX8010_OK;
+    for (fx8010_gpu* h : c->st) {                            // every stage's earlier work, on any stream, comes first
+        rc = order_on(h, h0->s_comp);
+        if (rc) return chain_fail(c, rc, h->err);
+    }
+    CurveRows rows = {};
+    rows.n = n_curves;
+    for (int q = 0; q < n_curves; ++q) {
+        rows.reg[q] = curves[q].reg_index;
+        rows.cv.p[q] = curves[q].values; rows.cv.bcast[q] = curves[q].broadcast ? 1 : 0;
+    }
+    bool all_fused = true, step_failed = false;
+    std::string why;
+    rc = process_host_impl(h0, in, out, n_samples, wait, host_n, false, n_curves > 0 ? &rows : nullptr, true,
+                           [&](const float* d_in, float* d_out, size_t, int len, const CurveRows* staged) {
+        int r;
+        if (staged) {
+            fx8010_chain_curve cv[FX8010_MAX_CONTROL_CURVES];
+            for (int q = 0; q < n_curves; ++q) cv[q] = fx8010_chain_curve{curves[q].stage, curves[q].reg_index, rows.cv.bcast[q], 0, staged->cv.p[q]};
+            r = fx8010_chain_process_batch_curves(c, d_in, d_out, len, cv, n_curves, h0->s_comp);
+        } else
+            r = fx8010_chain_process_batch(c, d_in, d_out, len, h0->s_comp);
+        if (r) { step_failed = true; return r; }
+        if (!c->fused_last && all_fused) { all_fused = false; why = c->why; }
+        return (int)FX8010_OK;
+    });
+    if (rc) return step_failed ? rc : chain_fail(c, rc, h0->err);
+    c->fused_last = all_fused ? 1 : 0;
+    c->why = all_fused ? std::string() : why;
+    // Stage 0's compute stream now carries other handles' launches: none of its later launches may count on following its own.
+    for (fx8010_gpu* h : c->st) h->chain.clear();
+    return FX8010_OK;
+}
+
+int fx8010_chain_process_batch_host(fx8010_chain* c, const float* in, float* out, int n_samples, size_t host_instances, int wait) {
+    return chain_host(c, in, out, n_samples, nullptr, 0, host_instances, wait != 0);
+}
+int fx8010_chain_process_batch_host_curves(fx8010_chain* c, const float* in, float* out, int n_samples, const fx8010_chain_host_curve* curves,
+                                           int n_curves, size_t host_instances, int wait) {
+    return chain_host(c, in, out, n_samples, curves, n_curves, host_instances, wait != 0);
+}
+
+int fx8010_chain_synchronize(fx8010_chain* c) {
+    if (!c) return FX8010_ERR_ARG;
+    for (fx8010_gpu* h : c->st) {
+        const int rc = sync_all(h);
+        if (rc) return chain_fail(c, rc, h->err);
+    }
+    return FX8010_OK;
 }
 
 int fx8010_gpu_synchronize(fx8010_gpu* h, void* stream) {

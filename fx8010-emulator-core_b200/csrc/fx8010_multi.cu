@@ -252,4 +252,131 @@ int fx8010_multi_get_runtime_flags(fx8010_multi* m, unsigned int* flags, int cle
 
 const char* fx8010_multi_last_error(fx8010_multi* m) { return m ? m->err.c_str() : g_multi_create_error.c_str(); }
 
+void fx8010_multi_shard_chain_curves(const fx8010_chain_host_curve* curves, int n_curves, int n_total, int g, int G, fx8010_chain_host_curve* out) {
+    int lo = 0;
+    fx8010_multi_shard_range(n_total, g, G, &lo, nullptr);
+    for (int j = 0; j < n_curves; ++j) {
+        out[j] = curves[j];
+        if (!curves[j].broadcast && curves[j].values) out[j].values = curves[j].values + lo;
+    }
+}
+
+}  // extern "C"
+
+// A chain of executors (fx8010_multi_chain_*): one fx8010_chain per shard over the stages' handles of that shard, driven by the shard
+// threads of stage 0's executor.
+struct fx8010_multi_chain {
+    fx8010_multi* m = nullptr;                       // stage 0's executor (its threads run the calls)
+    std::vector<fx8010_chain*> chains;               // per shard
+    std::string err;
+};
+
+namespace {
+
+thread_local std::string g_multi_chain_create_error;
+
+int multi_chain_fail(const std::string& msg) {
+    g_multi_chain_create_error = msg;
+    return FX8010_ERR_ARG;
+}
+
+// Runs `job` (shard g's chain) on every shard thread of the chain; a failure is reported with the chain's own error text.
+int multi_chain_run(fx8010_multi_chain* mc, const std::function<int(Shard&, fx8010_chain*)>& job) {
+    const int rc = run_all(mc->m, [&](Shard& s) { return job(s, mc->chains[(size_t)s.g]); });
+    if (rc == FX8010_OK) return rc;
+    for (Shard* s : mc->m->shards) {
+        if (!s->rc) continue;
+        mc->err = "device " + std::to_string(s->device) + " (instances " + std::to_string(s->lo) + ".." + std::to_string(s->hi) + "): " +
+                  fx8010_chain_last_error(mc->chains[(size_t)s->g]);
+        break;
+    }
+    return rc;
+}
+
+int multi_chain_process(fx8010_multi_chain* mc, const float* in, float* out, int n_samples, const fx8010_chain_host_curve* curves, int n_curves,
+                        int wait) {
+    if (!mc) return FX8010_ERR_ARG;
+    if (!out || n_samples < 0) {
+        mc->err = "out is NULL or n_samples negative";
+        return FX8010_ERR_ARG;
+    }
+    if (n_curves < 0 || n_curves > FX8010_MAX_CONTROL_CURVES || (n_curves > 0 && !curves)) {
+        mc->err = "the curve list is NULL or the curve count outside 0..8";
+        return FX8010_ERR_ARG;
+    }
+    fx8010_multi* m = mc->m;
+    const size_t N = (size_t)m->N;
+    const int G = (int)m->shards.size();
+    // Every shard checks the list before it queues anything, against the same programs: a list one shard refuses, all refuse.
+    return multi_chain_run(mc, [=](Shard& s, fx8010_chain* c) {
+        fx8010_chain_host_curve mine[FX8010_MAX_CONTROL_CURVES];
+        fx8010_multi_shard_chain_curves(curves, n_curves, m->N, s.g, G, mine);
+        return fx8010_chain_process_batch_host_curves(c, in ? in + s.lo : nullptr, out + s.lo, n_samples, mine, n_curves, N, wait);
+    });
+}
+
+}  // namespace
+
+extern "C" {
+
+int fx8010_multi_chain_create(fx8010_multi* const* stages, int n_stages, fx8010_multi_chain** out) {
+    if (!out) return multi_chain_fail("out is NULL");
+    *out = nullptr;
+    if (!stages || n_stages < 1 || n_stages > FX8010_MAX_CHAIN_STAGES) return multi_chain_fail("the stage count must be 1..FX8010_MAX_CHAIN_STAGES");
+    for (int j = 0; j < n_stages; ++j) {
+        if (!stages[j]) return multi_chain_fail("stage " + std::to_string(j) + " is NULL");
+        for (int k = 0; k < j; ++k) if (stages[k] == stages[j]) return multi_chain_fail("an executor appears twice in the chain");
+        if (stages[j]->N != stages[0]->N || stages[j]->C != stages[0]->C)
+            return multi_chain_fail("stage " + std::to_string(j) + " differs in instance count or channel count");
+        if (stages[j]->shards.size() != stages[0]->shards.size())
+            return multi_chain_fail("stage " + std::to_string(j) + " differs in shard count");
+        for (size_t g = 0; g < stages[0]->shards.size(); ++g)
+            if (stages[j]->shards[g]->device != stages[0]->shards[g]->device)
+                return multi_chain_fail("stage " + std::to_string(j) + ": shard " + std::to_string(g) + " is on another device");
+    }
+    fx8010_multi_chain* mc = new fx8010_multi_chain();
+    mc->m = stages[0];
+    for (size_t g = 0; g < stages[0]->shards.size(); ++g) {
+        std::vector<fx8010_gpu*> h;
+        for (int j = 0; j < n_stages; ++j) h.push_back(stages[j]->shards[g]->h);
+        fx8010_chain* c = nullptr;
+        const int rc = fx8010_chain_create(h.data(), n_stages, &c);
+        if (rc) {
+            g_multi_chain_create_error = "shard " + std::to_string(g) + ": " + fx8010_chain_last_error(nullptr);
+            fx8010_multi_chain_destroy(mc);
+            return rc;
+        }
+        mc->chains.push_back(c);
+    }
+    *out = mc;
+    return FX8010_OK;
+}
+
+void fx8010_multi_chain_destroy(fx8010_multi_chain* mc) {
+    if (!mc) return;
+    for (fx8010_chain* c : mc->chains) fx8010_chain_destroy(c);
+    delete mc;
+}
+
+int fx8010_multi_chain_process_batch_host(fx8010_multi_chain* mc, const float* in, float* out, int n_samples, int wait) {
+    return multi_chain_process(mc, in, out, n_samples, nullptr, 0, wait);
+}
+
+int fx8010_multi_chain_process_batch_host_curves(fx8010_multi_chain* mc, const float* in, float* out, int n_samples,
+                                                 const fx8010_chain_host_curve* curves, int n_curves, int wait) {
+    return multi_chain_process(mc, in, out, n_samples, curves, n_curves, wait);
+}
+
+int fx8010_multi_chain_synchronize(fx8010_multi_chain* mc) {
+    if (!mc) return FX8010_ERR_ARG;
+    return multi_chain_run(mc, [](Shard&, fx8010_chain* c) { return fx8010_chain_synchronize(c); });
+}
+
+fx8010_chain* fx8010_multi_chain_shard(fx8010_multi_chain* mc, int g) {
+    if (!mc || g < 0 || g >= (int)mc->chains.size()) return nullptr;
+    return mc->chains[(size_t)g];
+}
+
+const char* fx8010_multi_chain_last_error(fx8010_multi_chain* mc) { return mc ? mc->err.c_str() : g_multi_chain_create_error.c_str(); }
+
 }  // extern "C"

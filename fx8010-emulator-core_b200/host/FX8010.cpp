@@ -68,33 +68,77 @@ void FX8010::ensureUploaded() {
 }
 
 FX8010Chain::FX8010Chain(const std::vector<FX8010*>& stages) : stages_(stages) {
-    std::vector<fx8010_gpu*> h;
-    for (FX8010* s : stages_) {
+    for (FX8010* s : stages_)
         if (!s) throw std::runtime_error("FX8010Chain (B200): a stage is NULL");
-        h.push_back(s->gpuHandle());                           // (throws for an object spread over several devices)
+    if (stages_.empty() || !stages_[0]->multiHandle()) {
+        std::vector<fx8010_gpu*> h;
+        for (FX8010* s : stages_) {
+            if (s->multiHandle()) throw std::runtime_error("FX8010Chain (B200): objects on one device and on several cannot be mixed");
+            h.push_back(s->gpuHandle());
+        }
+        if (fx8010_chain_create(h.data(), (int)h.size(), &chain_) != FX8010_OK)
+            throw std::runtime_error(std::string("FX8010Chain (B200): ") + fx8010_chain_last_error(nullptr));
+        return;
     }
-    if (fx8010_chain_create(h.data(), (int)h.size(), &chain_) != FX8010_OK)
-        throw std::runtime_error(std::string("FX8010Chain (B200): ") + fx8010_chain_last_error(nullptr));
+    std::vector<fx8010_multi*> m;
+    for (FX8010* s : stages_) {
+        fx8010_multi* e = s->multiHandle();
+        if (!e) throw std::runtime_error("FX8010Chain (B200): objects on one device and on several cannot be mixed");
+        m.push_back(e);
+    }
+    if (fx8010_multi_chain_create(m.data(), (int)m.size(), &multi_) != FX8010_OK)
+        throw std::runtime_error(std::string("FX8010Chain (B200): ") + fx8010_multi_chain_last_error(nullptr));
 }
 
-FX8010Chain::~FX8010Chain() { fx8010_chain_destroy(chain_); }
+FX8010Chain::~FX8010Chain() {
+    fx8010_chain_destroy(chain_);
+    fx8010_multi_chain_destroy(multi_);
+}
+
+void FX8010Chain::upload() {
+    for (FX8010* s : stages_) s->multiHandle();                // (ensures the upload on one device and on several)
+}
+
+int FX8010Chain::registerOf(int stage, const std::string& key) {
+    if (stage < 0 || stage >= (int)stages_.size())
+        throw std::runtime_error("FX8010Chain (B200): curve stage " + std::to_string(stage) + " out of range");
+    const int reg = stages_[stage]->frontend().findRegister(key);
+    if (reg < 0) throw std::runtime_error("FX8010Chain: unknown register '" + key + "' of stage " + std::to_string(stage));
+    return reg;
+}
+
+void FX8010Chain::processBlock(const float* in, float* out, int n_samples) {
+    upload();
+    const int rc = multi_ ? fx8010_multi_chain_process_batch_host(multi_, in, out, n_samples, 1)
+                          : fx8010_chain_process_batch_host(chain_, in, out, n_samples, 0, 1);
+    if (rc != FX8010_OK)
+        throw std::runtime_error(std::string("FX8010Chain (B200): process_batch_host failed: ") +
+                                 (multi_ ? fx8010_multi_chain_last_error(multi_) : fx8010_chain_last_error(chain_)));
+}
+
+void FX8010Chain::processBlockWithCurves(const float* in, float* out, int n_samples, const std::vector<HostCurve>& curves) {
+    upload();
+    std::vector<fx8010_chain_host_curve> cv;
+    for (const HostCurve& c : curves) cv.push_back(fx8010_chain_host_curve{c.stage, registerOf(c.stage, c.key), c.broadcast ? 1 : 0, 0, c.values});
+    const int rc = multi_ ? fx8010_multi_chain_process_batch_host_curves(multi_, in, out, n_samples, cv.data(), (int)cv.size(), 1)
+                          : fx8010_chain_process_batch_host_curves(chain_, in, out, n_samples, cv.data(), (int)cv.size(), 0, 1);
+    if (rc != FX8010_OK)
+        throw std::runtime_error(std::string("FX8010Chain (B200): process_batch_host_curves failed: ") +
+                                 (multi_ ? fx8010_multi_chain_last_error(multi_) : fx8010_chain_last_error(chain_)));
+}
 
 void FX8010Chain::processBlockDevice(const float* d_in, float* d_out, int n_samples, void* stream) {
-    for (FX8010* s : stages_) s->gpuHandle();                  // uploads a program loaded since the last block
+    if (multi_) throw std::runtime_error("FX8010Chain (B200): device-pointer members need a single device");
+    upload();
     if (fx8010_chain_process_batch(chain_, d_in, d_out, n_samples, stream) != FX8010_OK)
         throw std::runtime_error(std::string("FX8010Chain (B200): process_batch failed: ") + fx8010_chain_last_error(chain_));
 }
 
 void FX8010Chain::processBlockDeviceWithCurves(const float* d_in, float* d_out, int n_samples, const std::vector<Curve>& curves, void* stream) {
-    for (FX8010* s : stages_) s->gpuHandle();                  // uploads a program loaded since the last block
+    if (multi_) throw std::runtime_error("FX8010Chain (B200): device-pointer members need a single device");
+    upload();
     std::vector<fx8010_chain_curve> cv;
-    for (const Curve& c : curves) {
-        if (c.stage < 0 || c.stage >= (int)stages_.size())
-            throw std::runtime_error("FX8010Chain (B200): curve stage " + std::to_string(c.stage) + " out of range");
-        const int reg = stages_[c.stage]->frontend().findRegister(c.key);
-        if (reg < 0) throw std::runtime_error("FX8010Chain: unknown register '" + c.key + "' of stage " + std::to_string(c.stage));
-        cv.push_back(fx8010_chain_curve{c.stage, reg, c.broadcast ? 1 : 0, 0, c.d_values});
-    }
+    for (const Curve& c : curves) cv.push_back(fx8010_chain_curve{c.stage, registerOf(c.stage, c.key), c.broadcast ? 1 : 0, 0, c.d_values});
     if (fx8010_chain_process_batch_curves(chain_, d_in, d_out, n_samples, cv.data(), (int)cv.size(), stream) != FX8010_OK)
         throw std::runtime_error(std::string("FX8010Chain (B200): process_batch_curves failed: ") + fx8010_chain_last_error(chain_));
 }
@@ -103,6 +147,11 @@ fx8010_gpu* FX8010::gpuHandle() {
     ensureUploaded();
     if (multi_) throw std::runtime_error("FX8010 (B200): this object drives several GPUs; there is no single device handle");
     return gpu_;
+}
+
+fx8010_multi* FX8010::multiHandle() {
+    ensureUploaded();
+    return multi_;
 }
 
 void FX8010::setTranslation(int mode) {

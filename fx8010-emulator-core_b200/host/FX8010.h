@@ -92,6 +92,7 @@ public:
     static void setKernelCacheDir(const std::string& dir);
     unsigned long long getInstructionCounterTotal();           // summed over instances
     fx8010_gpu* gpuHandle();                                   // creates the handle / uploads the program if needed
+    fx8010_multi* multiHandle();                               // the same for the executor of an object on several GPUs; NULL for one on one device
     fx8010::Frontend& frontend() { return front_; }
 
 private:
@@ -111,14 +112,25 @@ private:
 };
 
 // Several objects' programs one after another within every sample period (include/fx8010_gpu.h, fx8010_chain_*): output channel c of
-// one stage is input channel c of the next, and a block costs one launch when every stage is stateless.  The objects must drive one
-// device each, the same one, with equal channel and instance counts (the constructor throws otherwise), and outlive the chain.
+// one stage is input channel c of the next, and a block costs one launch when every stage is stateless.  The objects must all drive one
+// device, the same one, or all be made with the multi-device constructor over the same device list (fx8010_multi_chain_* of
+// include/fx8010_multi.h), with equal channel and instance counts (the constructor throws otherwise, and for a mix of the two kinds), and
+// outlive the chain.  On several devices the host-buffer members work as on one and the device-pointer members throw.
 class FX8010_CLASS FX8010Chain {
 public:
     explicit FX8010Chain(const std::vector<FX8010*>& stages);
     ~FX8010Chain();
     FX8010Chain(const FX8010Chain&) = delete;
     FX8010Chain& operator=(const FX8010Chain&) = delete;
+    // n_samples sample periods of every instance through every stage; HOST buffers [channel][sample][instance] (in may be NULL when the
+    // first stage reads no input, out may equal in); every sub-block crosses PCIe once, whatever the number of stages; returns when `out`
+    // is complete
+    void processBlock(const float* in, float* out, int n_samples);
+    // the same with sample-accurate automation of any stage's registers (fx8010_chain_process_batch_host_curves): register `key` of stage
+    // `stage` takes values[s] (broadcast) or values[s * numInstances + i] right before that stage's sample period s; HOST buffers; throws
+    // on a stage out of range or an unknown name
+    struct HostCurve { int stage; std::string key; const float* values; bool broadcast; };
+    void processBlockWithCurves(const float* in, float* out, int n_samples, const std::vector<HostCurve>& curves);
     // n_samples sample periods of every instance through every stage; DEVICE buffers [channel][sample][instance], asynchronous on `stream`
     void processBlockDevice(const float* d_in, float* d_out, int n_samples, void* stream);
     // the same with sample-accurate automation of any stage's registers (include/fx8010_gpu.h, fx8010_chain_process_batch_curves): register
@@ -128,8 +140,12 @@ public:
     void processBlockDeviceWithCurves(const float* d_in, float* d_out, int n_samples, const std::vector<Curve>& curves, void* stream);
 
 private:
+    void upload();                                             // uploads a program loaded since the last block, on every stage
+    int registerOf(int stage, const std::string& key);
+
     std::vector<FX8010*> stages_;
-    fx8010_chain* chain_ = nullptr;
+    fx8010_chain* chain_ = nullptr;                            // stages on one device
+    fx8010_multi_chain* multi_ = nullptr;                      // stages on several
 };
 
 }  // namespace Klangraum

@@ -181,6 +181,19 @@ int fx8010_host_chain_process_block_device_curves(fx8010_host_chain* c, const fl
         return 0;
     } catch (const std::exception& e) { c->err = e.what(); return 1; }
 }
+int fx8010_host_chain_process_block(fx8010_host_chain* c, const float* in, float* out, int n_samples) {
+    try { c->chain.processBlock(in, out, n_samples); return 0; }
+    catch (const std::exception& e) { c->err = e.what(); return 1; }
+}
+int fx8010_host_chain_process_block_curves(fx8010_host_chain* c, const float* in, float* out, int n_samples, const int* stages,
+                                           const char* const* names, const float* const* values, const int* broadcast, int n_curves) {
+    try {
+        std::vector<Klangraum::FX8010Chain::HostCurve> cv;
+        for (int j = 0; j < n_curves; ++j) cv.push_back(Klangraum::FX8010Chain::HostCurve{stages[j], names[j], values[j], broadcast[j] != 0});
+        c->chain.processBlockWithCurves(in, out, n_samples, cv);
+        return 0;
+    } catch (const std::exception& e) { c->err = e.what(); return 1; }
+}
 const char* fx8010_host_chain_last_error(fx8010_host_chain* c) { return c ? c->err.c_str() : g_chain_create_error.c_str(); }
 
 }  // extern "C"

@@ -352,12 +352,13 @@ FX8010_API long long fx8010_translate_source_curves(const fx8010_program_image* 
  * compiles it in the background — the calls until then run stage by stage —, mode 2 before the call).  Otherwise it runs stage by stage
  * through intermediate blocks the chain owns.  The fused launch is booked in fx8010_chain_status, not in the stages' launch info; it
  * follows every stage's earlier work on any stream, and later work of any stage follows it.  Control curves on any stage's registers:
- * fx8010_chain_process_batch_curves.  Host-buffer and multi-GPU calls have no chain form. */
+ * fx8010_chain_process_batch_curves.  Host buffers: fx8010_chain_process_batch_host(_curves); several GPUs: fx8010_multi_chain_* of
+ * fx8010_multi.h. */
 #define FX8010_MAX_CHAIN_STAGES 8
 typedef struct fx8010_chain fx8010_chain;
 /* stages[n_stages] (1..FX8010_MAX_CHAIN_STAGES distinct handles of one device, instance count and channel count; FX8010_ERR_ARG
  * otherwise).  Programs may be loaded or reloaded after creation: the chain looks at its stages at every call.  Destroy the chain
- * before any of its handles. */
+ * before any of its handles: fx8010_chain_destroy reads them (it waits for the work a host-buffer call left on stage 0's stream). */
 FX8010_API int fx8010_chain_create(fx8010_gpu* const* stages, int n_stages, fx8010_chain** out);
 FX8010_API void fx8010_chain_destroy(fx8010_chain* c);
 /* d_in / d_out as in fx8010_gpu_process_batch (d_out may equal d_in).  Checks everything before it queues anything: FX8010_ERR_NO_PROGRAM when a stage has no
@@ -395,6 +396,37 @@ FX8010_API int fx8010_chain_process_batch_curves(fx8010_chain* c, const float* d
  * fx8010_gpu_translate_status; 0 also before any curve call), registers and local memory, and why it is not in use ("" when it is). */
 FX8010_API int fx8010_chain_status_curves(fx8010_chain* c, int* state, int* regs_per_thread, int* local_bytes, char* message,
                                           size_t message_cap);
+
+/* A chain over HOST buffers (pageable or page-locked): bit for bit, in `out` and in every stage's whole final state, what
+ * fx8010_chain_process_batch gives on device copies of the same buffers, and what the stages' own fx8010_gpu_process_batch_host calls
+ * give one after another through host temporaries.  `in`, `out` and host_instances (0 = n_instances) mean what they mean in
+ * fx8010_gpu_process_batch_host_slice: `in` may be NULL when stage 0 reads no input, and `out` may equal `in`.  The host pipeline of stage 0
+ * (its internal streams, staging buffers and sub-block length, FX8010_TUNE_SUB included) moves the sub-blocks; each sub-block runs the
+ * device chain call on its staging buffers, fused or stage by stage as that call decides (in mode 1 a compile that ends inside the call
+ * switches the later sub-blocks to the fused kernel), so a chain of k stages moves its samples over PCIe once instead of k times.  Every stage's earlier work on any stream comes first, and every stage's later work (its state getters included) follows.
+ * fx8010_chain_status afterwards: fused_last = 1 only when every sub-block ran fused, one launch counted per fused sub-block, and the
+ * message of the first sub-block that did not.  wait == 0 queues the work: `in`, `out` (and every curve array of the _curves form) must
+ * then stay untouched until fx8010_chain_synchronize; consecutive calls chain in order, and with page-locked buffers their copies overlap.
+ * Checks everything before it queues anything: the rules of fx8010_chain_process_batch with `in` / `out` for d_in / d_out, and
+ * FX8010_ERR_ARG for host_instances below n_instances. */
+FX8010_API int fx8010_chain_process_batch_host(fx8010_chain* c, const float* in, float* out, int n_samples, size_t host_instances, int wait);
+/* A control curve of a host-buffer chain call: fx8010_chain_curve with its values in HOST memory. */
+typedef struct fx8010_chain_host_curve {
+    int32_t stage;          /* 0 .. n_stages-1                                                                            */
+    int32_t reg_index;      /* a CONTROL or STATIC register of that stage's program                                       */
+    int32_t broadcast;      /* 0: values is [n_samples][host_instances] from the chain's first column; != 0: [n_samples]  */
+    int32_t reserved;
+    const float* values;    /* HOST pointer, float32                                                                      */
+} fx8010_chain_host_curve;
+/* fx8010_chain_process_batch_host with control curves: bit for bit what fx8010_chain_process_batch_curves gives on device copies.  Each
+ * sub-block copies its rows of every curve with its inputs (a per-instance curve adds 4 * n_instances bytes per period, and every stage's
+ * per-instance curves shorten the sub-blocks as in fx8010_gpu_process_batch_host_curves).  FX8010_ERR_ARG, with nothing queued, for the
+ * lists fx8010_chain_process_batch_curves refuses and for host_instances below n_instances.  With n_curves == 0 it is
+ * fx8010_chain_process_batch_host. */
+FX8010_API int fx8010_chain_process_batch_host_curves(fx8010_chain* c, const float* in, float* out, int n_samples,
+                                                      const fx8010_chain_host_curve* curves, int n_curves, size_t host_instances, int wait);
+/* Blocks until all work queued on every stage's internal streams (and the streams of their latest work) is done. */
+FX8010_API int fx8010_chain_synchronize(fx8010_chain* c);
 /* NULL: the last error of fx8010_chain_create on this thread. */
 FX8010_API const char* fx8010_chain_last_error(fx8010_chain* c);
 /* The source of the fused kernel for images[n_stages] (as fx8010_translate_source; -2 when some stage is not stateless). */

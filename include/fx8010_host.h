@@ -74,8 +74,9 @@ FX8010_API int fx8010_host_instruction_counter(fx8010_host* h);                 
 FX8010_API unsigned long long fx8010_host_instruction_counter_total(fx8010_host* h);
 FX8010_API fx8010_gpu* fx8010_host_gpu(fx8010_host* h);
 
-/* Klangraum::FX8010Chain: the programs of stages[n_stages] one after another within every sample period (fx8010_chain_* of fx8010_gpu.h).
- * create returns NULL when the objects do not share one device, channel and instance count (fx8010_host_chain_last_error(NULL) says why);
+/* Klangraum::FX8010Chain: the programs of stages[n_stages] one after another within every sample period (fx8010_chain_* of fx8010_gpu.h,
+ * fx8010_multi_chain_* of fx8010_multi.h for objects on several devices).  create returns NULL when the objects do not share one device, or
+ * one device list of the multi-device constructor, and one channel and instance count (fx8010_host_chain_last_error(NULL) says why);
  * destroy the chain before its objects. */
 typedef struct fx8010_host_chain fx8010_host_chain;
 FX8010_API fx8010_host_chain* fx8010_host_chain_create(fx8010_host* const* stages, int n_stages);
@@ -87,6 +88,12 @@ FX8010_API int fx8010_host_chain_process_block_device(fx8010_host_chain* c, cons
 FX8010_API int fx8010_host_chain_process_block_device_curves(fx8010_host_chain* c, const float* d_in, float* d_out, int n_samples,
                                                              const int* stages, const char* const* names, const float* const* d_values,
                                                              const int* broadcast, int n_curves, void* stream);
+/* processBlock(): HOST buffers [channel][sample][instance], on one device or several; returns when `out` is complete */
+FX8010_API int fx8010_host_chain_process_block(fx8010_host_chain* c, const float* in, float* out, int n_samples);
+/* processBlockWithCurves(): curve j drives register names[j] of stage stages[j] (values[j]: HOST pointer, broadcast[j]: see
+ * fx8010_chain_process_batch_host_curves); on one device or several */
+FX8010_API int fx8010_host_chain_process_block_curves(fx8010_host_chain* c, const float* in, float* out, int n_samples, const int* stages,
+                                                      const char* const* names, const float* const* values, const int* broadcast, int n_curves);
 FX8010_API const char* fx8010_host_chain_last_error(fx8010_host_chain* c);                          /* NULL on failure */
 
 #ifdef __cplusplus

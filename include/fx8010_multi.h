@@ -74,6 +74,35 @@ FX8010_API int fx8010_multi_get_runtime_flags(fx8010_multi* m, unsigned int* fla
 
 FX8010_API const char* fx8010_multi_last_error(fx8010_multi* m);
 
+/* ---- program chains across GPUs -------------------------------------------------------------------------------------------
+ * Executors run one after another within every sample period (fx8010_chain_* of fx8010_gpu.h, shard by shard): shard g's chain is
+ * fx8010_chain_create over the stages' shard-g handles, and a call runs fx8010_chain_process_batch_host(_curves) on every shard's own
+ * columns of the one caller buffer, from the shard threads of stage 0's executor. */
+typedef struct fx8010_multi_chain fx8010_multi_chain;
+/* stages[n_stages]: 1..FX8010_MAX_CHAIN_STAGES distinct executors with the same shard count, the same ordinal per shard and equal instance
+ * and channel counts (so their shard ranges match); FX8010_ERR_ARG otherwise, and fx8010_multi_chain_last_error(NULL) says why.  Calls on
+ * a multi chain and on its executors are serialised by the caller; destroy the multi chain before its executors. */
+FX8010_API int fx8010_multi_chain_create(fx8010_multi* const* stages, int n_stages, fx8010_multi_chain** out);
+FX8010_API void fx8010_multi_chain_destroy(fx8010_multi_chain* mc);
+/* in / out as in fx8010_multi_process_batch_host (out may equal in); wait == 0 queues the work: in and out stay untouched until
+ * fx8010_multi_chain_synchronize. */
+FX8010_API int fx8010_multi_chain_process_batch_host(fx8010_multi_chain* mc, const float* in, float* out, int n_samples, int wait);
+/* With control curves: a per-instance curve is [n_samples][n_instances] over ALL instances, and shard g reads its own columns; a broadcast
+ * one ([n_samples]) reaches every shard as it is.  Every shard checks the list before it queues anything, so a refused list
+ * (FX8010_ERR_ARG) leaves every shard untouched.  wait == 0: every values array also stays untouched until the synchronize. */
+FX8010_API int fx8010_multi_chain_process_batch_host_curves(fx8010_multi_chain* mc, const float* in, float* out, int n_samples,
+                                                            const fx8010_chain_host_curve* curves, int n_curves, int wait);
+FX8010_API int fx8010_multi_chain_synchronize(fx8010_multi_chain* mc);
+/* Shard g's chain (for fx8010_chain_status), NULL for g out of range. */
+FX8010_API fx8010_chain* fx8010_multi_chain_shard(fx8010_multi_chain* mc, int g);
+/* NULL: the last error of fx8010_multi_chain_create on this thread. */
+FX8010_API const char* fx8010_multi_chain_last_error(fx8010_multi_chain* mc);
+/* The curve list shard g of G (over n_total instances) passes to its chain: a per-instance curve's values moved to the shard's first column
+ * (fx8010_multi_shard_range), a broadcast one and a NULL pointer as they are; stage and reg_index kept.  out: n_curves entries.  Pure
+ * function, no device needed. */
+FX8010_API void fx8010_multi_shard_chain_curves(const fx8010_chain_host_curve* curves, int n_curves, int n_total, int g, int G,
+                                                fx8010_chain_host_curve* out);
+
 #ifdef __cplusplus
 }
 #endif
